@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo, N GPUs (torchrun for N > 1)
     python bench.py --impl reference --gpus N --steps K ...  # the reference's CPU path (oracle port), host cores
+    python bench.py ... --dump-outputs DIR                   # also save the last timed step's outputs (dump_outputs)
 
 Workload (BASELINE.json configs c3/c5, SURVEY.md section 8d): CombinatorialEnv, setup_8_channels.p, N = 6 devices,
 C = 8 channels, deadlines [7,14]x3, heterogeneous traffic at load 1/3, homogeneous_size=True (30 f32 per
@@ -57,6 +58,8 @@ def parse():
     ap.add_argument("--train-envs", type=int, default=65536,
                     help="envs per GPU of the c3 train-SPS sections (BASELINE config 3 names 65,536)")
     ap.add_argument("--train-envs-small", type=int, default=4096, help="extra c3 train-SPS point (round-1 shape)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed (rank 0's envs) to DIR/<name>.npy, see dump_outputs")
     return ap.parse_args()
 
 
@@ -591,6 +594,27 @@ def bench_env_configs(dev, hbm_peak, steps=200):
 # ------------------------------------------------------------------------------------------------
 # native arm
 # ------------------------------------------------------------------------------------------------
+DUMP_ENVS = 65536     # envs sampled by --dump-outputs: 180 observation rows x 65,536 envs x 4 B = 47 MB
+
+
+def dump_outputs(directory, env, obs, reward):
+    """What a caller of the timed run_random_access call holds after its last step, for a fixed, seeded sample of
+    envs: obs [N * OBS_DIM, S] and reward [S] of that step, and the discarded / received packet counters [S, N] the
+    URLLC score is computed from, as float32 (every value is exact); env_index [S] float64 names the sampled envs."""
+    import numpy as np
+    import torch
+    idx = np.sort(np.random.default_rng(0).choice(env.n_envs, size=min(env.n_envs, DUMP_ENVS), replace=False))
+    sel = torch.from_numpy(idx).to(obs.device)
+    out = {"env_index": idx.astype(np.float64),
+           "obs": obs.index_select(1, sel).cpu().numpy(),
+           "reward": reward.index_select(0, sel).float().cpu().numpy(),
+           "discarded": env.discarded_packets.index_select(0, sel).float().cpu().numpy(),
+           "received": env.received_packets.index_select(0, sel).float().cpu().numpy()}
+    os.makedirs(directory, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(directory, f"{name}.npy"), a)
+
+
 def run_native(args):
     import numpy as np
     import torch
@@ -668,6 +692,10 @@ def run_native(args):
     torch.cuda.synchronize()
     per = np.array([ev[i].elapsed_time(ev[i + 1]) for i in range(n_probe)])
     kernel_ms = float(np.median(per))             # gaps that contain a reset launch do not move the median
+    # the timed steps start from a reset into a fixed episode (Philox streams are keyed by episode and timestep), so
+    # their inputs do not depend on how many spin-up steps fitted into the spin-up time
+    env.set_episode(0)
+    env.reset_into(obs_buf)
     launches0 = _lib.launch_count()
     t_at_start = env.timestep
     barrier()
@@ -685,6 +713,8 @@ def run_native(args):
     barrier()
     clocks = sampler.stop(t_begin, time.perf_counter())
     launches_all = _lib.launch_count() - launches0
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, env, obs_buf, rew_buf)
     # launches inside [e0, e1]: the K steps + the resets that fell between them (the lead-in's are not counted)
     t_sim, n_resets = t_at_start, 0
     for i in range(LEAD_IN + K):
