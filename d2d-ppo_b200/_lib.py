@@ -50,8 +50,7 @@ DIST_BERNOULLI, DIST_CATEGORICAL = 0, 1
 ACT_SAMPLE, ACT_GREEDY, ACT_GIVEN = 0, 1, 2
 ACT_HOST_REFERENCE, ACT_HOST_DEVICE_LAYOUT = 0, 1
 QLOSS_HUBER, QLOSS_MSE = 0, 1
-SWITCH_GRU_WINDOW_TC, SWITCH_GRU_BPTT_TC, SWITCH_DENSE_TC, SWITCH_WGRAD_TC, SWITCH_FUSED_HEAD, SWITCH_ALL_TC, \
-    SWITCH_BPTT_RECOMPUTE, SWITCH_WINDOW_HEAD, SWITCH_WINDOW_WIDE, SWITCH_ENV_MULTISTEP, SWITCH_HOST_PACK = range(11)
+SWITCH_ALL_TC, SWITCH_ENV_MULTISTEP, SWITCH_HOST_PACK = 5, 9, 10
 
 _lib = None
 
@@ -166,7 +165,7 @@ def check(code):
 
 
 def set_kernel_switch(which: int, enabled: bool) -> None:
-    """A/B and debugging control of the kernel families (d2d_set_kernel_switch); process-wide."""
+    """A/B and debugging control of the SWITCH_* paths (d2d_set_kernel_switch); process-wide."""
     check(lib().d2d_set_kernel_switch(int(which), int(bool(enabled))))
 
 

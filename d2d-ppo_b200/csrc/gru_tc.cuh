@@ -186,28 +186,25 @@ struct Smem {
   static constexpr int kAx = kM * kKx;
   static constexpr size_t bytes = (size_t)(2 * kWih + 2 * kWhh + 2 * 2 * kAh + 2 * kAx) * 2 + 4 * H * 4 + 64;
   // fused head: W1 planes [2][H][H] fp16, then fp32: b1 [H], W2^T [H][OMAX], b2 [OMAX], partial sums [2 slots][128][OMAX]
-  static constexpr size_t head_bytes(int omax, int q = 2) {
-    return (size_t)2 * H * H * 2 + (size_t)(H + H * omax + omax + (q - 1) * 2 * kM * omax) * 4 + 16;
+  static constexpr size_t head_bytes(int omax) {
+    return (size_t)2 * H * H * 2 + (size_t)(H + H * omax + omax + 2 * kM * omax) * 4 + 16;
   }
 };
 
 }  // namespace tc
 
 // STORE: the training direction (a.store); compile time so that the rollout kernel carries none of the store code.
-// 1: h and the gates (r, z, n, gh_n) of every step are kept (BPTT kernels that read them: recompute switched off);
-// 2: only h is kept (the recomputing BPTT kernel) and the gate maths takes the rollout's shared-reciprocal form.
+// 1: h and the gates (r, z, n, gh_n) of every step are kept (H 16 / 48: the FP32 gate backward reads them);
+// 2: only h is kept (H 32 / 64: the recomputing BPTT kernel) and the gate maths takes the rollout's shared-reciprocal
+// form.
 // OMAX > 0: the network head is fused behind the last step -- Linear(H, H) as one more
 // two-plane GEMM on the h planes the step already staged (12 MMAs), ReLU and Linear(H, O <= OMAX) on the CUDA cores from
 // TMEM, the two unit halves of a row combined through shared memory -- and the kernel writes the O pre-activation
 // outputs instead of h_last: no head kernel, no h_last round trip through HBM.
-// Q: threads per row (each owns H / Q hidden units).  Q = 2: 16 warps of 128 registers.  Q = 4: 32 warps of 64
-// registers -- four instead of two warps per scheduler are in a slot's gate phase, which is latency bound (dependent
-// MUFU / FMA chains at an IPC of ~0.5 per scheduler with two warps).
-template <int H, int STORE, int OMAX = 0, int Q = 2>
-__global__ void __launch_bounds__(256 * Q, 1) gru_window_tc_kernel(const GruTcArgs a) {
+template <int H, int STORE, int OMAX = 0>
+__global__ void __launch_bounds__(tc::kThreads, 1) gru_window_tc_kernel(const GruTcArgs a) {
   using namespace tc;
   using S = Smem<H>;
-  constexpr int kThreads = 256 * Q, kGateThreads = 128 * Q;   // shadow the namespace constants (Q = 2 values)
   static_assert(H % 16 == 0 && H >= 16 && H <= 64, "H in {16, 32, 48, 64}");
   extern __shared__ __align__(1024) uint8_t smem_raw[];
   __half* wih = reinterpret_cast<__half*>(smem_raw);                    // [2 planes][4H][kKx], rows [r; z; 0; n]
@@ -296,12 +293,12 @@ __global__ void __launch_bounds__(256 * Q, 1) gru_window_tc_kernel(const GruTcAr
   const int n_pairs = (a.t1 - a.t0) * pairs_per_t;
 
   {
-    // =================== gate warps: slot = warp / 4Q, lane quadrant = warp % 4, unit part = (warp / 4) % Q ====
-    constexpr int HH = H / Q;          // hidden units per thread
-    constexpr int KH = kKx / Q;        // input features staged per thread
+    // =================== gate warps: slot = warp / 8, lane quadrant = warp % 4, unit half = (warp / 4) % 2 ====
+    constexpr int HH = H / 2;          // hidden units per thread
+    constexpr int KH = kKx / 2;        // input features staged per thread
     static_assert(HH % 8 == 0 && KH % 8 == 0, "units / features per thread in groups of 8");
-    const int slot = warp / (4 * Q);
-    const int half = (warp >> 2) % Q;
+    const int slot = warp / 8;
+    const int half = (warp >> 2) % 2;
     const int row = ((warp & 3) << 5) + lane;
     const uint32_t lane_addr = (uint32_t)((warp & 3) << 5) << 16;
     __half* my_ax = ax + slot * S::kAx;
@@ -409,7 +406,6 @@ __global__ void __launch_bounds__(256 * Q, 1) gru_window_tc_kernel(const GruTcAr
         ph ^= 1u;
         asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
         const uint32_t d = tmem + (uint32_t)slot * (4 * H) + lane_addr + (uint32_t)u0;
-        const bool first = s == s0;
         float* acts_row = nullptr;
         float* hs_row = nullptr;
         if (STORE && b < a.B) {   // acts.p == nullptr: only h is kept (the recomputing BPTT kernel, gru_bptt_tc.cuh)
@@ -505,19 +501,16 @@ __global__ void __launch_bounds__(256 * Q, 1) gru_window_tc_kernel(const GruTcAr
               for (int o = 0; o < OP; ++o) po[o] = fmaf(w2t[u * OP + o], yv, po[o]);
             }
           }
-          // the row's Q unit parts live in different warps: parts 1 .. Q - 1 hand their partial sums over through smem
+          // the row's two unit halves live in different warps: half 1 hands its partial sums to half 0 through smem
           float* pp = part + ((size_t)slot * kM + row) * OP;
-          if (half > 0) {
-            float* mine = pp + (size_t)(half - 1) * 2 * kM * OP;
+          if (half == 1) {
 #pragma unroll
-            for (int o = 0; o < OP; ++o) mine[o] = po[o];
+            for (int o = 0; o < OP; ++o) pp[o] = po[o];
           }
           asm volatile("bar.sync %0, %1;" ::"r"(1 + slot), "r"(kGateThreads) : "memory");
           if (half == 0 && b < a.B) {
 #pragma unroll
-            for (int q = 0; q < Q - 1; ++q)
-#pragma unroll
-              for (int o = 0; o < OP; ++o) po[o] += pp[(size_t)q * 2 * kM * OP + o];
+            for (int o = 0; o < OP; ++o) po[o] += pp[o];
 #pragma unroll
             for (int o = 0; o < OP; ++o) po[o] += b2s[o];
             if (a.out.p) {

@@ -60,25 +60,37 @@ static View make_view(float* p, long long t_stride, int t_off, int N, int feat_p
   return v;
 }
 
-// Kernel-family switches (d2d_set_kernel_switch in the C ABI): an A/B and debugging control set explicitly by the
-// caller -- the library reads no environment variables.  A family that is switched off runs on its FP32 CUDA-core
-// kernel.  Not thread-safe; set before the first launch.
-enum { kSwGruTc = D2D_SWITCH_GRU_WINDOW_TC, kSwBwdTc = D2D_SWITCH_GRU_BPTT_TC, kSwDenseTc = D2D_SWITCH_DENSE_TC,
-       kSwWgradTc = D2D_SWITCH_WGRAD_TC, kSwFusedHead = D2D_SWITCH_FUSED_HEAD, kSwAllTc = D2D_SWITCH_ALL_TC,
-       kSwBpttRecompute = D2D_SWITCH_BPTT_RECOMPUTE, kSwWindowHead = D2D_SWITCH_WINDOW_HEAD,
-       kSwWindowWide = D2D_SWITCH_WINDOW_WIDE, kSwEnvMultistep = D2D_SWITCH_ENV_MULTISTEP,
-       kSwHostPack = D2D_SWITCH_HOST_PACK, kSwCount };
-static int g_switch_off[kSwCount] = {0, 0, 0, 0, 0, 0, 0, 0, 1, 0, 0};   // the 32-warp window variant is opt-in (measured slower)
-static bool switched_off(int which) { return g_switch_off[which] != 0; }
-static bool tc_enabled() { return g_switch_off[kSwAllTc] == 0; }
+// the observations: agent g's features are rows in_off[g] ... of each time block; time block t is x_lead blocks in
+static View input_view(const d2d_net* n, const float* x, int x_lead) {
+  View v;
+  memset(&v, 0, sizeof(v));
+  v.p = const_cast<float*>(x), v.t_stride = (long long)n->in_rows * n->B, v.t_off = x_lead;
+  for (int g = 0; g < n->N; ++g) v.f_off[g] = n->in_off[g];
+  return v;
+}
+
+// Kernel switches (d2d_set_kernel_switch in the C ABI): an A/B and debugging control set explicitly by the caller --
+// the library reads no environment variables.  Not thread-safe; set before the first launch.
+static int g_all_tc = 1, g_env_multistep = 1, g_host_pack = 1;
+static int* switch_ptr(int which) {
+  switch (which) {
+    case D2D_SWITCH_ALL_TC: return &g_all_tc;
+    case D2D_SWITCH_ENV_MULTISTEP: return &g_env_multistep;
+    case D2D_SWITCH_HOST_PACK: return &g_host_pack;
+    default: return nullptr;
+  }
+}
+static bool tc_enabled() { return g_all_tc != 0; }
 
 extern "C" int d2d_set_kernel_switch(int which, int enabled) {
-  D2D_REQUIRE(which >= 0 && which < kSwCount, "d2d_set_kernel_switch: unknown kernel family %d", which);
-  g_switch_off[which] = enabled ? 0 : 1;
+  int* sw = switch_ptr(which);
+  D2D_REQUIRE(sw, "d2d_set_kernel_switch: unknown switch %d", which);
+  *sw = enabled ? 1 : 0;
   return D2D_OK;
 }
 extern "C" int d2d_get_kernel_switch(int which) {
-  return (which >= 0 && which < kSwCount) ? (g_switch_off[which] ? 0 : 1) : D2D_ERR_INVALID;
+  const int* sw = switch_ptr(which);
+  return sw ? *sw : D2D_ERR_INVALID;
 }
 
 template <int RPT, int OPT>
@@ -148,7 +160,7 @@ static int launch_dense(const d2d_net* n, DenseArgs& a, int max_in, cudaStream_t
   }
   // tensor-core path (dense_tc.cuh) for single-chunk reductions (K <= 64); with K = 3H the three stage -> MMA round
   // trips per tile serialise inside a slot and the register-tiled FP32 kernel is faster (measured 212 vs 480 us)
-  if (tc_enabled() && !switched_off(kSwDenseTc) && n->B >= 256 && a.out_dim <= 192 && max_in <= tcd::kKc &&
+  if (tc_enabled() && n->B >= 256 && a.out_dim <= 192 && max_in <= tcd::kKc &&
       tcd::smem_bytes(max_in, a.out_dim) <= 225 * 1024) {
     static bool attr = false;
     if (!attr) {
@@ -223,6 +235,32 @@ static void launch_wgrad_t(const WgradArgs& a, dim3 grid, cudaStream_t s) {
   wgrad_kernel<TO, TK><<<grid, 256, smem, s>>>(a);
 }
 
+// row length of the gradient of `w` per agent (zero_in: the input was zero, only the bias gradient is taken)
+static int wgrad_in_dims(const d2d_net* n, const Wt& w, bool zero_in, int* in_dim) {
+  int maxK = 0;
+  for (int g = 0; g < n->N; ++g) {
+    in_dim[g] = zero_in ? 0 : (w.in_dim ? (*w.in_dim)[g] : w.in_const);
+    maxK = std::max(maxK, in_dim[g]);
+  }
+  return maxK;
+}
+
+// dW (+ db) of `w` += the fixed-order sum of the `strips` per-CTA partial sums in n->partial
+static int launch_wreduce(const d2d_net* n, const Wt& w, bool zero_in, int strips, float* grads, cudaStream_t s) {
+  WreduceArgs r;
+  memset(&r, 0, sizeof(r));
+  r.partial = n->partial, r.part_stride = n->part_stride, r.n_strips = strips, r.grads = grads;
+  r.g_agent_stride = n->stride, r.out_dim = w.out_dim, r.with_bias = w.b_off != nullptr;
+  for (int g = 0; g < n->N; ++g) {
+    r.w_off[g] = (*w.w_off)[g];
+    r.b_off[g] = w.b_off ? (*w.b_off)[g] : 0;
+  }
+  const int total = w.out_dim * wgrad_in_dims(n, w, zero_in, r.in_dim) + w.out_dim;
+  wreduce_kernel<<<dim3((total + 255) / 256, n->N), 256, 0, s>>>(r);
+  D2D_LAUNCHED();
+  return D2D_OK;
+}
+
 // dW (+ db) of `w` from dy [out_dim] and x [K]; accumulated into grads
 static int launch_wgrad(d2d_net* n, const View& dy, const View& x, const Wt& w, bool zero_in, float* grads, int t0,
                         int t1, cudaStream_t s, bool x_is_input = false) {
@@ -231,11 +269,7 @@ static int launch_wgrad(d2d_net* n, const View& dy, const View& x, const Wt& w, 
   a.x_planes = (x_is_input && n->x_exact) ? 1 : 0;   // x = the observations, exact in bf16 by the caller's promise
   a.dy = dy, a.x = x, a.partial = n->partial, a.part_stride = n->part_stride;
   a.out_dim = w.out_dim, a.B = n->B, a.t0 = t0, a.t1 = t1, a.with_bias = w.b_off != nullptr;
-  int maxK = 0;
-  for (int g = 0; g < n->N; ++g) {
-    a.in_dim[g] = zero_in ? 0 : (w.in_dim ? (*w.in_dim)[g] : w.in_const);
-    maxK = std::max(maxK, a.in_dim[g]);
-  }
+  const int maxK = wgrad_in_dims(n, w, zero_in, a.in_dim);
   int strips = n->n_strips;
   const int O = w.out_dim;
   if (maxK > 128) {
@@ -261,7 +295,7 @@ static int launch_wgrad(d2d_net* n, const View& dy, const View& x, const Wt& w, 
     }
     return D2D_OK;
   }
-  if (tc_enabled() && !switched_off(kSwWgradTc) && n->B % 8 == 0) {
+  if (tc_enabled() && n->B % 8 == 0) {
     // tensor-core path (wgrad_tc.cuh): bf16 x 3 planes on tcgen05, accumulators in TMEM
     const size_t smem = tcw::smem_bytes(maxK);
     static bool attr = false;
@@ -280,19 +314,7 @@ static int launch_wgrad(d2d_net* n, const View& dy, const View& x, const Wt& w, 
 #undef WG
   }
   D2D_LAUNCHED();
-  WreduceArgs r;
-  memset(&r, 0, sizeof(r));
-  r.partial = n->partial, r.part_stride = n->part_stride, r.n_strips = strips, r.grads = grads;
-  r.g_agent_stride = n->stride, r.out_dim = O, r.with_bias = a.with_bias;
-  for (int g = 0; g < n->N; ++g) {
-    r.w_off[g] = (*w.w_off)[g];
-    r.b_off[g] = w.b_off ? (*w.b_off)[g] : 0;
-    r.in_dim[g] = a.in_dim[g];
-  }
-  const int total = O * maxK + O;
-  wreduce_kernel<<<dim3((total + 255) / 256, n->N), 256, 0, s>>>(r);
-  D2D_LAUNCHED();
-  return D2D_OK;
+  return launch_wreduce(n, w, zero_in, strips, grads, s);
 }
 
 // fused hidden projection + gates (B % 4 == 0)
@@ -319,93 +341,88 @@ static int launch_gru_step(const d2d_net* n, GruStepArgs& a, const float* params
   return D2D_OK;
 }
 
-// tensor-core fused GRU window (gru_tc.cuh): x windows -> last hidden state, no intermediate in HBM
-static bool gru_tc_eligible(const d2d_net* n) {
-  return tc_enabled() && !switched_off(kSwGruTc) && n->arch == D2D_NET_GRU && n->x_exact && n->max_in <= tc::kKx &&
-         (n->H == 16 || n->H == 32 || n->H == 48 || n->H == 64);
+// Which kernels a call on the net runs.  It depends on the net's shape and D2D_SWITCH_ALL_TC only, and is evaluated
+// per call (plan_chunk keeps it in Chunk::plan) because the switch may change between calls on the same net: the
+// scratch layout and the launches all read this one decision.
+enum class Bptt { kFp32, kRecompute, kStoredTc };
+enum class Head { kDense, kKernel, kWindow };
+struct Plan {
+  bool window_tc;   // GRU forward on the tcgen05 window kernel (gru_tc.cuh); else input projection + FP32 step kernels
+  Bptt bptt;        // kRecompute: gru_bptt_tc recomputes the gates, the forward keeps h only; kStoredTc: gru_bwd_tc
+                    // reads the gates the forward stored; kFp32: gate kernels + FP32 GEMMs on the stored gates
+  Head head;        // kWindow: fused behind the window kernel; kKernel: head_fused_kernel; kDense: dense kernels
+};
+
+static Plan make_plan(const d2d_net* n) {
+  const bool gru = n->arch == D2D_NET_GRU, all_tc = tc_enabled(), h32_64 = n->H == 32 || n->H == 64;
+  Plan p;
+  // the window stages the inputs as one fp16 plane (integer observations, the caller's promise) with I <= 32
+  p.window_tc = all_tc && gru && n->x_exact && n->max_in <= tc::kKx && (h32_64 || n->H == 16 || n->H == 48);
+  p.bptt = !(all_tc && gru && h32_64) ? Bptt::kFp32 : (p.window_tc ? Bptt::kRecompute : Bptt::kStoredTc);
+  const bool head_fused = gru && h32_64 && n->O <= 16 && !n->head2;
+  p.head = !head_fused ? Head::kDense : (p.window_tc ? Head::kWindow : Head::kKernel);
+  return p;
 }
 
-template <int H, int STORE, int OMAX, int Q>
-static int launch_gru_tc_q(const d2d_net* n, const GruTcArgs& a, cudaStream_t s) {
+template <int H, int STORE, int OMAX>
+static int launch_gru_tc_k(const d2d_net* n, const GruTcArgs& a, cudaStream_t s) {
   const size_t smem =
-      OMAX > 0 ? ((tc::Smem<H>::bytes + 15) & ~(size_t)15) + tc::Smem<H>::head_bytes(OMAX, Q) : tc::Smem<H>::bytes;
+      OMAX > 0 ? ((tc::Smem<H>::bytes + 15) & ~(size_t)15) + tc::Smem<H>::head_bytes(OMAX) : tc::Smem<H>::bytes;
   static bool attr = false;
   if (!attr) {
-    D2D_CUDA(cudaFuncSetAttribute(gru_window_tc_kernel<H, STORE, OMAX, Q>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+    D2D_CUDA(cudaFuncSetAttribute(gru_window_tc_kernel<H, STORE, OMAX>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                   (int)smem));
     attr = true;
   }
   const int pairs = (a.t1 - a.t0) * ((n->B + 2 * tc::kM - 1) / (2 * tc::kM));
   if (pairs <= 0) return D2D_OK;
   const int gx = std::max(1, std::min(pairs, 148 / n->N));   // one CTA per SM (all of its shared memory and TMEM)
-  gru_window_tc_kernel<H, STORE, OMAX, Q><<<dim3(gx, n->N), 256 * Q, smem, s>>>(a);
+  gru_window_tc_kernel<H, STORE, OMAX><<<dim3(gx, n->N), tc::kThreads, smem, s>>>(a);
   D2D_LAUNCHED();
   return D2D_OK;
 }
 
-template <int H, int STORE, int OMAX>
-static int launch_gru_tc_hs(const d2d_net* n, const GruTcArgs& a, cudaStream_t s) {
-  // two threads per row (16 warps of 128 registers).  The four-threads-per-row variant (32 warps of 64 registers, more
-  // warps per scheduler in the latency-bound gate phase) is kept behind D2D_SWITCH_WINDOW_WIDE: measured SLOWER on
-  // B200 (rollout 3.81e8 vs 4.52e8 agent-steps/s, epoch 61 vs 55 ms): at 64 registers ptxas spills 100-500 bytes per
-  // thread and the extra tcgen05.ld / staging instructions outweigh the added warps
-  if constexpr ((H == 32 || H == 64) && OMAX <= 8) {
-    if (!switched_off(kSwWindowWide)) return launch_gru_tc_q<H, STORE, OMAX, 4>(n, a, s);
-  }
-  return launch_gru_tc_q<H, STORE, OMAX, 2>(n, a, s);
-}
-
+// Only the instantiations a plan reaches: H 32 / 64 train for the recomputing BPTT (STORE 2: h only) and may have the
+// head fused (OMAX > 0); H 16 / 48 train for the FP32 gate backward (STORE 1: h and the gates), their head runs apart.
 template <int H>
 static int launch_gru_tc_h(const d2d_net* n, const GruTcArgs& a, cudaStream_t s, bool head) {
+  constexpr int kStore = (H == 32 || H == 64) ? 2 : 1;
   if constexpr (H == 32 || H == 64) {
-    if (head && a.store && a.acts.p) {   // gates kept for a BPTT kernel that reads them
-      if (a.O <= 1) return launch_gru_tc_hs<H, 1, 1>(n, a, s);
-      if (a.O <= 8) return launch_gru_tc_hs<H, 1, 8>(n, a, s);
-      return launch_gru_tc_hs<H, 1, 16>(n, a, s);
-    }
-    if (head && a.store) {               // only h kept (recomputing BPTT kernel)
-      if (a.O <= 1) return launch_gru_tc_hs<H, 2, 1>(n, a, s);
-      if (a.O <= 8) return launch_gru_tc_hs<H, 2, 8>(n, a, s);
-      return launch_gru_tc_hs<H, 2, 16>(n, a, s);
-    }
     if (head) {
-      if (a.O <= 1) return launch_gru_tc_hs<H, 0, 1>(n, a, s);
-      if (a.O <= 8) return launch_gru_tc_hs<H, 0, 8>(n, a, s);
-      return launch_gru_tc_hs<H, 0, 16>(n, a, s);
+      if (a.O <= 1) return a.store ? launch_gru_tc_k<H, kStore, 1>(n, a, s) : launch_gru_tc_k<H, 0, 1>(n, a, s);
+      if (a.O <= 8) return a.store ? launch_gru_tc_k<H, kStore, 8>(n, a, s) : launch_gru_tc_k<H, 0, 8>(n, a, s);
+      return a.store ? launch_gru_tc_k<H, kStore, 16>(n, a, s) : launch_gru_tc_k<H, 0, 16>(n, a, s);
     }
   }
-  if (a.store && a.acts.p) return launch_gru_tc_hs<H, 1, 0>(n, a, s);
-  if (a.store) return launch_gru_tc_hs<H, 2, 0>(n, a, s);
-  return launch_gru_tc_hs<H, 0, 0>(n, a, s);
+  return a.store ? launch_gru_tc_k<H, kStore, 0>(n, a, s) : launch_gru_tc_k<H, 0, 0>(n, a, s);
 }
 
-static bool head_fused_eligible(const d2d_net* n);
-
-// head_out != nullptr (inference direction): the network head is fused behind the window and *head_out receives the
-// pre-activation outputs; h_out is then not written
+// tensor-core fused GRU window (gru_tc.cuh): x windows -> last hidden state in h_out, no intermediate in HBM.
+// hs != nullptr (training): h of every step goes to *hs instead, the L steps hs_step floats apart, and the gates to
+// *acts (4 hs_step apart) unless acts->p is null.  out != nullptr: the network head is fused behind the window and
+// *out receives the pre-activation outputs (out->p == nullptr: not written), *y1 relu(W1 h + b1) if given; sel turns
+// the outputs into actions and log-probs.
 static int launch_gru_tc(const d2d_net* n, const float* params, const View& x, const View& h_out, int t0, int t1,
-                         int padded, cudaStream_t s, const View* acts = nullptr, const View* hs = nullptr,
-                         long long acts_step = 0, long long hs_step = 0, const View* head_out = nullptr,
-                         const View* y1_out = nullptr, const DistArgs* sel = nullptr) {
+                         int padded, cudaStream_t s, const View* hs, const View* acts, long long hs_step,
+                         const View* out, const View* y1, const DistArgs* sel) {
   GruTcArgs a;
   memset(&a, 0, sizeof(a));
   a.x = x, a.h_out = h_out, a.w = params, a.w_agent_stride = n->stride;
-  if (hs) a.store = 1, a.acts = *acts, a.hs = *hs, a.acts_step = acts_step, a.hs_step = hs_step;
+  if (hs) a.store = 1, a.acts = *acts, a.hs = *hs, a.acts_step = 4 * hs_step, a.hs_step = hs_step;
   for (int g = 0; g < n->N; ++g) {
     a.wih_off[g] = n->o_wih[g], a.whh_off[g] = n->o_whh[g], a.bih_off[g] = n->o_bih[g], a.bhh_off[g] = n->o_bhh[g];
     a.in_dim[g] = n->in_dim[g];
     a.w1_off[g] = n->o_w1[g], a.b1_off[g] = n->o_b1[g], a.w2_off[g] = n->o_w2[g], a.b2_off[g] = n->o_b2[g];
   }
   a.L = n->L, a.B = n->B, a.t0 = t0, a.t1 = t1, a.padded = padded, a.O = n->O;
-  const bool head = head_out != nullptr;
-  if (head) a.out = *head_out;
+  if (out) a.out = *out;
+  if (y1) a.y1 = *y1;
   if (sel) a.sel = *sel;
-  if (y1_out) a.y1 = *y1_out;
   switch (n->H) {
     case 16: return launch_gru_tc_h<16>(n, a, s, false);
-    case 32: return launch_gru_tc_h<32>(n, a, s, head);
+    case 32: return launch_gru_tc_h<32>(n, a, s, out != nullptr);
     case 48: return launch_gru_tc_h<48>(n, a, s, false);
-    default: return launch_gru_tc_h<64>(n, a, s, head);
+    default: return launch_gru_tc_h<64>(n, a, s, out != nullptr);
   }
 }
 
@@ -415,10 +432,6 @@ static void launch_head_fused_t(const HeadFusedArgs& a, int N, int tiles, cudaSt
   const int gx = std::max(1, std::min(tiles, (148 * 2) / N));
   if (a.y1.p) head_fused_kernel<H, OMAX, true><<<dim3(gx, N), kHeadThreads, 0, s>>>(a);
   else head_fused_kernel<H, OMAX, false><<<dim3(gx, N), kHeadThreads, 0, s>>>(a);
-}
-
-static bool head_fused_eligible(const d2d_net* n) {
-  return !switched_off(kSwFusedHead) && n->arch == D2D_NET_GRU && (n->H == 32 || n->H == 64) && n->O <= 16 && !n->head2;
 }
 
 static int launch_head_fused(const d2d_net* n, const float* params, const View& h, float* y1, const View& out, int t0,
@@ -438,18 +451,6 @@ static int launch_head_fused(const d2d_net* n, const float* params, const View& 
 #undef HF
   D2D_LAUNCHED();
   return D2D_OK;
-}
-
-// tensor-core fused BPTT through the window (gru_bwd_tc.cuh)
-static bool gru_bwd_tc_eligible(const d2d_net* n) {
-  return tc_enabled() && !switched_off(kSwBwdTc) && n->arch == D2D_NET_GRU && (n->H == 32 || n->H == 64) && n->L >= 1;
-}
-static bool gru_tc_eligible(const d2d_net* n);
-
-// recomputing BPTT (gru_bptt_tc.cuh): needs the inputs exact in one fp16 plane (integer observations) and I <= 32;
-// then the forward kernel keeps only h of every step
-static bool gru_bptt_recompute_eligible(const d2d_net* n) {
-  return gru_bwd_tc_eligible(n) && gru_tc_eligible(n) && !switched_off(kSwBpttRecompute);
 }
 
 template <int H>
@@ -501,17 +502,18 @@ static int launch_gate(const GateArgs& a, int N, bool bwd, cudaStream_t s) {
 // ------------------------------------------------------------------------------------------------
 struct Chunk {
   int Tc, halo;
+  Plan plan;
   float *gi, *gh, *acts, *hs, *y1, *y2, *logits, *dl, *dy1, *dy2, *dh0, *dh1, *dgi;
 };
 
-static long long floats_per_t(const d2d_net* n, bool train) {
+static long long floats_per_t(const d2d_net* n, bool train, const Plan& plan) {
   const long long NB = (long long)n->N * n->B;
   const long long H = n->H, O = n->O, L = n->arch == D2D_NET_GRU ? n->L : 0;
   long long f = H + O;                                // y1, logits
   if (n->head2) f += train ? 2 * H : H;               // y2 (+ dy2)
   if (n->arch == D2D_NET_GRU) f += 3 * H + 3 * H;     // gi, gh
   // hs of every step; the 4H activations per step only for the BPTT kernels that do not recompute them
-  if (n->arch == D2D_NET_GRU) f += train ? L * H + (gru_bptt_recompute_eligible(n) ? 0 : 4 * L * H) : 2 * H;
+  if (n->arch == D2D_NET_GRU) f += train ? L * H + (plan.bptt == Bptt::kRecompute ? 0 : 4 * L * H) : 2 * H;
   if (train) f += O + H;                              // dl, dy1
   if (train && n->arch == D2D_NET_GRU) f += 2 * H + 3 * H;   // dh ping-pong, dgi
   return f * NB;
@@ -520,7 +522,8 @@ static long long floats_per_t(const d2d_net* n, bool train) {
 static int plan_chunk(d2d_net* n, bool train, int n_t, Chunk& c) {
   const long long NB = (long long)n->N * n->B;
   const int halo = n->arch == D2D_NET_GRU ? n->L - 1 : 0;
-  const long long per_t = floats_per_t(n, train);
+  c.plan = make_plan(n);
+  const long long per_t = floats_per_t(n, train, c.plan);
   const long long halo_f = (long long)halo * 3 * n->H * NB * (train ? 2 : 1);
   long long budget = n->scratch_bytes / 4;
   int Tc = (int)std::max<long long>(1, std::min<long long>(n_t, (budget - halo_f) / per_t));
@@ -541,7 +544,7 @@ static int plan_chunk(d2d_net* n, bool train, int n_t, Chunk& c) {
     c.gh = take((long long)Tc * 3 * H * NB);
     if (train) {
       c.hs = take((long long)L * Tc * H * NB);
-      if (!gru_bptt_recompute_eligible(n)) c.acts = take((long long)L * Tc * 4 * H * NB);
+      if (c.plan.bptt != Bptt::kRecompute) c.acts = take((long long)L * Tc * 4 * H * NB);
     } else {
       c.hs = take((long long)2 * Tc * H * NB);
     }
@@ -607,86 +610,67 @@ static int forward_chunk(d2d_net* n, const float* params, const float* x, int x_
                          bool train, const Chunk& c, cudaStream_t s) {
   const int N = n->N, B = n->B, H = n->H, O = n->O;
   const long long NB = (long long)N * B;
-  View xin;
-  memset(&xin, 0, sizeof(xin));
-  xin.p = const_cast<float*>(x), xin.t_stride = (long long)n->in_rows * B, xin.t_off = x_lead;
-  for (int g = 0; g < N; ++g) xin.f_off[g] = n->in_off[g];
+  const View xin = input_view(n, x, x_lead);
   const View y1 = make_view(c.y1, H * NB, -c0, N, H, B);
   const View lg = make_view(c.logits, O * NB, -c0, N, O, B);
-  Wt w1{&n->o_w1, &n->o_b1, nullptr, H, H};
-  Wt w2{&n->o_w2, &n->o_b2, nullptr, H, O};
   int rc;
-  View last;
-  if (n->arch == D2D_NET_MLP) {
-    w1.in_dim = &n->in_dim;
-    last = xin;
-  } else {
+  View last = xin;
+  if (n->arch == D2D_NET_GRU) {
     const int L = n->L, halo = c.halo;
-    // tcgen05 fused window (gru_tc.cuh); training windows are always padded and keep every step's activations
-    const bool use_tc = gru_tc_eligible(n) && (!train || padded);
-    if (use_tc) {
+    if (c.plan.window_tc) {   // tcgen05 fused window (gru_tc.cuh); training windows are padded and keep every step's h
+      const bool head = c.plan.head == Head::kWindow;   // window + head (+ y1 when training) in one launch
       const View hl = make_view(hs_ptr(n, c, train, L - 1), H * NB, -c0, N, H, B);
-      if (train) {
-        View av = make_view(c.acts, 4 * H * NB, -c0, N, 4 * H, B);
-        if (!c.acts) av.p = nullptr;          // the recomputing BPTT kernel needs h only
-        const View hv = make_view(c.hs, H * NB, -c0, N, H, B);
-        if (head_fused_eligible(n) && !switched_off(kSwWindowHead))   // window + head + y1 in one launch
-          return launch_gru_tc(n, params, xin, hl, c0, c1, padded, s, &av, &hv, (long long)c.Tc * 4 * H * NB,
-                               (long long)c.Tc * H * NB, &lg, &y1);
-        rc = launch_gru_tc(n, params, xin, hl, c0, c1, padded, s, &av, &hv, (long long)c.Tc * 4 * H * NB,
-                           (long long)c.Tc * H * NB);
-      } else if (head_fused_eligible(n) && !switched_off(kSwWindowHead)) {
-        // inference direction: the head is fused behind the window, the kernel writes the outputs directly
-        return launch_gru_tc(n, params, xin, hl, c0, c1, padded, s, nullptr, nullptr, 0, 0, &lg);
-      } else {
-        rc = launch_gru_tc(n, params, xin, hl, c0, c1, padded, s);
-      }
-      if (rc) return rc;
-    }
-    // input projections of every observation the chunk's windows touch: times [c0 - halo, c1)
-    const View gi = make_view(c.gi, 3 * H * NB, -(c0 - halo), N, 3 * H, B);
-    if (!use_tc) {
-      DenseArgs a;
-      memset(&a, 0, sizeof(a));
-      Wt wih{&n->o_wih, &n->o_bih, &n->in_dim, 0, 3 * H};
-      fill_dense_w(n, a, params, wih, 0);
-      a.x = xin, a.y = gi, a.epilogue = kEpiNone, a.t0 = c0 - halo, a.t1 = c1;
-      if ((rc = launch_dense(n, a, n->max_in, s, n->x_exact))) return rc;
-    }
-    const View gh = make_view(c.gh, 3 * H * NB, -c0, N, 3 * H, B);
-    for (int st = 0; st < L && !use_tc; ++st) {
-      const View hprev = make_view(hs_ptr(n, c, train, st - 1 < 0 ? 0 : st - 1), H * NB, -c0, N, H, B);
-      const View hout = make_view(hs_ptr(n, c, train, st), H * NB, -c0, N, H, B);
-      if (B % 4 == 0 && H <= 128) {   // fused hidden projection + gates (a register tile covers 64 units; H > 64: 2 launches)
-        GruStepArgs fa;
-        memset(&fa, 0, sizeof(fa));
-        fa.h_prev = hprev, fa.h_out = hout, fa.gi = gi, fa.gi.t_off = gi.t_off - (L - 1 - st);
-        if (train) fa.acts = make_view(c.acts + (long long)st * c.Tc * 4 * H * NB, 4 * H * NB, -c0, N, 4 * H, B);
-        fa.t0 = c0, fa.t1 = c1, fa.back = L - 1 - st, fa.padded = padded, fa.first = st == 0, fa.store = train;
-        if ((rc = launch_gru_step(n, fa, params, s))) return rc;
-        continue;
-      }
+      const View hv = make_view(c.hs, H * NB, -c0, N, H, B);
+      const View av = make_view(c.acts, 4 * H * NB, -c0, N, 4 * H, B);   // c.acts null: the BPTT recomputes the gates
+      rc = launch_gru_tc(n, params, xin, hl, c0, c1, padded, s, train ? &hv : nullptr, train ? &av : nullptr,
+                         (long long)c.Tc * H * NB, head ? &lg : nullptr, head && train ? &y1 : nullptr, nullptr);
+      if (rc || head) return rc;
+    } else {
+      // input projections of every observation the chunk's windows touch: times [c0 - halo, c1)
+      const View gi = make_view(c.gi, 3 * H * NB, -(c0 - halo), N, 3 * H, B);
       {
         DenseArgs a;
         memset(&a, 0, sizeof(a));
-        Wt whh{&n->o_whh, &n->o_bhh, nullptr, st == 0 ? 0 : H, 3 * H};   // step 0: h = 0, gh = b_hh
-        fill_dense_w(n, a, params, whh, 0);
-        for (int g = 0; g < N; ++g) a.w_ld[g] = H;
-        a.x = hprev, a.y = gh, a.epilogue = kEpiNone, a.t0 = c0, a.t1 = c1;
-        if ((rc = launch_dense(n, a, H, s))) return rc;
+        Wt wih{&n->o_wih, &n->o_bih, &n->in_dim, 0, 3 * H};
+        fill_dense_w(n, a, params, wih, 0);
+        a.x = xin, a.y = gi, a.epilogue = kEpiNone, a.t0 = c0 - halo, a.t1 = c1;
+        if ((rc = launch_dense(n, a, n->max_in, s, n->x_exact))) return rc;
       }
-      GateArgs ga;
-      memset(&ga, 0, sizeof(ga));
-      ga.gi = gi, ga.gi.t_off = gi.t_off - (L - 1 - st);
-      ga.gh = gh, ga.h_prev = hprev, ga.h_out = hout;
-      if (train) ga.acts = make_view(c.acts + (long long)st * c.Tc * 4 * H * NB, 4 * H * NB, -c0, N, 4 * H, B);
-      ga.H = H, ga.B = B, ga.t0 = c0, ga.t1 = c1, ga.back = L - 1 - st, ga.padded = padded, ga.first = st == 0;
-      ga.store = train, ga.t_episode0 = 0;
-      if ((rc = launch_gate(ga, N, false, s))) return rc;
+      const View gh = make_view(c.gh, 3 * H * NB, -c0, N, 3 * H, B);
+      for (int st = 0; st < L; ++st) {
+        const View hprev = make_view(hs_ptr(n, c, train, st - 1 < 0 ? 0 : st - 1), H * NB, -c0, N, H, B);
+        const View hout = make_view(hs_ptr(n, c, train, st), H * NB, -c0, N, H, B);
+        if (B % 4 == 0 && H <= 128) {   // fused hidden projection + gates (a register tile covers 64 units; H > 64: 2 launches)
+          GruStepArgs fa;
+          memset(&fa, 0, sizeof(fa));
+          fa.h_prev = hprev, fa.h_out = hout, fa.gi = gi, fa.gi.t_off = gi.t_off - (L - 1 - st);
+          if (train) fa.acts = make_view(c.acts + (long long)st * c.Tc * 4 * H * NB, 4 * H * NB, -c0, N, 4 * H, B);
+          fa.t0 = c0, fa.t1 = c1, fa.back = L - 1 - st, fa.padded = padded, fa.first = st == 0, fa.store = train;
+          if ((rc = launch_gru_step(n, fa, params, s))) return rc;
+          continue;
+        }
+        {
+          DenseArgs a;
+          memset(&a, 0, sizeof(a));
+          Wt whh{&n->o_whh, &n->o_bhh, nullptr, st == 0 ? 0 : H, 3 * H};   // step 0: h = 0, gh = b_hh
+          fill_dense_w(n, a, params, whh, 0);
+          for (int g = 0; g < N; ++g) a.w_ld[g] = H;
+          a.x = hprev, a.y = gh, a.epilogue = kEpiNone, a.t0 = c0, a.t1 = c1;
+          if ((rc = launch_dense(n, a, H, s))) return rc;
+        }
+        GateArgs ga;
+        memset(&ga, 0, sizeof(ga));
+        ga.gi = gi, ga.gi.t_off = gi.t_off - (L - 1 - st);
+        ga.gh = gh, ga.h_prev = hprev, ga.h_out = hout;
+        if (train) ga.acts = make_view(c.acts + (long long)st * c.Tc * 4 * H * NB, 4 * H * NB, -c0, N, 4 * H, B);
+        ga.H = H, ga.B = B, ga.t0 = c0, ga.t1 = c1, ga.back = L - 1 - st, ga.padded = padded, ga.first = st == 0;
+        ga.store = train, ga.t_episode0 = 0;
+        if ((rc = launch_gate(ga, N, false, s))) return rc;
+      }
     }
     last = make_view(hs_ptr(n, c, train, L - 1), H * NB, -c0, N, H, B);
   }
-  if (head_fused_eligible(n)) return launch_head_fused(n, params, last, train ? c.y1 : nullptr, lg, c0, c1, s);
+  if (c.plan.head == Head::kKernel) return launch_head_fused(n, params, last, train ? c.y1 : nullptr, lg, c0, c1, s);
   return head_dense(n, params, last, y1, c.y2, lg, c0, c1, s);
 }
 
@@ -695,10 +679,7 @@ static int backward_chunk(d2d_net* n, const float* params, const float* x, int x
                           const Chunk& c, float* grads, float inv_rows, cudaStream_t s) {
   const int N = n->N, B = n->B, H = n->H, O = n->O;
   const long long NB = (long long)N * B;
-  View xin;
-  memset(&xin, 0, sizeof(xin));
-  xin.p = const_cast<float*>(x), xin.t_stride = (long long)n->in_rows * B, xin.t_off = x_lead;
-  for (int g = 0; g < N; ++g) xin.f_off[g] = n->in_off[g];
+  const View xin = input_view(n, x, x_lead);
   const View y1 = make_view(c.y1, H * NB, -c0, N, H, B);
   const View dl = make_view(c.dl, O * NB, -c0, N, O, B);
   const View dy1 = make_view(c.dy1, H * NB, -c0, N, H, B);
@@ -757,77 +738,58 @@ static int backward_chunk(d2d_net* n, const float* params, const float* x, int x
   const View dgi = make_view(c.dgi, 3 * H * NB, -(c0 - halo), N, 3 * H, B);
   const View dgh = make_view(c.gh, 3 * H * NB, -c0, N, 3 * H, B);
   Wt whh{&n->o_whh, &n->o_bhh, nullptr, H, 3 * H};
-  const bool fused = gru_bwd_tc_eligible(n);
-  if (fused && gru_bptt_recompute_eligible(n)) {
-    // one kernel walks the whole window backwards and RECOMPUTES every step's gates from (x, h_prev) on the tensor
-    // cores: the forward kernel kept only h.  d(gi) is accumulated per observation, dW_hh / db_hh per CTA.
-    GruBpttArgs ba;
-    memset(&ba, 0, sizeof(ba));
-    ba.x = xin;
-    ba.hs = make_view(c.hs, H * NB, -c0, N, H, B);
-    ba.dh = make_view(dh_cur, H * NB, -c0, N, H, B);
-    ba.dgi = dgi;
-    ba.w = params, ba.w_agent_stride = n->stride;
-    for (int g = 0; g < N; ++g) {
-      ba.wih_off[g] = n->o_wih[g], ba.whh_off[g] = n->o_whh[g], ba.bih_off[g] = n->o_bih[g], ba.bhh_off[g] = n->o_bhh[g];
-      ba.in_dim[g] = n->in_dim[g];
-    }
-    ba.hs_step = (long long)c.Tc * H * NB;
-    // d(gh) ~ 1 / rows (the loss is a mean): the kernel scales it into the fp16 range by a power of two taken from the
-    // largest |dh| of the chunk
-    {
-      unsigned int* amax = reinterpret_cast<unsigned int*>(n->partial + (long long)n->N * n->n_strips * n->part_stride);
-      D2D_CUDA(cudaMemsetAsync(amax, 0, 4, s));
-      const long long cnt = (long long)(c1 - c0) * H * NB;
-      absmax_kernel<<<grid_for(cnt, 256), 256, 0, s>>>(dh_cur, cnt, amax);
-      D2D_LAUNCHED();
-      ba.dh_absmax = reinterpret_cast<const float*>(amax);
-    }
-    (void)inv_rows;
-    ba.L = L, ba.B = B, ba.t0 = c0, ba.t1 = c1;
-    ba.partial = n->partial, ba.part_stride = n->part_stride;
+  if (c.plan.bptt != Bptt::kFp32) {
+    // one kernel walks the whole window backwards (d(h) in registers, d(gh) W_hh on tcgen05) and accumulates d(gi) per
+    // observation and dW_hh / db_hh per CTA
     int strips = 0;
-    rc = n->H == 32 ? launch_gru_bptt_tc_h<32>(n, ba, s, &strips) : launch_gru_bptt_tc_h<64>(n, ba, s, &strips);
-    if (rc) return rc;
-    if (strips > 0) {   // dW_hh / db_hh: fixed-order sum of the per-CTA partials
-      WreduceArgs r;
-      memset(&r, 0, sizeof(r));
-      r.partial = n->partial, r.part_stride = n->part_stride, r.n_strips = strips, r.grads = grads;
-      r.g_agent_stride = n->stride, r.out_dim = 3 * H, r.with_bias = 1;
-      for (int g = 0; g < N; ++g) r.w_off[g] = n->o_whh[g], r.b_off[g] = n->o_bhh[g], r.in_dim[g] = H;
-      const int total = 3 * H * H + 3 * H;
-      wreduce_kernel<<<dim3((total + 255) / 256, N), 256, 0, s>>>(r);
-      D2D_LAUNCHED();
+    if (c.plan.bptt == Bptt::kRecompute) {
+      // gru_bptt_tc RECOMPUTES every step's gates from (x, h_prev) on the tensor cores: the forward kept only h
+      GruBpttArgs ba;
+      memset(&ba, 0, sizeof(ba));
+      ba.x = xin;
+      ba.hs = make_view(c.hs, H * NB, -c0, N, H, B);
+      ba.dh = make_view(dh_cur, H * NB, -c0, N, H, B);
+      ba.dgi = dgi;
+      ba.w = params, ba.w_agent_stride = n->stride;
+      for (int g = 0; g < N; ++g) {
+        ba.wih_off[g] = n->o_wih[g], ba.whh_off[g] = n->o_whh[g], ba.bih_off[g] = n->o_bih[g], ba.bhh_off[g] = n->o_bhh[g];
+        ba.in_dim[g] = n->in_dim[g];
+      }
+      ba.hs_step = (long long)c.Tc * H * NB;
+      // d(gh) ~ 1 / rows (the loss is a mean): the kernel scales it into the fp16 range by a power of two taken from
+      // the largest |dh| of the chunk
+      {
+        unsigned int* amax = reinterpret_cast<unsigned int*>(n->partial + (long long)n->N * n->n_strips * n->part_stride);
+        D2D_CUDA(cudaMemsetAsync(amax, 0, 4, s));
+        const long long cnt = (long long)(c1 - c0) * H * NB;
+        absmax_kernel<<<grid_for(cnt, 256), 256, 0, s>>>(dh_cur, cnt, amax);
+        D2D_LAUNCHED();
+        ba.dh_absmax = reinterpret_cast<const float*>(amax);
+      }
+      (void)inv_rows;
+      ba.L = L, ba.B = B, ba.t0 = c0, ba.t1 = c1;
+      ba.partial = n->partial, ba.part_stride = n->part_stride;
+      rc = n->H == 32 ? launch_gru_bptt_tc_h<32>(n, ba, s, &strips) : launch_gru_bptt_tc_h<64>(n, ba, s, &strips);
+    } else {
+      // gru_bwd_tc reads the gates the forward stored; it leaves d(gh) of step s in the first 3H features of that
+      // step's activation block
+      GruBwdTcArgs ba;
+      memset(&ba, 0, sizeof(ba));
+      ba.acts = make_view(c.acts, 4 * H * NB, -c0, N, 4 * H, B);
+      ba.hs = make_view(c.hs, H * NB, -c0, N, H, B);
+      ba.dh = make_view(dh_cur, H * NB, -c0, N, H, B);
+      ba.dgi = dgi;
+      ba.w = params, ba.w_agent_stride = n->stride;
+      for (int g = 0; g < N; ++g) ba.whh_off[g] = n->o_whh[g];
+      ba.acts_step = (long long)c.Tc * 4 * H * NB, ba.hs_step = (long long)c.Tc * H * NB;
+      ba.L = L, ba.B = B, ba.t0 = c0, ba.t1 = c1;
+      ba.partial = n->partial, ba.part_stride = n->part_stride;
+      rc = n->H == 32 ? launch_gru_bwd_tc_h<32>(n, ba, s, &strips) : launch_gru_bwd_tc_h<64>(n, ba, s, &strips);
     }
-  } else if (fused) {
-    // one kernel walks the whole window backwards (d(h) in registers, d(gh) W_hh on tcgen05); it leaves d(gh) of
-    // step s in the first 3H features of that step's activation block and d(gi) accumulated per observation
-    GruBwdTcArgs ba;
-    memset(&ba, 0, sizeof(ba));
-    ba.acts = make_view(c.acts, 4 * H * NB, -c0, N, 4 * H, B);
-    ba.hs = make_view(c.hs, H * NB, -c0, N, H, B);
-    ba.dh = make_view(dh_cur, H * NB, -c0, N, H, B);
-    ba.dgi = dgi;
-    ba.w = params, ba.w_agent_stride = n->stride;
-    for (int g = 0; g < N; ++g) ba.whh_off[g] = n->o_whh[g];
-    ba.acts_step = (long long)c.Tc * 4 * H * NB, ba.hs_step = (long long)c.Tc * H * NB;
-    ba.L = L, ba.B = B, ba.t0 = c0, ba.t1 = c1;
-    ba.partial = n->partial, ba.part_stride = n->part_stride;
-    int strips = 0;
-    rc = n->H == 32 ? launch_gru_bwd_tc_h<32>(n, ba, s, &strips) : launch_gru_bwd_tc_h<64>(n, ba, s, &strips);
     if (rc) return rc;
-    if (strips > 0) {   // dW_hh / db_hh: fixed-order sum of the per-CTA partials
-      WreduceArgs r;
-      memset(&r, 0, sizeof(r));
-      r.partial = n->partial, r.part_stride = n->part_stride, r.n_strips = strips, r.grads = grads;
-      r.g_agent_stride = n->stride, r.out_dim = 3 * H, r.with_bias = 1;
-      for (int g = 0; g < N; ++g) r.w_off[g] = n->o_whh[g], r.b_off[g] = n->o_bhh[g], r.in_dim[g] = H;
-      const int total = 3 * H * H + 3 * H;
-      wreduce_kernel<<<dim3((total + 255) / 256, N), 256, 0, s>>>(r);
-      D2D_LAUNCHED();
-    }
+    if (strips > 0 && (rc = launch_wreduce(n, whh, false, strips, grads, s))) return rc;
   }
-  for (int st = L - 1; st >= 0 && !fused; --st) {
+  for (int st = L - 1; st >= 0 && c.plan.bptt == Bptt::kFp32; --st) {
     const View hprev = make_view(hs_ptr(n, c, true, st - 1 < 0 ? 0 : st - 1), H * NB, -c0, N, H, B);
     GateArgs ga;
     memset(&ga, 0, sizeof(ga));
@@ -1018,48 +980,40 @@ extern "C" int d2d_net_rollout_step(d2d_net* n, const float* params, const float
   const long long NB = (long long)N * B;
   Chunk c;
   if ((rc = plan_chunk(n, false, 1, c))) return rc;
-  View xin;
-  memset(&xin, 0, sizeof(xin));
-  xin.p = const_cast<float*>(x), xin.t_stride = (long long)n->in_rows * B, xin.t_off = x_lead;
-  for (int g = 0; g < N; ++g) xin.f_off[g] = n->in_off[g];
-  const bool use_tc = gru_tc_eligible(n);
-  if (use_tc) {   // the tensor-core window kernel re-reads the L observations (L x I floats per row): no ring needed
-    const View hl = make_view(hs_ptr(n, c, false, L - 1), H * NB, -t, N, H, B);
-    if (head_fused_eligible(n) && !switched_off(kSwWindowHead)) {   // window + head in ONE launch, outputs written in place
-      const View lgo = make_view(out, O * NB, -t, N, O, B);
-      return launch_gru_tc(n, params, xin, hl, t, t + 1, 0, s, nullptr, nullptr, 0, 0, &lgo);
-    }
-    if ((rc = launch_gru_tc(n, params, xin, hl, t, t + 1, 0, s))) return rc;
-  }
-  if (!use_tc && !n->gi_ring) D2D_CUDA(cudaMalloc((void**)&n->gi_ring, (size_t)L * 3 * H * NB * 4));
-  if (!use_tc) {   // input projection of the NEW observation only; the previous L - 1 are still in the ring
-    DenseArgs a;
-    memset(&a, 0, sizeof(a));
-    Wt wih{&n->o_wih, &n->o_bih, &n->in_dim, 0, 3 * H};
-    fill_dense_w(n, a, params, wih, 0);
-    a.x = xin, a.y = make_view(n->gi_ring, 3 * H * NB, (t % L) - t, N, 3 * H, B), a.epilogue = kEpiNone;
-    a.t0 = t, a.t1 = t + 1;
-    if ((rc = launch_dense(n, a, n->max_in, s))) return rc;
-  }
-  for (int st = 0; st < L && !use_tc; ++st) {
-    const int back = L - 1 - st;
-    if (t - back < 0 && st < L - 1) continue;   // the step does not exist and h stays zero: nothing to do
-    GruStepArgs fa;
-    memset(&fa, 0, sizeof(fa));
-    const bool first = (t - back <= 0) || st == 0;   // first EXISTING step starts from h = 0
-    fa.h_prev = make_view(hs_ptr(n, c, false, st - 1 < 0 ? 0 : st - 1), H * NB, -t, N, H, B);
-    fa.h_out = make_view(hs_ptr(n, c, false, st), H * NB, -t, N, H, B);
-    fa.gi = make_view(n->gi_ring, 3 * H * NB, -back, N, 3 * H, B);
-    fa.t_mod_gi = L;
-    fa.t0 = t, fa.t1 = t + 1, fa.back = back, fa.padded = 0, fa.first = first, fa.store = 0;
-    if ((rc = launch_gru_step(n, fa, params, s))) return rc;
-  }
-  const View y1 = make_view(c.y1, H * NB, -t, N, H, B);
+  const View xin = input_view(n, x, x_lead);
+  const View hl = make_view(hs_ptr(n, c, false, L - 1), H * NB, -t, N, H, B);
   const View lg = make_view(out, O * NB, -t, N, O, B);
-  if (head_fused_eligible(n))
-    return launch_head_fused(n, params, make_view(hs_ptr(n, c, false, L - 1), H * NB, -t, N, H, B), nullptr, lg, t,
-                             t + 1, s);
-  return head_dense(n, params, make_view(hs_ptr(n, c, false, L - 1), H * NB, -t, N, H, B), y1, c.y2, lg, t, t + 1, s);
+  if (c.plan.window_tc) {   // the tensor-core window kernel re-reads the L observations (L x I floats per row): no ring
+    const bool head = c.plan.head == Head::kWindow;   // window + head in ONE launch, outputs written in place
+    rc = launch_gru_tc(n, params, xin, hl, t, t + 1, 0, s, nullptr, nullptr, 0, head ? &lg : nullptr, nullptr, nullptr);
+    if (rc || head) return rc;
+  } else {
+    if (!n->gi_ring) D2D_CUDA(cudaMalloc((void**)&n->gi_ring, (size_t)L * 3 * H * NB * 4));
+    {   // input projection of the NEW observation only; the previous L - 1 are still in the ring
+      DenseArgs a;
+      memset(&a, 0, sizeof(a));
+      Wt wih{&n->o_wih, &n->o_bih, &n->in_dim, 0, 3 * H};
+      fill_dense_w(n, a, params, wih, 0);
+      a.x = xin, a.y = make_view(n->gi_ring, 3 * H * NB, (t % L) - t, N, 3 * H, B), a.epilogue = kEpiNone;
+      a.t0 = t, a.t1 = t + 1;
+      if ((rc = launch_dense(n, a, n->max_in, s))) return rc;
+    }
+    for (int st = 0; st < L; ++st) {
+      const int back = L - 1 - st;
+      if (t - back < 0 && st < L - 1) continue;   // the step does not exist and h stays zero: nothing to do
+      GruStepArgs fa;
+      memset(&fa, 0, sizeof(fa));
+      const bool first = (t - back <= 0) || st == 0;   // first EXISTING step starts from h = 0
+      fa.h_prev = make_view(hs_ptr(n, c, false, st - 1 < 0 ? 0 : st - 1), H * NB, -t, N, H, B);
+      fa.h_out = make_view(hs_ptr(n, c, false, st), H * NB, -t, N, H, B);
+      fa.gi = make_view(n->gi_ring, 3 * H * NB, -back, N, 3 * H, B);
+      fa.t_mod_gi = L;
+      fa.t0 = t, fa.t1 = t + 1, fa.back = back, fa.padded = 0, fa.first = first, fa.store = 0;
+      if ((rc = launch_gru_step(n, fa, params, s))) return rc;
+    }
+  }
+  if (c.plan.head == Head::kKernel) return launch_head_fused(n, params, hl, nullptr, lg, t, t + 1, s);
+  return head_dense(n, params, hl, make_view(c.y1, H * NB, -t, N, H, B), c.y2, lg, t, t + 1, s);
 }
 
 static void fill_head(HeadArgs& h, int N, int B, int O, int out_kind, int dist_kind) {
@@ -1103,26 +1057,21 @@ extern "C" int d2d_net_rollout_act(d2d_net* n, const float* params, const float*
   cudaStream_t s = as_stream(stream);
   const int N = n->N, B = n->B, H = n->H, O = n->O;
   const long long NB = (long long)N * B;
-  if (gru_tc_eligible(n) && head_fused_eligible(n) && !switched_off(kSwWindowHead) && O > 1 && n->B % 4 == 0) {
+  Chunk c;
+  if ((rc = plan_chunk(n, false, 1, c))) return rc;
+  if (c.plan.head == Head::kWindow && O > 1 && n->B % 4 == 0) {
     HeadArgs h;
     fill_head(h, N, B, O, n->out_kind, dist_kind);
     h.act_mode = act_mode, h.actions = actions, h.logp = logp, h.act_t_off = -t;
     h.k0 = (uint32_t)(seed & 0xFFFFFFFFull), h.k1 = (uint32_t)(seed >> 32), h.env_offset = (uint32_t)env_offset;
     h.t_abs_off = t_abs0 - t;
-    Chunk c;
-    if ((rc = plan_chunk(n, false, 1, c))) return rc;
-    View xin;
-    memset(&xin, 0, sizeof(xin));
-    xin.p = const_cast<float*>(x), xin.t_stride = (long long)n->in_rows * B, xin.t_off = x_lead;
-    for (int g = 0; g < N; ++g) xin.f_off[g] = n->in_off[g];
     const View hl = make_view(hs_ptr(n, c, false, n->L - 1), H * NB, -t, N, H, B);
-    View lgo = make_view(logits_out, O * NB, -t, N, O, B);   // p == nullptr: outputs are not written
+    const View lgo = make_view(logits_out, O * NB, -t, N, O, B);   // p == nullptr: outputs are not written
     const DistArgs sel = h;
-    return launch_gru_tc(n, params, xin, hl, t, t + 1, 0, s, nullptr, nullptr, 0, 0, &lgo, nullptr, &sel);
+    return launch_gru_tc(n, params, input_view(n, x, x_lead), hl, t, t + 1, 0, s, nullptr, nullptr, 0, &lgo, nullptr,
+                         &sel);
   }
   // generic path: outputs into the chunk scratch (or the caller's buffer), then the head kernel
-  Chunk c;
-  if ((rc = plan_chunk(n, false, 1, c))) return rc;
   float* lg = logits_out ? logits_out : c.logits;
   if ((rc = d2d_net_rollout_step(n, params, x, x_lead, t, lg, stream))) return rc;
   return d2d_policy_head(N, B, O, 1, n->out_kind, dist_kind, act_mode, lg, actions, logp, nullptr, nullptr, seed,

@@ -291,19 +291,11 @@ int d2d_net_forward(d2d_net* net, const float* params, const float* x, int x_lea
 int d2d_net_check_inputs(const d2d_net* net, const float* x, int x_lead, int t0, int t1,
                          unsigned long long* n_inexact, void* stream);
 
-/* Kernel-family switches: A/B comparison and debugging (the library reads no environment variables).  A family that
- * is switched off (enabled = 0) runs on its FP32 CUDA-core kernel; D2D_SWITCH_ALL_TC = 0 keeps every GEMM off the
- * tensor cores.  Process-wide, not thread-safe: set before the first launch.  Default: everything enabled except D2D_SWITCH_WINDOW_WIDE. */
-#define D2D_SWITCH_GRU_WINDOW_TC 0
-#define D2D_SWITCH_GRU_BPTT_TC 1
-#define D2D_SWITCH_DENSE_TC 2
-#define D2D_SWITCH_WGRAD_TC 3
-#define D2D_SWITCH_FUSED_HEAD 4
-#define D2D_SWITCH_ALL_TC 5
-#define D2D_SWITCH_WINDOW_WIDE 8      /* 1: the GRU window kernel runs 32 warps of 64 registers instead of 16 of 128
-                                         (default 0: measured slower, kept for A/B runs) */
-#define D2D_SWITCH_WINDOW_HEAD 7      /* 0: the network head runs as its own kernel behind the GRU window kernel */
-#define D2D_SWITCH_BPTT_RECOMPUTE 6   /* 0: the BPTT kernel reads stored activations instead of recomputing the gates */
+/* Kernel switches: A/B comparison and debugging (the library reads no environment variables).  All three are enabled
+ * by default; any other id is rejected with D2D_ERR_INVALID.  Process-wide, not thread-safe: set before the first
+ * launch. */
+#define D2D_SWITCH_ALL_TC 5           /* 0: every GEMM, GRU window and BPTT of the learner runs on its FP32 CUDA-core
+                                         kernel instead of the tensor cores */
 #define D2D_SWITCH_ENV_MULTISTEP 9    /* 0: d2d_env_run_random_access launches one step kernel per step even where the
                                          register-resident multi-step kernel applies (single-channel env, N <= 4) */
 #define D2D_SWITCH_HOST_PACK 10       /* 0: d2d_env_step_host always copies the reference-layout actions as they are and

@@ -37,6 +37,22 @@ def test_version_and_error_string():
     assert b"null" in lib.d2d_last_error()
 
 
+def test_kernel_switch_ids():
+    """The header's D2D_SWITCH_* ids are the binding's; any other id is rejected (no CUDA is touched)."""
+    from d2d_ppo_b200 import _lib
+    src = open(os.path.join(ROOT, "include", "d2d_b200.h")).read()
+    declared = {k: int(v) for k, v in re.findall(r"#define D2D_(SWITCH_\w+)\s+(\d+)", src)}
+    assert declared == {k: getattr(_lib, k) for k in ("SWITCH_ALL_TC", "SWITCH_ENV_MULTISTEP", "SWITCH_HOST_PACK")}
+    lib = _lib.lib()
+    for which in declared.values():
+        on = lib.d2d_get_kernel_switch(which)
+        assert on in (0, 1)
+        assert lib.d2d_set_kernel_switch(which, on) == _lib.OK and lib.d2d_get_kernel_switch(which) == on
+    for which in set(range(-1, 12)) - set(declared.values()):
+        assert lib.d2d_set_kernel_switch(which, 1) == _lib.ERR_INVALID
+        assert lib.d2d_get_kernel_switch(which) == _lib.ERR_INVALID
+
+
 def test_no_oracle_import_in_product():
     pkg = os.path.join(ROOT, "d2d-ppo_b200")
     for dirpath, _, files in os.walk(pkg):
