@@ -69,7 +69,8 @@ __global__ void __launch_bounds__(256, 4) comb_step_kernel(const StepArgs a) {
           uint32_t want = ww[j];
           if constexpr (RA) {
             const uint32_t thr = a.tp_thr;
-            want = lane_mask_rk<CFIX>(a, env, (uint32_t)k | (kPurposePolicy << 16), C, [thr](int) { return thr; });
+            want = lane_mask_rk<CFIX>(a, env, a.t, (uint32_t)k | (kPurposePolicy << 16), C,
+                                      [thr](int) { return thr; });
             if (act_out) act_out[(size_t)k * B + b] = (MaskT)want;
           }
           const uint32_t at = rec_any<W>(rr[j]) ? (want & cmask) : 0u;
@@ -134,7 +135,8 @@ __global__ void __launch_bounds__(256, 4) comb_step_kernel(const StepArgs a) {
         sw = rp_sw[idx];
       } else {
         const uint32_t* thr = swthr + k * C;
-        sw = lane_mask_rk<CFIX>(a, env, (uint32_t)k | (kPurposeSwitch << 16), C, [thr](int c) { return thr[c]; });
+        sw = lane_mask_rk<CFIX>(a, env, a.t, (uint32_t)k | (kPurposeSwitch << 16), C,
+                                [thr](int c) { return thr[c]; });
       }
       const uint32_t ch_new = (ch ^ sw) & cmask;
       chan[idx] = (MaskT)ch_new;
@@ -201,6 +203,120 @@ int launch_comb_mode(const StepArgs& a, int grid, int block, cudaStream_t s, boo
     case 2: comb_step_kernel<W, MaskT, CFIX, PACK, 2><<<grid, block, a.params_bytes, s>>>(a); break;
     default: comb_step_kernel<W, MaskT, CFIX, PACK, 3><<<grid, block, a.params_bytes, s>>>(a); break;
   }
+  D2D_LAUNCHED();
+  return D2D_OK;
+}
+
+// n_inner consecutive fused random-access steps of ONE episode in one launch, one thread per env (the run form of
+// comb_step_kernel<W, uint8_t, CFIX, true, 2>, as sc_run_kernel is of sc_step_kernel).  The env's N <= NK records,
+// channel masks and disc / recv counters are loaded once, live in registers for every step and are stored once, so a
+// step moves no state through HBM: what it writes is the observation rows and the reward.  With the observations of
+// every step written to the same block (obs_stride 0, CombinatorialRandomAccess.run / bench.py) those rows of the
+// resident envs can stay in L2 (2 blocks of 256 per SM: 75,776 envs x 720 B = 55 MB of the 126 MB; one block per SM
+// measured slower, DESIGN.md section 3).  Same Philox counters and update order as comb_step_kernel: bit-identical.
+template <int W, int CFIX, int NK>
+__global__ void __launch_bounds__(256, 2) comb_run_kernel(const StepArgs a, const RunArgs ra) {
+  extern __shared__ __align__(16) uint8_t smem[];
+  const EnvParamsHdr* P = stage_params(a, smem);
+  const uint32_t* cdf = reinterpret_cast<const uint32_t*>(smem + P->off_cdf);
+  const uint32_t* swthr = reinterpret_cast<const uint32_t*>(smem + P->off_sw);
+  const int N = P->N;
+  constexpr int C = CFIX;
+  constexpr uint32_t cmask = (1u << C) - 1u;
+  const size_t B = (size_t)a.B;
+  const uint32_t Bu = (uint32_t)a.B;
+  uint8_t* chan = reinterpret_cast<uint8_t*>(a.chan);
+  const int b = blockIdx.x * blockDim.x + threadIdx.x;
+  if (b >= a.B) return;
+  const uint32_t env = a.env_offset + (uint32_t)b;
+  Rec<W> rec[NK];
+  uint32_t chv[NK], discv[NK], recvv[NK];
+#pragma unroll
+  for (int k = 0; k < NK; ++k) {
+    const size_t idx = (size_t)min(k, N - 1) * B + b;
+    rec[k] = rec_load<W>(a.buf, idx);
+    chv[k] = chan[idx], discv[k] = a.disc[idx], recvv[k] = a.recv[idx];
+  }
+  int32_t rew = a.reward_accum ? a.reward[b] : 0;
+  const uint32_t thr = a.tp_thr;
+#pragma unroll 1
+  for (int i = 0; i < ra.n_inner; ++i) {
+    const uint32_t t = a.t + (uint32_t)i;
+    const uint64_t active = ra.active[ra.t_plain + i];
+    // ---- who transmits where (combinatorial_env.py:135-148); the draws do not depend on the state ----
+    uint32_t once = 0, twice = 0, good_any = 0;
+    uint64_t att_pack = 0;
+#pragma unroll
+    for (int k = 0; k < NK; ++k) {
+      if (k < N) {
+        const uint32_t want =
+            lane_mask_rk<CFIX>(a, env, t, (uint32_t)k | (kPurposePolicy << 16), C, [thr](int) { return thr; });
+        const uint32_t at = rec_any<W>(rec[k]) ? (want & cmask) : 0u;
+        twice |= once & at;
+        once |= at;
+        good_any |= at & chv[k];
+        att_pack |= (uint64_t)at << (k * 8);
+      }
+    }
+    const uint32_t acked = once & ~twice & good_any;          // :155-157
+    const uint32_t nacked = once & ~acked;
+    // ---- serve, age, switch, arrive, observe (:160-206) ----
+    int n_success = 0;
+    uint4 arr4 = make_uint4(0u, 0u, 0u, 0u);
+    float* obs_i = a.obs ? a.obs + (size_t)i * (size_t)ra.obs_stride : nullptr;
+#pragma unroll
+    for (int k = 0; k < NK; ++k) {
+      if (k < N) {
+        Rec<W>& r = rec[k];
+        const uint32_t at = (uint32_t)(att_pack >> (k * 8)) & 0xFFu;
+        const uint32_t ch = chv[k];
+        const bool success = (at & ch & acked) != 0;
+        n_success += success;
+        rec_pop_earliest<W>(r, success);
+        discv[k] += rec_age<W>(r);
+        const uint32_t* sthr = swthr + k * C;
+        const uint32_t sw =
+            lane_mask_rk<CFIX>(a, env, t, (uint32_t)k | (kPurposeSwitch << 16), C, [sthr](int c) { return sthr[c]; });
+        chv[k] = (ch ^ sw) & cmask;
+        const int dl = P->deadline[k];
+        // one Philox call per four devices (env_common.cuh: ArrivalWords), drawn when any device of the group is active
+        if ((k & 3) == 0 && ((active >> k) & 0xFull))
+          arr4 = philox_rk(a, env, t, (uint32_t)(k >> 2) | (kPurposeArrival << 16), 0u);
+        if ((active >> k) & 1ull) {
+          const uint32_t arrived = arrival_from_u(P, cdf, k, pick_word(arr4, k & 3));
+          rec_set_byte<W>(r, dl - 1, arrived);
+          recvv[k] += arrived;
+        }
+        if (obs_i) {
+          float* o = obs_i + (size_t)P->obs_off[k] * B + b;
+          o = emit_slots<W>(r, P->homog ? P->D : dl, o, Bu);
+          o = emit_bits<CFIX>(ch, C, o, Bu);                  // pre-switch copy (:145)
+          emit_ack<CFIX>(acked, nacked, C, o, Bu);
+        }
+      }
+    }
+    if (a.reward_accum) rew += n_success;                     // :211
+    else a.reward[(size_t)i * ra.reward_stride + b] = n_success;
+  }
+#pragma unroll
+  for (int k = 0; k < NK; ++k) {
+    if (k < N) {
+      const size_t idx = (size_t)k * B + b;
+      rec_store<W>(a.buf, idx, rec[k]);
+      chan[idx] = (uint8_t)chv[k];
+      a.disc[idx] = discv[k], a.recv[idx] = recvv[k];
+    }
+  }
+  if (a.reward_accum) a.reward[b] = rew;
+  if (a.done) a.done[b] = (uint8_t)a.done_flag;
+}
+
+// d2d_env_run_random_access's episode-in-one-launch path for the combinatorial env; C must be 4 or 8, N <= 8
+template <int W>
+int launch_comb_run(const StepArgs& a, const RunArgs& ra, int C, cudaStream_t s) {
+  const int block = 256, grid = (a.B + block - 1) / block;
+  if (C == 8) comb_run_kernel<W, 8, 8><<<grid, block, a.params_bytes, s>>>(a, ra);
+  else comb_run_kernel<W, 4, 8><<<grid, block, a.params_bytes, s>>>(a, ra);
   D2D_LAUNCHED();
   return D2D_OK;
 }

@@ -2,4 +2,5 @@
 #include "env_comb_step.cuh"
 namespace d2d {
 template int launch_comb_step<2>(const StepArgs&, int, int, int, cudaStream_t);
+template int launch_comb_run<2>(const StepArgs&, const RunArgs&, int, cudaStream_t);
 }

@@ -53,6 +53,15 @@ struct StepArgs {
   int reward_accum;  // 1: reward[b] += this step's reward (d2d_env_run_random_access), 0: overwrite
 };
 
+// the multi-step kernels (sc_run_kernel, sc_run_lanes_kernel, comb_run_kernel): n_inner steps of one episode per launch
+struct RunArgs {
+  const uint64_t* active;      // device copy of the per-timestep arrival masks, indexed by the episode timestep
+  int t_plain;                 // episode timestep of the first step produced (a.t is its Philox counter)
+  int n_inner;
+  long long reward_stride;     // elements between the reward rows of consecutive steps (0 with reward_accum)
+  long long obs_stride;        // elements between the observation blocks of consecutive steps (comb_run_kernel)
+};
+
 __device__ __forceinline__ const EnvParamsHdr* stage_params(const StepArgs& a, uint8_t* smem) {
   const uint32_t* src = reinterpret_cast<const uint32_t*>(a.params);
   uint32_t* dst = reinterpret_cast<uint32_t*>(smem);
@@ -230,16 +239,16 @@ __device__ __forceinline__ uint4 philox_rk(const StepArgs& a, uint32_t c0, uint3
   return make_uint4(c0, c1, c2, c3);
 }
 
-// bit c = (16-bit lane c < thr(c)) for c < C;  CFIX > 0 makes the lane count a compile-time constant
+// bit c = (16-bit lane c < thr(c)) for c < C at Philox timestep t;  CFIX > 0 makes the lane count a compile-time constant
 template <int CFIX, typename ThrFn>
-__device__ __forceinline__ uint32_t lane_mask_rk(const StepArgs& a, uint32_t env, uint32_t dev_purpose, int C,
-                                                 ThrFn thr) {
+__device__ __forceinline__ uint32_t lane_mask_rk(const StepArgs& a, uint32_t env, uint32_t t, uint32_t dev_purpose,
+                                                 int C, ThrFn thr) {
   uint32_t m = 0;
   const int nl = CFIX ? CFIX : C;
 #pragma unroll
   for (int blk = 0; blk < (CFIX ? (CFIX + 7) / 8 : 4); ++blk) {
     if (blk * 8 < nl) {
-      const uint4 r = philox_rk(a, env, a.t, dev_purpose, (uint32_t)blk);
+      const uint4 r = philox_rk(a, env, t, dev_purpose, (uint32_t)blk);
       const uint32_t w[4] = {r.x, r.y, r.z, r.w};
 #pragma unroll
       for (int l = 0; l < 8; ++l) {

@@ -30,6 +30,8 @@ namespace d2d {
 
 template <int W>
 int launch_comb_step(const StepArgs& a, int N, int C, int mask_bytes, cudaStream_t s);  // env_comb_w{2,4,8}.cu
+template <int W>
+int launch_comb_run(const StepArgs& a, const RunArgs& ra, int C, cudaStream_t s);         // env_comb_w{2,4}.cu
 
 // ================================================================================================
 // CombinatorialEnv reset (the step kernel lives in env_comb_step.cuh)
@@ -243,13 +245,7 @@ __global__ void __launch_bounds__(256, NK ? 5 : 4) sc_step_kernel(const StepArgs
 // env, so no step needs a grid-wide barrier.  The per-step kernel at the named c2 size (4,096 envs) is launch-latency
 // bound (8.2 us a step for ~0.5 MB of state); this one is bound by the dependent-issue chain of a single warp.
 // Same Philox counters and the same update order as sc_step_kernel: trajectories are bit-identical.
-struct RunArgs {
-  const uint64_t* active;      // device copy of the per-timestep arrival masks, indexed by the episode timestep
-  int t_plain;                 // episode timestep of the first step produced (a.t is its Philox counter)
-  int n_inner;
-  long long reward_stride;     // elements between the reward rows of consecutive steps (0 with reward_accum)
-};
-
+// (RunArgs: env_common.cuh)
 template <int W, int NK>
 __global__ void __launch_bounds__(256) sc_run_kernel(const StepArgs a, const RunArgs ra) {
   extern __shared__ __align__(16) uint8_t smem[];
@@ -1098,11 +1094,13 @@ extern "C" int d2d_env_run_random_access(d2d_env* e, double tp, int n_steps, int
     }
   }
   const uint32_t tp_thr = (uint32_t)std::min(65536.0, std::max(0.0, std::floor(tp * 65536.0 + 0.5)));
-  // single-channel env, N <= 4, no per-step observation / state rows wanted: the steps of one episode run inside ONE
-  // kernel with the env state in registers (sc_run_kernel)
-  const bool multi = e->kind == D2D_ENV_SINGLE_CHANNEL && e->N <= 4 && (e->W == 2 || e->W == 4) &&
-                     e->rng_mode == D2D_RNG_PHILOX && !obs && !state &&
-                     d2d_get_kernel_switch(D2D_SWITCH_ENV_MULTISTEP) == 1;
+  // the steps of one episode run inside ONE kernel with the env state in registers: the single-channel env with N <= 4
+  // and no per-step observation rows (sc_run_kernel), the combinatorial env with N <= 8, C = 4 or 8 and the
+  // one-thread-per-env mapping, observations at any stride or none (comb_run_kernel); never with state rows
+  const bool philox = e->rng_mode == D2D_RNG_PHILOX && (e->W == 2 || e->W == 4) && !state &&
+                      d2d_get_kernel_switch(D2D_SWITCH_ENV_MULTISTEP) == 1;
+  const bool comb_multi = philox && e->kind == D2D_ENV_COMBINATORIAL && e->N <= 8 && (e->C == 4 || e->C == 8);
+  const bool multi = comb_multi || (philox && e->kind == D2D_ENV_SINGLE_CHANNEL && e->N <= 4 && !obs);
   for (int i = 0; i < n_steps; ++i) {
     float* obs_i = obs ? obs + (size_t)i * obs_step_stride : nullptr;
     float* state_i = state ? state + (size_t)i * state_step_stride : nullptr;
@@ -1122,18 +1120,25 @@ extern "C" int d2d_env_run_random_access(d2d_env* e, double tp, int n_steps, int
       a.done_flag = e->t + n_inner >= e->T;
       RunArgs ra;
       ra.active = e->active_dev, ra.t_plain = e->t + 1, ra.n_inner = n_inner, ra.reward_stride = reward_step_stride;
-      if (e->B <= kRunLanesMaxEnvs) {
+      ra.obs_stride = obs_step_stride;
+      if (comb_multi) {
+        a.obs = obs_i;
+        rc = e->W == 2 ? launch_comb_run<2>(a, ra, e->C, as_stream(stream))
+                       : launch_comb_run<4>(a, ra, e->C, as_stream(stream));
+        if (rc) return rc;
+      } else if (e->B <= kRunLanesMaxEnvs) {
         // small batches: four lanes per env (sc_run_lanes_kernel), 64-thread blocks = 16 envs spread over the SMs
         const int block = 64, grid = (int)(((long long)e->B * 4 + block - 1) / block);
         if (e->W == 2) sc_run_lanes_kernel<2><<<grid, block, e->params_bytes, as_stream(stream)>>>(a, ra);
         else sc_run_lanes_kernel<4><<<grid, block, e->params_bytes, as_stream(stream)>>>(a, ra);
+        D2D_LAUNCHED();
       } else {
         // few envs: 64-thread blocks spread the warps over the SMs (each warp is one dependent-issue chain)
         const int block = e->B >= 148 * 256 ? 256 : 64, grid = (e->B + block - 1) / block;
         if (e->W == 2) sc_run_kernel<2, 4><<<grid, block, e->params_bytes, as_stream(stream)>>>(a, ra);
         else sc_run_kernel<4, 4><<<grid, block, e->params_bytes, as_stream(stream)>>>(a, ra);
+        D2D_LAUNCHED();
       }
-      D2D_LAUNCHED();
       e->t += n_inner;
       i += n_inner - 1;
       if (steps_done) *steps_done = i + 1;

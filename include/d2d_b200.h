@@ -151,9 +151,11 @@ int d2d_env_step_random_access(d2d_env* env, double transmission_prob, void* act
  *                     (stride 0) every step ADDS its reward into the one [B] buffer (zero it first): the
  *                     per-episode reward sum of baselines.py:211
  *   done              u8 [B] of the last step (may be NULL);  *steps_done (may be NULL): steps actually run
- * Single-channel env with N <= 4 and obs == state == NULL (rewards only, RandomAccess.run): the steps of an episode
- * run in ONE launch with the env state in registers (sc_run_kernel), bit-identical to the per-step launches
- * (D2D_SWITCH_ENV_MULTISTEP = 0 restores them). */
+ * With Philox streams and state == NULL the steps of an episode run in ONE launch with the env state in registers,
+ * bit-identical to the per-step launches (D2D_SWITCH_ENV_MULTISTEP = 0 restores them): the single-channel env with
+ * N <= 4 and obs == NULL (rewards only, RandomAccess.run; sc_run_kernel), and the combinatorial env with N <= 8 and
+ * C = 4 or 8, observations at any stride or NULL (CombinatorialRandomAccess.run; comb_run_kernel).  Everything else
+ * (replayed streams, state rows, C = 16, N > 8) runs one step kernel per step.  Resets stay launches of their own. */
 int d2d_env_run_random_access(d2d_env* env, double transmission_prob, int n_steps, int auto_reset, float* obs,
                               int64_t obs_step_stride, float* state, int64_t state_step_stride, int32_t* reward,
                               int64_t reward_step_stride, int reward_accumulate, uint8_t* done, void* stream,
@@ -296,8 +298,10 @@ int d2d_net_check_inputs(const d2d_net* net, const float* x, int x_lead, int t0,
  * launch. */
 #define D2D_SWITCH_ALL_TC 5           /* 0: every GEMM, GRU window and BPTT of the learner runs on its FP32 CUDA-core
                                          kernel instead of the tensor cores */
-#define D2D_SWITCH_ENV_MULTISTEP 9    /* 0: d2d_env_run_random_access launches one step kernel per step even where the
-                                         register-resident multi-step kernel applies (single-channel env, N <= 4) */
+#define D2D_SWITCH_ENV_MULTISTEP 9    /* 0: d2d_env_run_random_access launches one step kernel per step even where a
+                                         register-resident multi-step kernel applies (Philox streams, no state rows:
+                                         single-channel env with N <= 4 and no observations; combinatorial env with
+                                         N <= 8 and C = 4 or 8) */
 #define D2D_SWITCH_HOST_PACK 10       /* 0: d2d_env_step_host always copies the reference-layout actions as they are and
                                          packs them on the device (default: packed on the host when >= 12 host threads) */
 int d2d_set_kernel_switch(int which, int enabled);
