@@ -98,6 +98,8 @@ _SIGNATURES = {
     "d2d_net_check_inputs": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_int, _P, _P]),
     "d2d_set_kernel_switch": (C.c_int, [C.c_int, C.c_int]),
     "d2d_get_kernel_switch": (C.c_int, [C.c_int]),
+    "d2d_set_deterministic": (C.c_int, [C.c_int]),
+    "d2d_get_deterministic": (C.c_int, []),
     "d2d_net_rollout_step": (C.c_int, [_P, _P, _P, C.c_int, C.c_int, _P, _P]),
     "d2d_net_rollout_act": (C.c_int, [_P, _P, _P, C.c_int, C.c_int, C.c_int, C.c_int, _P, _P, C.c_uint64, C.c_uint64,
                                       C.c_int, _P, _P]),

@@ -3,6 +3,11 @@
 The sequential chain M <- ratio_i * M (d2d_ppo.py:427-436) uses each agent's PRE-update ratio, and the agents'
 networks are disjoint, so all N forward passes run in one launch, the chain is a running product inside the loss
 kernel (csrc/learner_pointwise.cuh: ppo_dlogits_kernel), and all N backward passes run in one launch.
+
+Reproducibility: with ``d2d_ppo_b200.use_deterministic_algorithms(True)`` a seeded single-GPU run is bit-identical
+from run to run (same build, GPU model, ``seed``, ``n_envs`` and ``scratch_bytes``).  ``train`` shuffles the HAPPO agent
+order with the GLOBAL ``np.random``, as the reference does (d2d_ppo.py:421-422): call ``np.random.seed`` before it, as
+the reference scripts do, for a repeatable run.
 """
 from __future__ import annotations
 

@@ -3,6 +3,10 @@
 Same constructor, ``train`` / ``test`` / ``create_rollouts`` / ``save`` / ``load`` as the reference ``iPPO``; the
 rollout of B lockstep envs, the per-agent networks, the lambda-returns and the clipped-surrogate update run as
 sm_100a kernels (csrc/learner_api.cu), all N agents per launch.
+
+Reproducibility: with ``d2d_ppo_b200.use_deterministic_algorithms(True)`` a seeded single-GPU run (same build, GPU
+model, ``seed``, ``n_envs`` and ``scratch_bytes``) gives bit-identical parameters, Adam moments, losses, scores and
+``test`` results; by default the learner's sums use atomics and runs differ in the last bits.
 """
 from __future__ import annotations
 

@@ -7,6 +7,10 @@ each run one episode per iteration of ``train`` (B plays the role of B sequentia
 learners); every env column keeps its own transition deque inside one device-resident ring, all N agents' networks
 run in one launch (net sets with ``head_layers = 2``), and action selection, TD target, loss gradient and the replay
 gather are kernels of csrc/dqn_pointwise.cuh.  No step of the path runs in eager PyTorch.
+
+Reproducibility: with ``d2d_ppo_b200.use_deterministic_algorithms(True)`` a seeded single-GPU run (same build, GPU
+model, ``seed``, ``n_envs`` and ``scratch_bytes``) is bit-identical from run to run; the replay sampling draws from its
+own seeded generator.
 """
 from __future__ import annotations
 

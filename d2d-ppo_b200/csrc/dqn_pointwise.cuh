@@ -84,7 +84,9 @@ struct QLossArgs {
   double* loss_sum;       // [N]
 };
 
-__global__ void q_loss_grad_kernel(const QLossArgs a) {
+// part != nullptr (deterministic mode): warp w of agent g's blocks stores its sum to part[g][w] instead of the atomic
+template <bool PART>
+__device__ __forceinline__ void q_loss_grad_body(const QLossArgs& a, double* part) {
   const int g = blockIdx.y, N = gridDim.y;
   const long long n = (long long)(a.t1 - a.t0) * a.B;
   double local = 0.0;
@@ -109,8 +111,13 @@ __global__ void q_loss_grad_kernel(const QLossArgs a) {
     if (a.q_out) a.q_out[idx] = qa;
   }
   for (int o = 16; o > 0; o >>= 1) local += __shfl_down_sync(0xFFFFFFFFu, local, o);
-  if ((threadIdx.x & 31) == 0) atomicAdd(&a.loss_sum[g], local);
+  if ((threadIdx.x & 31) == 0) {
+    if constexpr (PART) part[(long long)g * gridDim.x * (blockDim.x >> 5) + ((blockIdx.x * blockDim.x + threadIdx.x) >> 5)] = local;
+    else atomicAdd(&a.loss_sum[g], local);
+  }
 }
+__global__ void q_loss_grad_kernel(const QLossArgs a) { q_loss_grad_body<false>(a, nullptr); }
+__global__ void q_loss_grad_part_kernel(const QLossArgs a, double* part) { q_loss_grad_body<true>(a, part); }
 
 // ---- ReplayBuffer.sample_chunk (irdqn.py:24-42) ----
 struct GatherArgs {

@@ -26,7 +26,8 @@
 //      thread 0 issues the 16 recompute MMAs (x: N = 4H over W_ih as [r; z; 0; n]; h: N = 3H, W_hh^T read MN-major from
 //      the SAME tiles the data-gradient GEMM reads K-major);
 //   B. threads read the 4H pre-activations of their units from TMEM, evaluate gates and derivatives, write G = d(gh)
-//      (2 planes), add d(gi) to the observation's gradient row (red.global: up to L windows share an observation) and
+//      (2 planes), add d(gi) to the observation's gradient row (red.global: up to L windows share an observation; the
+//      kDgiSlices variant stores it into slice s at the window's own time instead, see dgi_slice_sum_kernel) and
 //      pre-load D with the direct path dh z; lane 0 of every warp issues its share of D += G W_hh (36 MMAs) and
 //      dW += G^T P (48 MMAs, both tiles read along their contiguous dimension);
 //   C. threads read dh_prev from D while the next step's h and x are in flight.
@@ -42,7 +43,8 @@ struct GruBpttArgs {
   View x;      // observations: element (agent g, feature f, time t, env b); time blocks before 0 are zero
   View hs;     // [.. H ..] h after step 0 (forward kernel, store mode); step s is hs_step floats further
   View dh;     // [.. H ..] in: d(loss) / d(h after the last step)
-  View dgi;    // [.. 3H ..] accumulated at observation time t - (L - 1 - s); zeroed by the caller
+  View dgi;    // [.. 3H ..] accumulated at observation time t - (L - 1 - s); zeroed by the caller (the slices kernel:
+               // slice 0 of the [L][..] d(gi) slices, written at time t)
   const float* w;
   long long w_agent_stride;
   int wih_off[D2D_MAX_AGENTS], whh_off[D2D_MAX_AGENTS], bih_off[D2D_MAX_AGENTS], bhh_off[D2D_MAX_AGENTS];
@@ -54,6 +56,7 @@ struct GruBpttArgs {
                            // that brings it to ~2^10 before the fp16 split, so that values down to 2^-22 of the
                            // largest one keep 22 significant bits (fp16 max 65504 leaves a factor 64 of headroom)
   int L, B, t0, t1;
+  long long slice_step;    // kDgiSlices instantiation: floats between two d(gi) slices
 };
 
 #ifdef D2D_BPTT_TRACE
@@ -126,9 +129,14 @@ __device__ __forceinline__ uint32_t idesc_f16_major(int n, bool a_mn, bool b_mn)
 }
 }  // namespace tcr
 
-template <int H>
+// HS = H: d(gi) is added into a.dgi at the observation's time (fp32 reductions, order not fixed).
+// HS = H | kDgiSlices (deterministic mode): window step s stores its d(gi) into slice s, a.slice_step floats from
+// slice 0 = a.dgi, at the window's own time t; dgi_slice_sum_kernel then sums the L slices in a fixed order.
+template <int HS>
 __global__ void __launch_bounds__(tcr::kThreads, 1) gru_bptt_tc_kernel(const GruBpttArgs a) {
   using namespace tc;
+  constexpr int H = HS & ~kDgiSlices;
+  constexpr bool SLICES = (HS & kDgiSlices) != 0;
   using S = tcr::Smem<H>;
   static_assert(H == 32 || H == 64, "units per thread (H / 4) must be a multiple of 8");
   constexpr int UT = H / 4;            // hidden units per thread
@@ -350,7 +358,8 @@ __global__ void __launch_bounds__(tcr::kThreads, 1) gru_bptt_tc_kernel(const Gru
     };
     load_step(L - 1);
     for (int s = L - 1; s >= 0; --s) {
-      float* gp = view_ptr(a.dgi, g, t - (L - 1 - s), a.B, bb) + (long long)u0 * a.B;
+      float* gp = SLICES ? view_ptr(a.dgi, g, t, a.B, bb) + s * a.slice_step + (long long)u0 * a.B
+                         : view_ptr(a.dgi, g, t - (L - 1 - s), a.B, bb) + (long long)u0 * a.B;
       D2D_TR(0);
       // ---- A. h_{s-1} (2 planes) -> tensor memory, X = x_s -> shared memory ----
       // (D's columns are free: this thread read its own in phase C, the MMAs that wrote them completed before that;
@@ -419,12 +428,11 @@ __global__ void __launch_bounds__(tcr::kThreads, 1) gru_bptt_tc_kernel(const Gru
           const float dr = dn * ghn * r * (1.0f - r);
           dg[0][j] = dr * gs, dg[1][j] = dz * gs, dg[2][j] = dn * r * gs;
           dd[j] = dv * z * d_scale;          // direct path: pre-loaded into D, d(gh) W_hh accumulates on top
-#ifndef D2D_BPTT_NO_ATOMICS   // (timing experiment only)
           if (ok) {
             const long long f = (long long)u * a.B;
-            atomicAdd(gp + f, dr), atomicAdd(gp + f + HB, dz), atomicAdd(gp + f + 2 * HB, dn);
+            if constexpr (SLICES) gp[f] = dr, gp[f + HB] = dz, gp[f + 2 * HB] = dn;
+            else atomicAdd(gp + f, dr), atomicAdd(gp + f + HB, dz), atomicAdd(gp + f + 2 * HB, dn);
           }
-#endif
         }
         if (c == 0) D2D_TR(3);
         if (c == 0 && n_steps > 0) {         // G and P are free once the previous step's weight-gradient MMAs are done

@@ -38,7 +38,8 @@ struct GruBwdTcArgs {
   View acts;   // [.. 4H ..] step 0; step s is acts_step floats further: r, z, n, gh_n
   View hs;     // [.. H ..]  h after step 0; step s is hs_step floats further
   View dh;     // [.. H ..]  in: d(loss) / d(h after the last step)
-  View dgi;    // [.. 3H ..] accumulated at observation time t - (L - 1 - s); zeroed by the caller
+  View dgi;    // [.. 3H ..] accumulated at observation time t - (L - 1 - s); zeroed by the caller (the slices kernel:
+               // slice 0 of the [L][..] d(gi) slices, written at time t)
   const float* w;
   long long w_agent_stride;
   int whh_off[D2D_MAX_AGENTS];
@@ -46,7 +47,11 @@ struct GruBwdTcArgs {
   long long part_stride;
   long long acts_step, hs_step;
   int L, B, t0, t1;
+  long long slice_step;    // kDgiSlices instantiation: floats between two d(gi) slices
 };
+
+// or-ed into the H template argument of the BPTT kernels: d(gi) per window step into slices (deterministic mode)
+constexpr int kDgiSlices = 1024;
 
 namespace tcb {
 constexpr int kThreads = 512;
@@ -80,9 +85,16 @@ __device__ __forceinline__ uint32_t idesc_bf16_mn(int n) {
 }
 }  // namespace tcb
 
-template <int H>
+// HS = H | kDgiSlices (deterministic mode): d(gi) of window step s is stored into slice s (a.slice_step floats from
+// slice 0 = a.dgi) at the window's own time, for dgi_slice_sum_kernel; HS = H: added atomically as described above.
+template <int HS>
 __global__ void __launch_bounds__(tcb::kThreads, 1) gru_bwd_tc_kernel(const GruBwdTcArgs a) {
   using namespace tc;
+  constexpr int H = HS & ~kDgiSlices;
+  constexpr bool SLICES = (HS & kDgiSlices) != 0;
+  // MMAs that accumulate into one TMEM tile run in issue order, and the order of issue across warps is not fixed: the
+  // deterministic variant issues every MMA from warp 0 in a fixed order
+  constexpr int kIssuers = SLICES ? 1 : tcb::kThreads / 32;
   using S = tcb::Smem<H>;
   static_assert(H == 32 || H == 64, "units per thread (H / 4) must be a multiple of 8");
   constexpr int UT = H / 4;            // hidden units per thread
@@ -115,7 +127,7 @@ __global__ void __launch_bounds__(tcb::kThreads, 1) gru_bwd_tc_kernel(const GruB
     sp0[canon16(r, H + c, NP0)] = __float2bfloat16_rn(c == 0 ? 1.0f : 0.0f);
   }
   if (tid == 0) {
-    mbar_init(a_ready, tcb::kThreads), mbar_init(d_ready, tcb::kThreads / 32), mbar_init(w_done, tcb::kThreads / 32);
+    mbar_init(a_ready, tcb::kThreads), mbar_init(d_ready, kIssuers), mbar_init(w_done, kIssuers);
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
   }
   constexpr uint32_t kColsUsed = H + NBLK * NP0;
@@ -190,7 +202,8 @@ __global__ void __launch_bounds__(tcb::kThreads, 1) gru_bwd_tc_kernel(const GruB
     };
     load_step(L - 1);
     for (int s = L - 1; s >= 0; --s) {
-      float* gp = view_ptr(a.dgi, g, t - (L - 1 - s), a.B, bb) + (long long)u0 * a.B;
+      float* gp = SLICES ? view_ptr(a.dgi, g, t, a.B, bb) + s * a.slice_step + (long long)u0 * a.B
+                         : view_ptr(a.dgi, g, t - (L - 1 - s), a.B, bb) + (long long)u0 * a.B;
       // the operand tiles are free once the weight-gradient MMAs of the previous staging have completed
       if (staged_before) {
         mbar_wait(w_done, ph_w);
@@ -211,7 +224,8 @@ __global__ void __launch_bounds__(tcb::kThreads, 1) gru_bwd_tc_kernel(const GruB
           dh[u] = d * z[u];                  // direct path: pre-loaded into D, d(gh) W_hh accumulates on top
           if (ok) {
             const long long f = (long long)u * a.B;
-            atomicAdd(gp + f, dr), atomicAdd(gp + f + HB, dz), atomicAdd(gp + f + 2 * HB, dn);
+            if constexpr (SLICES) gp[f] = dr, gp[f + HB] = dz, gp[f + 2 * HB] = dn;
+            else atomicAdd(gp + f, dr), atomicAdd(gp + f + HB, dz), atomicAdd(gp + f + 2 * HB, dn);
           }
         }
         if (s > 0) tcb::tmem_st8(tmem + lane_addr + (uint32_t)(u0 + c * 8), &dh[c * 8]);
@@ -246,11 +260,11 @@ __global__ void __launch_bounds__(tcb::kThreads, 1) gru_bwd_tc_kernel(const GruB
       asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
       asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
       mbar_arrive(a_ready);
-      if (lane == 0) {
+      if (lane == 0 && (!SLICES || warp == 0)) {
         mbar_wait(a_ready, ph_a);
         ph_a ^= 1u;
         asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-        constexpr int kWarps = tcb::kThreads / 32;
+        constexpr int kWarps = kIssuers;
         if (s > 0) {
           // D += d(gh) W_hh : G K-major x W_hh^T K-major, five plane products x 3H / 16 reduction steps, dealt round
           // robin to the warps' issuing lanes

@@ -46,6 +46,8 @@ struct d2d_net {
   float* partial = nullptr;   // wgrad partial sums
   long long part_stride = 0;
   int n_strips = 0;
+  double* red = nullptr;      // deterministic mode: per-warp partial loss sums (sum_partials_kernel)
+  long long red_cap = 0;      // doubles
 };
 
 // ------------------------------------------------------------------------------------------------
@@ -91,6 +93,34 @@ extern "C" int d2d_set_kernel_switch(int which, int enabled) {
 extern "C" int d2d_get_kernel_switch(int which) {
   const int* sw = switch_ptr(which);
   return sw ? *sw : D2D_ERR_INVALID;
+}
+
+// Deterministic mode (d2d_set_deterministic): fixed-order sums in place of the floating-point atomics.  Read at every
+// call; off by default, and with it off every launch is the one the library makes without it.
+static int g_deterministic = 0;
+extern "C" int d2d_set_deterministic(int enabled) {
+  g_deterministic = enabled ? 1 : 0;
+  return D2D_OK;
+}
+extern "C" int d2d_get_deterministic(void) { return g_deterministic; }
+
+// out[grp][k] += the fixed-order sum of part[grp][0 .. n_parts)[k]  (grp < n_groups, k < n_vals)
+static int launch_sum_partials(const double* part, int n_groups, int n_parts, int n_vals, double* out, cudaStream_t s) {
+  sum_partials_kernel<<<n_groups * n_vals, 256, 0, s>>>(part, n_parts, n_vals, out);
+  D2D_LAUNCHED();
+  return D2D_OK;
+}
+
+// the net's scratch for per-warp partial sums, at least `count` doubles
+static int reduce_scratch(d2d_net* n, long long count, double** out) {
+  if (count > n->red_cap) {
+    if (n->red) cudaFree(n->red);
+    n->red = nullptr, n->red_cap = 0;
+    D2D_CUDA(cudaMalloc((void**)&n->red, (size_t)count * sizeof(double)));
+    n->red_cap = count;
+  }
+  *out = n->red;
+  return D2D_OK;
 }
 
 template <int RPT, int OPT>
@@ -341,9 +371,9 @@ static int launch_gru_step(const d2d_net* n, GruStepArgs& a, const float* params
   return D2D_OK;
 }
 
-// Which kernels a call on the net runs.  It depends on the net's shape and D2D_SWITCH_ALL_TC only, and is evaluated
-// per call (plan_chunk keeps it in Chunk::plan) because the switch may change between calls on the same net: the
-// scratch layout and the launches all read this one decision.
+// Which kernels a call on the net runs.  It depends on the net's shape, D2D_SWITCH_ALL_TC and the deterministic mode
+// only, and is evaluated per call (plan_chunk keeps it in Chunk::plan) because both may change between calls on the
+// same net: the scratch layout and the launches all read this one decision.
 enum class Bptt { kFp32, kRecompute, kStoredTc };
 enum class Head { kDense, kKernel, kWindow };
 struct Plan {
@@ -351,6 +381,9 @@ struct Plan {
   Bptt bptt;        // kRecompute: gru_bptt_tc recomputes the gates, the forward keeps h only; kStoredTc: gru_bwd_tc
                     // reads the gates the forward stored; kFp32: gate kernels + FP32 GEMMs on the stored gates
   Head head;        // kWindow: fused behind the window kernel; kKernel: head_fused_kernel; kDense: dense kernels
+  bool det;         // deterministic mode: the loss sums are per-warp partials reduced in a fixed order
+  bool dgi_slices;  // the tcgen05 BPTT stores d(gi) per window step into L slices that dgi_slice_sum_kernel sums in a
+                    // fixed order, instead of adding it atomically (deterministic mode; kFp32 is ordered already)
 };
 
 static Plan make_plan(const d2d_net* n) {
@@ -361,6 +394,8 @@ static Plan make_plan(const d2d_net* n) {
   p.bptt = !(all_tc && gru && h32_64) ? Bptt::kFp32 : (p.window_tc ? Bptt::kRecompute : Bptt::kStoredTc);
   const bool head_fused = gru && h32_64 && n->O <= 16 && !n->head2;
   p.head = !head_fused ? Head::kDense : (p.window_tc ? Head::kWindow : Head::kKernel);
+  p.det = g_deterministic != 0;
+  p.dgi_slices = p.det && p.bptt != Bptt::kFp32;
   return p;
 }
 
@@ -459,12 +494,15 @@ static int launch_gru_bptt_tc_h(const d2d_net* n, const GruBpttArgs& a, cudaStre
   if (!attr) {
     D2D_CUDA(cudaFuncSetAttribute(gru_bptt_tc_kernel<H>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                   (int)tcr::Smem<H>::bytes));
+    D2D_CUDA(cudaFuncSetAttribute(gru_bptt_tc_kernel<H | kDgiSlices>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                  (int)tcr::Smem<H>::bytes));
     attr = true;
   }
   const int tiles = (a.t1 - a.t0) * ((n->B + tc::kM - 1) / tc::kM);
   if (tiles <= 0) return D2D_OK;
   const int gx = std::max(1, std::min(std::min(tiles, 148 / n->N), n->n_strips));
-  gru_bptt_tc_kernel<H><<<dim3(gx, n->N), tcr::kThreads, tcr::Smem<H>::bytes, s>>>(a);
+  if (a.slice_step) gru_bptt_tc_kernel<H | kDgiSlices><<<dim3(gx, n->N), tcr::kThreads, tcr::Smem<H>::bytes, s>>>(a);
+  else gru_bptt_tc_kernel<H><<<dim3(gx, n->N), tcr::kThreads, tcr::Smem<H>::bytes, s>>>(a);
   D2D_LAUNCHED();
   *strips = gx;
   return D2D_OK;
@@ -476,12 +514,15 @@ static int launch_gru_bwd_tc_h(const d2d_net* n, const GruBwdTcArgs& a, cudaStre
   if (!attr) {
     D2D_CUDA(cudaFuncSetAttribute(gru_bwd_tc_kernel<H>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                   (int)tcb::Smem<H>::bytes));
+    D2D_CUDA(cudaFuncSetAttribute(gru_bwd_tc_kernel<H | kDgiSlices>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                  (int)tcb::Smem<H>::bytes));
     attr = true;
   }
   const int tiles = (a.t1 - a.t0) * ((n->B + tc::kM - 1) / tc::kM);
   if (tiles <= 0) return D2D_OK;
   const int gx = std::max(1, std::min(std::min(tiles, 148 / n->N), n->n_strips));
-  gru_bwd_tc_kernel<H><<<dim3(gx, n->N), tcb::kThreads, tcb::Smem<H>::bytes, s>>>(a);
+  if (a.slice_step) gru_bwd_tc_kernel<H | kDgiSlices><<<dim3(gx, n->N), tcb::kThreads, tcb::Smem<H>::bytes, s>>>(a);
+  else gru_bwd_tc_kernel<H><<<dim3(gx, n->N), tcb::kThreads, tcb::Smem<H>::bytes, s>>>(a);
   D2D_LAUNCHED();
   *strips = gx;
   return D2D_OK;
@@ -504,6 +545,7 @@ struct Chunk {
   int Tc, halo;
   Plan plan;
   float *gi, *gh, *acts, *hs, *y1, *y2, *logits, *dl, *dy1, *dy2, *dh0, *dh1, *dgi;
+  float* dgi_s;   // plan.dgi_slices: [L][Tc][3H][N B] d(gi) of every window step, at the window's time
 };
 
 static long long floats_per_t(const d2d_net* n, bool train, const Plan& plan) {
@@ -516,6 +558,7 @@ static long long floats_per_t(const d2d_net* n, bool train, const Plan& plan) {
   if (n->arch == D2D_NET_GRU) f += train ? L * H + (plan.bptt == Bptt::kRecompute ? 0 : 4 * L * H) : 2 * H;
   if (train) f += O + H;                              // dl, dy1
   if (train && n->arch == D2D_NET_GRU) f += 2 * H + 3 * H;   // dh ping-pong, dgi
+  if (train && plan.dgi_slices) f += L * 3 * H;       // the L d(gi) slices
   return f * NB;
 }
 
@@ -527,7 +570,7 @@ static int plan_chunk(d2d_net* n, bool train, int n_t, Chunk& c) {
   const long long halo_f = (long long)halo * 3 * n->H * NB * (train ? 2 : 1);
   long long budget = n->scratch_bytes / 4;
   int Tc = (int)std::max<long long>(1, std::min<long long>(n_t, (budget - halo_f) / per_t));
-  const long long need = per_t * Tc + halo_f;
+  const long long need = per_t * Tc + halo_f + (c.plan.dgi_slices ? 8 : 0);   // + the float4 alignment below
   if (need > n->scratch_cap) {
     if (n->scratch) cudaFree(n->scratch);
     n->scratch = nullptr, n->scratch_cap = 0;
@@ -538,7 +581,7 @@ static int plan_chunk(d2d_net* n, bool train, int n_t, Chunk& c) {
   float* p = n->scratch;
   auto take = [&](long long f) { float* q = p; p += f; return q; };
   const long long H = n->H, O = n->O, L = n->L;
-  c.gi = c.gh = c.acts = c.hs = c.dl = c.dy1 = c.dh0 = c.dh1 = c.dgi = nullptr;
+  c.gi = c.gh = c.acts = c.hs = c.dl = c.dy1 = c.dh0 = c.dh1 = c.dgi = c.dgi_s = nullptr;
   if (n->arch == D2D_NET_GRU) {
     c.gi = take((long long)(Tc + halo) * 3 * H * NB);
     c.gh = take((long long)Tc * 3 * H * NB);
@@ -560,7 +603,10 @@ static int plan_chunk(d2d_net* n, bool train, int n_t, Chunk& c) {
     if (n->arch == D2D_NET_GRU) {
       c.dh0 = take((long long)Tc * H * NB);
       c.dh1 = take((long long)Tc * H * NB);
+      // dgi_slice_sum_kernel moves float4s (3H N B is a multiple of 4 for H = 32 / 64): 16-byte aligned starts
+      if (c.plan.dgi_slices) p += (4 - ((p - n->scratch) & 3)) & 3;
       c.dgi = take((long long)(Tc + halo) * 3 * H * NB);
+      if (c.plan.dgi_slices) c.dgi_s = take((long long)L * Tc * 3 * H * NB);
     }
   }
   return D2D_OK;
@@ -734,8 +780,11 @@ static int backward_chunk(d2d_net* n, const float* params, const float* x, int x
     a.x = dy1, a.y = make_view(dh_cur, H * NB, -c0, N, H, B), a.epilogue = kEpiNone, a.t0 = c0, a.t1 = c1;
     if ((rc = launch_dense(n, a, H, s))) return rc;
   }
-  D2D_CUDA(cudaMemsetAsync(c.dgi, 0, (size_t)(c.Tc + halo) * 3 * H * NB * 4, s));
+  // d(gi) slices: every element dgi_slice_sum_kernel reads is stored once, and it writes all of c.dgi
+  if (!c.plan.dgi_slices) D2D_CUDA(cudaMemsetAsync(c.dgi, 0, (size_t)(c.Tc + halo) * 3 * H * NB * 4, s));
   const View dgi = make_view(c.dgi, 3 * H * NB, -(c0 - halo), N, 3 * H, B);
+  const View dgi_s = c.plan.dgi_slices ? make_view(c.dgi_s, 3 * H * NB, -c0, N, 3 * H, B) : dgi;   // slice 0
+  const long long slice_step = c.plan.dgi_slices ? (long long)c.Tc * 3 * H * NB : 0;
   const View dgh = make_view(c.gh, 3 * H * NB, -c0, N, 3 * H, B);
   Wt whh{&n->o_whh, &n->o_bhh, nullptr, H, 3 * H};
   if (c.plan.bptt != Bptt::kFp32) {
@@ -749,7 +798,7 @@ static int backward_chunk(d2d_net* n, const float* params, const float* x, int x
       ba.x = xin;
       ba.hs = make_view(c.hs, H * NB, -c0, N, H, B);
       ba.dh = make_view(dh_cur, H * NB, -c0, N, H, B);
-      ba.dgi = dgi;
+      ba.dgi = dgi_s;
       ba.w = params, ba.w_agent_stride = n->stride;
       for (int g = 0; g < N; ++g) {
         ba.wih_off[g] = n->o_wih[g], ba.whh_off[g] = n->o_whh[g], ba.bih_off[g] = n->o_bih[g], ba.bhh_off[g] = n->o_bhh[g];
@@ -769,6 +818,7 @@ static int backward_chunk(d2d_net* n, const float* params, const float* x, int x
       (void)inv_rows;
       ba.L = L, ba.B = B, ba.t0 = c0, ba.t1 = c1;
       ba.partial = n->partial, ba.part_stride = n->part_stride;
+      ba.slice_step = slice_step;
       rc = n->H == 32 ? launch_gru_bptt_tc_h<32>(n, ba, s, &strips) : launch_gru_bptt_tc_h<64>(n, ba, s, &strips);
     } else {
       // gru_bwd_tc reads the gates the forward stored; it leaves d(gh) of step s in the first 3H features of that
@@ -778,15 +828,23 @@ static int backward_chunk(d2d_net* n, const float* params, const float* x, int x
       ba.acts = make_view(c.acts, 4 * H * NB, -c0, N, 4 * H, B);
       ba.hs = make_view(c.hs, H * NB, -c0, N, H, B);
       ba.dh = make_view(dh_cur, H * NB, -c0, N, H, B);
-      ba.dgi = dgi;
+      ba.dgi = dgi_s;
       ba.w = params, ba.w_agent_stride = n->stride;
       for (int g = 0; g < N; ++g) ba.whh_off[g] = n->o_whh[g];
       ba.acts_step = (long long)c.Tc * 4 * H * NB, ba.hs_step = (long long)c.Tc * H * NB;
       ba.L = L, ba.B = B, ba.t0 = c0, ba.t1 = c1;
       ba.partial = n->partial, ba.part_stride = n->part_stride;
+      ba.slice_step = slice_step;
       rc = n->H == 32 ? launch_gru_bwd_tc_h<32>(n, ba, s, &strips) : launch_gru_bwd_tc_h<64>(n, ba, s, &strips);
     }
     if (rc) return rc;
+    if (c.plan.dgi_slices) {
+      const long long per_t4 = 3 * H * NB / 4, cnt = (long long)(c1 - c0 + halo) * per_t4;
+      dgi_slice_sum_kernel<<<grid_for(cnt, 256), 256, 0, s>>>(reinterpret_cast<const float4*>(c.dgi_s),
+                                                              reinterpret_cast<float4*>(c.dgi), L, c1 - c0,
+                                                              slice_step / 4, per_t4);
+      D2D_LAUNCHED();
+    }
     if (strips > 0 && (rc = launch_wreduce(n, whh, false, strips, grads, s))) return rc;
   }
   for (int st = L - 1; st >= 0 && c.plan.bptt == Bptt::kFp32; --st) {
@@ -887,7 +945,7 @@ extern "C" int d2d_net_create(const d2d_net_config* cfg, d2d_net** out) {
 
 extern "C" int d2d_net_destroy(d2d_net* n) {
   if (!n) return D2D_OK;
-  cudaFree(n->scratch), cudaFree(n->partial), cudaFree(n->gi_ring);
+  cudaFree(n->scratch), cudaFree(n->partial), cudaFree(n->gi_ring), cudaFree(n->red);
   delete n;
   return D2D_OK;
 }
@@ -1102,8 +1160,18 @@ extern "C" int d2d_ppo_policy_grad(d2d_net* n, const float* params, const float*
     h.weight_per_agent = weight_per_agent, h.cycle = cycle, h.ratio_out = ratio_out, h.inv_rows = inv_rows;
     h.cliprange = cliprange, h.beta = beta, h.loss_sums = loss_sums;
     const long long rows = (long long)(c1 - c0) * n->B;
-    ppo_dlogits_kernel<<<grid_for(rows, 128), 128, 0, s>>>(h);
-    D2D_LAUNCHED();
+    const int gx = grid_for(rows, 128);
+    if (c.plan.det) {   // per-warp partial sums, then the fixed-order reduction into loss_sums
+      double* part;
+      if ((rc = reduce_scratch(n, 2ll * n->N * gx * 4, &part))) return rc;
+      D2D_CUDA(cudaMemsetAsync(part, 0, sizeof(double) * 2 * n->N * gx * 4, s));
+      ppo_dlogits_part_kernel<<<gx, 128, 0, s>>>(h, part);
+      D2D_LAUNCHED();
+      if ((rc = launch_sum_partials(part, n->N, gx * 4, 2, loss_sums, s))) return rc;
+    } else {
+      ppo_dlogits_kernel<<<gx, 128, 0, s>>>(h);
+      D2D_LAUNCHED();
+    }
     if ((rc = backward_chunk(n, params, x, x_lead, c0, c1, c, grads, inv_rows, s))) return rc;
   }
   return D2D_OK;
@@ -1132,8 +1200,17 @@ extern "C" int d2d_value_grad(d2d_net* n, const float* params, const float* x, i
     m.B = n->B, m.t0 = c0, m.t1 = c1, m.inv_rows = inv_rows, m.loss_sum = loss_sum;
     m.value_out = value_out, m.out_t_stride = NB;
     const long long rows = (long long)(c1 - c0) * n->B;
-    mse_dvalue_kernel<<<dim3(grid_for(rows, 128), n->N), 128, 0, s>>>(m);
-    D2D_LAUNCHED();
+    const int gx = grid_for(rows, 128);
+    if (c.plan.det) {
+      double* part;
+      if ((rc = reduce_scratch(n, (long long)n->N * gx * 4, &part))) return rc;
+      mse_dvalue_part_kernel<<<dim3(gx, n->N), 128, 0, s>>>(m, part);
+      D2D_LAUNCHED();
+      if ((rc = launch_sum_partials(part, n->N, gx * 4, 1, loss_sum, s))) return rc;
+    } else {
+      mse_dvalue_kernel<<<dim3(gx, n->N), 128, 0, s>>>(m);
+      D2D_LAUNCHED();
+    }
     if ((rc = backward_chunk(n, params, x, x_lead, c0, c1, c, grads, inv_rows, s))) return rc;
   }
   return D2D_OK;
@@ -1150,7 +1227,10 @@ extern "C" int d2d_adam_step_eps(float* params, float* m, float* v, const float*
   D2D_REQUIRE(max_norm <= 0.f || sqnorm, "d2d_adam_step: clipping needs the sqnorm scratch buffer");
   cudaStream_t s = as_stream(stream);
   const int gx = grid_for(per_agent, 256);
-  if (max_norm > 0.f) {
+  if (max_norm > 0.f && g_deterministic) {   // one block per agent, fixed tree: no atomics, no zeroing
+    grad_sqnorm_tree_kernel<<<N, 512, 0, s>>>(grads, per_agent, sqnorm);
+    D2D_LAUNCHED();
+  } else if (max_norm > 0.f) {
     D2D_CUDA(cudaMemsetAsync(sqnorm, 0, sizeof(double) * N, s));
     grad_sqnorm_kernel<<<dim3(gx, N), 256, 0, s>>>(grads, per_agent, sqnorm);
     D2D_LAUNCHED();
@@ -1220,8 +1300,17 @@ extern "C" int d2d_q_grad(d2d_net* n, const float* params, const float* x, int x
     q.actions = actions, q.target = target, q.q_out = q_out, q.O = n->O, q.B = n->B, q.t0 = c0, q.t1 = c1;
     q.loss_kind = loss_kind, q.inv_rows = inv_rows, q.loss_sum = loss_sum;
     const long long rows = (long long)(c1 - c0) * n->B;
-    q_loss_grad_kernel<<<dim3(grid_for(rows, 128), n->N), 128, 0, s>>>(q);
-    D2D_LAUNCHED();
+    const int gx = grid_for(rows, 128);
+    if (c.plan.det) {
+      double* part;
+      if ((rc = reduce_scratch(n, (long long)n->N * gx * 4, &part))) return rc;
+      q_loss_grad_part_kernel<<<dim3(gx, n->N), 128, 0, s>>>(q, part);
+      D2D_LAUNCHED();
+      if ((rc = launch_sum_partials(part, n->N, gx * 4, 1, loss_sum, s))) return rc;
+    } else {
+      q_loss_grad_kernel<<<dim3(gx, n->N), 128, 0, s>>>(q);
+      D2D_LAUNCHED();
+    }
     if ((rc = backward_chunk(n, params, x, x_lead, c0, c1, c, grads, inv_rows, s))) return rc;
   }
   return D2D_OK;
@@ -1246,6 +1335,22 @@ extern "C" int d2d_replay_gather(const float* obs_ring, const uint8_t* act_ring,
   return D2D_OK;
 }
 
+// deterministic mode of the returns scans: the per-warp statistics go to a stream-ordered scratch (there is no handle
+// to own one) and are added to a.stats in a fixed order
+template <int MODE>
+static int returns_scan_partials(ScanArgs a, cudaStream_t s) {
+  const int gx = grid_for(a.B, 128), n_parts = gx * 4;
+  double* part = nullptr;
+  D2D_CUDA(cudaMallocAsync((void**)&part, sizeof(double) * 4 * a.n_cols * n_parts, s));
+  double* stats = a.stats;
+  a.stats = part;
+  returns_scan_kernel<MODE><<<dim3(gx, a.n_cols), 128, 0, s>>>(a);
+  D2D_LAUNCHED();
+  const int rc = launch_sum_partials(part, a.n_cols, n_parts, 4, stats, s);
+  D2D_CUDA(cudaFreeAsync(part, s));
+  return rc;
+}
+
 extern "C" int d2d_returns_scan(const int32_t* reward, const float* value, double* adv_raw, double* ret_raw,
                                 double* stats, int T, int B, int n_cols, double gamma, double lam, int last_shard,
                                 void* stream) {
@@ -1256,6 +1361,7 @@ extern "C" int d2d_returns_scan(const int32_t* reward, const float* value, doubl
   memset(&a, 0, sizeof(a));
   a.reward_i = reward, a.value = value, a.adv_raw = adv_raw, a.ret_raw = ret_raw, a.stats = stats;
   a.T = T, a.B = B, a.n_cols = n_cols, a.gamma = gamma, a.lam = lam, a.last_env_is_global_last = last_shard;
+  if (g_deterministic) return returns_scan_partials<kScanRaw | kScanPartials>(a, as_stream(stream));
   returns_scan_kernel<kScanRaw><<<dim3(grid_for(B, 128), n_cols), 128, 0, as_stream(stream)>>>(a);
   D2D_LAUNCHED();
   return D2D_OK;
@@ -1272,6 +1378,7 @@ extern "C" int d2d_returns_stats(const int32_t* reward, const float* value, doub
   memset(&a, 0, sizeof(a));
   a.reward_i = reward, a.value = value, a.stats = stats, a.want_adv = want_adv, a.want_ret = want_ret;
   a.T = T, a.B = B, a.n_cols = n_cols, a.gamma = gamma, a.lam = lam, a.last_env_is_global_last = last_shard;
+  if (g_deterministic) return returns_scan_partials<kScanStats | kScanPartials>(a, as_stream(stream));
   returns_scan_kernel<kScanStats><<<dim3(grid_for(B, 128), n_cols), 128, 0, as_stream(stream)>>>(a);
   D2D_LAUNCHED();
   return D2D_OK;

@@ -257,7 +257,11 @@ __global__ void policy_head_kernel(const HeadArgs a) {
 // d(loss)/d(logits) of  loss = -mean_rows(min(ratio w, clip(ratio) w)) - beta mean_rows(entropy)
 // (reference d2d_ppo.py:201-207, ippo.py:196-202).  One thread per (time, env) handles ALL agents so that the
 // HAPPO weight M_j = adv * prod_{i before j in cycle} ratio_i (d2d_ppo.py:427-436) is a running product.
-__global__ void ppo_dlogits_kernel(const HeadArgs a) {
+// part == nullptr: the loss sums are added to a.loss_sums with fp64 atomics (order not fixed).  Deterministic mode:
+// warp w of the grid adds its sums to part[g][w][2] (zeroed by the caller, one writer per slot) and
+// sum_partials_kernel reduces them in a fixed order.
+template <bool PART>
+__device__ __forceinline__ void ppo_dlogits_body(const HeadArgs& a, double* part) {
   const long long n = (long long)(a.t1 - a.t0) * a.B;
   const long long n_round = (n + blockDim.x - 1) / blockDim.x * blockDim.x;   // whole warps stay in the loop
   for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < n_round;
@@ -295,8 +299,14 @@ __global__ void ppo_dlogits_kernel(const HeadArgs a) {
         s1 += __shfl_down_sync(0xFFFFFFFFu, s1, o);
       }
       if ((threadIdx.x & 31) == 0) {
-        atomicAdd(&a.loss_sums[2 * g], s0);
-        atomicAdd(&a.loss_sums[2 * g + 1], s1);
+        if constexpr (PART) {
+          const int n_warps = gridDim.x * (blockDim.x >> 5);
+          double* q = part + 2 * ((long long)g * n_warps + ((blockIdx.x * blockDim.x + threadIdx.x) >> 5));
+          q[0] += s0, q[1] += s1;
+        } else {
+          atomicAdd(&a.loss_sums[2 * g], s0);
+          atomicAdd(&a.loss_sums[2 * g + 1], s1);
+        }
       }
       if (!live) continue;
       // ---- d/dp, then through the output activation ----
@@ -339,6 +349,8 @@ __global__ void ppo_dlogits_kernel(const HeadArgs a) {
     }
   }
 }
+__global__ void ppo_dlogits_kernel(const HeadArgs a) { ppo_dlogits_body<false>(a, nullptr); }
+__global__ void ppo_dlogits_part_kernel(const HeadArgs a, double* part) { ppo_dlogits_body<true>(a, part); }
 
 // critic: d(mse)/d(value) = 2 (v - target) / R ; loss sum accumulated in fp64
 struct MseArgs {
@@ -355,7 +367,9 @@ struct MseArgs {
   long long out_t_stride;
 };
 
-__global__ void mse_dvalue_kernel(const MseArgs a) {
+// part != nullptr (deterministic mode): warp w of agent g's blocks stores its sum to part[g][w] instead of the atomic
+template <bool PART>
+__device__ __forceinline__ void mse_dvalue_body(const MseArgs& a, double* part) {
   const int g = blockIdx.y;
   const long long n = (long long)(a.t1 - a.t0) * a.B;
   double local = 0.0;
@@ -370,8 +384,13 @@ __global__ void mse_dvalue_kernel(const MseArgs a) {
     if (a.value_out) a.value_out[(long long)(t + a.tgt_t_off) * a.out_t_stride + (long long)g * a.B + b] = v;
   }
   for (int o = 16; o > 0; o >>= 1) local += __shfl_down_sync(0xFFFFFFFFu, local, o);
-  if ((threadIdx.x & 31) == 0) atomicAdd(&a.loss_sum[g], local);
+  if ((threadIdx.x & 31) == 0) {
+    if constexpr (PART) part[(long long)g * gridDim.x * (blockDim.x >> 5) + ((blockIdx.x * blockDim.x + threadIdx.x) >> 5)] = local;
+    else atomicAdd(&a.loss_sum[g], local);
+  }
 }
+__global__ void mse_dvalue_kernel(const MseArgs a) { mse_dvalue_body<false>(a, nullptr); }
+__global__ void mse_dvalue_part_kernel(const MseArgs a, double* part) { mse_dvalue_body<true>(a, part); }
 
 // ------------------------------------------------------------------------------------------------
 // lambda-returns (compute_gae, d2d_ppo.py:100-110) and discounted returns (discount_rewards, :112-124)
@@ -397,6 +416,9 @@ struct ScanArgs {
 };
 
 enum { kScanRaw = 0, kScanStats = 1, kScanEmit = 2 };
+// or-ed into kScanRaw / kScanStats (deterministic mode): warp w of column g's blocks stores its four sums to
+// a.stats[g][w][4] (a scratch of n_cols x gridDim.x x 4 warps) for sum_partials_kernel instead of the atomics
+constexpr int kScanPartials = 4;
 
 // One thread per (column, env) walks the episode backwards in float64 as numpy does.  The chain is serial and short of
 // arithmetic, so the kernel lives on memory-level parallelism and on a lean instruction stream:
@@ -407,8 +429,9 @@ enum { kScanRaw = 0, kScanStats = 1, kScanEmit = 2 };
 //  * the episode-end row (t = T - 1) is peeled, the main loop runs whole batches without predicates.
 // Normalisation multiplies by the float64 reciprocal of the std (one division per thread instead of one per element;
 // the result differs from numpy's quotient by at most one float64 ulp BEFORE the cast to fp32).
-template <int MODE>
+template <int MODE_BITS>
 __global__ void __launch_bounds__(128, 7) returns_scan_kernel(const ScanArgs a) {
+  constexpr int MODE = MODE_BITS & 3;
   const int g = blockIdx.y;
   const bool do_adv = MODE == kScanRaw ? a.adv_raw != nullptr : (MODE == kScanStats ? a.want_adv : a.adv_out != nullptr);
   const bool do_ret = MODE == kScanRaw ? a.ret_raw != nullptr : (MODE == kScanStats ? a.want_ret : a.ret_out != nullptr);
@@ -514,7 +537,54 @@ __global__ void __launch_bounds__(128, 7) returns_scan_kernel(const ScanArgs a) 
   for (int k = 0; k < 4; ++k) {
     double v = vals[k];
     for (int o = 16; o > 0; o >>= 1) v += __shfl_down_sync(0xFFFFFFFFu, v, o);
-    if ((threadIdx.x & 31) == 0 && v != 0.0) atomicAdd(&a.stats[4 * g + k], v);
+    if constexpr ((MODE_BITS & kScanPartials) != 0) {
+      const long long w = (long long)g * gridDim.x * (blockDim.x >> 5) + ((blockIdx.x * blockDim.x + threadIdx.x) >> 5);
+      if ((threadIdx.x & 31) == 0) a.stats[4 * w + k] = v;
+    } else {
+      if ((threadIdx.x & 31) == 0 && v != 0.0) atomicAdd(&a.stats[4 * g + k], v);
+    }
+  }
+}
+
+// out[grp][k] += sum over p = 0 .. n_parts - 1 of part[grp][p][k], in a fixed order: block = (grp, k), thread i sums
+// p = i, i + 256, ... in turn, then a fixed tree over the 256 threads.  The deterministic mode's replacement of the
+// fp64 atomics of the loss, returns-statistics and gradient-norm sums.
+__global__ void __launch_bounds__(256) sum_partials_kernel(const double* __restrict__ part, int n_parts, int n_vals,
+                                                           double* __restrict__ out) {
+  __shared__ double sh[256];
+  const int grp = blockIdx.x / n_vals, k = blockIdx.x % n_vals;
+  const double* p = part + (long long)grp * n_parts * n_vals + k;
+  double s = 0.0;
+  for (int i = threadIdx.x; i < n_parts; i += 256) s += p[(long long)i * n_vals];
+  sh[threadIdx.x] = s;
+  __syncthreads();
+  for (int w = 128; w > 0; w >>= 1) {
+    if (threadIdx.x < w) sh[threadIdx.x] += sh[threadIdx.x + w];
+    __syncthreads();
+  }
+  if (threadIdx.x == 0) out[blockIdx.x] += sh[0];
+}
+
+// d(gi) of the observations [c0 - halo, c1) of a chunk from the L d(gi) slices the SLICES BPTT kernels stored
+// (gru_bptt_tc.cuh, gru_bwd_tc.cuh): slice s holds, at the local time l of window t = c0 + l, the d(gi) that window
+// step s gives observation t - (L - 1 - s).  Hence, with halo = L - 1 and o the local time of the observation,
+//   dgi[o] = sum_{s = 0 .. L - 1, 0 <= o - s < n_win} slice_s[o - s]
+// summed in increasing s: the same terms as the atomic accumulation, in a fixed order.  Every element is written.
+//   slices [L][n_win_cap][per_t] floats;  dgi [n_win + L - 1][per_t];  per_t = 3H N B (a multiple of 4)
+__global__ void dgi_slice_sum_kernel(const float4* __restrict__ slices, float4* __restrict__ dgi, int L, int n_win,
+                                     long long slice_t, long long per_t4) {
+  const long long n = (long long)(n_win + L - 1) * per_t4;
+  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) {
+    const int o = (int)(i / per_t4);
+    const long long e = i % per_t4;
+    float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
+    for (int s = 0; s < L; ++s) {
+      const int l = o - s;
+      if (l < 0 || l >= n_win) continue;
+      const float4 v = __ldcs(slices + (long long)s * slice_t + (long long)l * per_t4 + e);
+      acc.x += v.x, acc.y += v.y, acc.z += v.z, acc.w += v.w;
+    }
+    dgi[i] = acc;
   }
 }
 
@@ -575,6 +645,26 @@ __global__ void normalize_kernel(const NormArgs a) {
 // ------------------------------------------------------------------------------------------------
 // optimiser: per-agent gradient norm (clip_grad_norm_, d2d_ppo.py:211,445) and torch.optim.Adam defaults
 // ------------------------------------------------------------------------------------------------
+// deterministic mode: one 512-thread block per agent; thread i sums elements i, i + 512, ... in turn, then a fixed tree;
+// out[agent] is stored (no zeroing needed)
+__global__ void __launch_bounds__(512) grad_sqnorm_tree_kernel(const float* __restrict__ g, long long per_agent,
+                                                               double* __restrict__ out) {
+  __shared__ double sh[512];
+  const float* p = g + blockIdx.x * per_agent;
+  double s = 0.0;
+  for (long long i = threadIdx.x; i < per_agent; i += 512) {
+    const double v = p[i];
+    s += v * v;
+  }
+  sh[threadIdx.x] = s;
+  __syncthreads();
+  for (int w = 256; w > 0; w >>= 1) {
+    if (threadIdx.x < w) sh[threadIdx.x] += sh[threadIdx.x + w];
+    __syncthreads();
+  }
+  if (threadIdx.x == 0) out[blockIdx.x] = sh[0];
+}
+
 __global__ void grad_sqnorm_kernel(const float* __restrict__ g, long long per_agent, double* __restrict__ out) {
   const int a = blockIdx.y;
   double s = 0.0;

@@ -307,6 +307,24 @@ int d2d_net_check_inputs(const d2d_net* net, const float* x, int x_lead, int t0,
 int d2d_set_kernel_switch(int which, int enabled);
 int d2d_get_kernel_switch(int which);
 
+/* Deterministic mode (off by default; process-wide, read at every call, so it may be changed between calls).
+ * With it on, every floating-point sum of the learner runs in a fixed order instead of through atomics:
+ *   - the d(gi) of the tcgen05 BPTT kernels: window step s stores into slice s of an [L][Tc][3H][N B] scratch and
+ *     one more streaming kernel per chunk sums the L slices in increasing s (the stored-gate kernel also issues its
+ *     tensor-core MMAs from one warp in a fixed order);
+ *   - the loss sums of d2d_ppo_policy_grad, d2d_value_grad and d2d_q_grad, and the statistics of d2d_returns_scan /
+ *     d2d_returns_stats: per-warp partials, then one small fixed-order reduction launch per call (per chunk for the
+ *     losses); the returns scans take their partials from cudaMallocAsync / cudaFreeAsync on the call's stream;
+ *   - the clip_grad_norm_ square norm of d2d_adam_step*: one block per agent with a fixed tree (same launch count).
+ * Guarantee: the same build, GPU model, seeds, n_envs, scratch_bytes and a single rank give bit-identical
+ * parameters, Adam moments, losses, scores and test results from run to run and from process to process.
+ * Nothing is claimed across GPU models, scratch_bytes (it sets the chunking) or world sizes.  The results equal the
+ * default mode's to rounding.  Cost: L x the d(gi) scratch of a chunk (so a fixed scratch_bytes takes smaller
+ * chunks), one more pass over that scratch per chunk, and the few tiny launches above.
+ * With the mode off, every launch is the one the library makes without this mode. */
+int d2d_set_deterministic(int enabled);
+int d2d_get_deterministic(void);
+
 /* Rollout step (PPO.select_action's network call, d2d_ppo.py:302-303): forward of the single time block t on
  * the UNPADDED window.  The input projections of the previous L - 1 observations are kept in a ring inside the
  * handle, so each observation is projected once per episode instead of L times.  Call with t = 0, 1, 2, ... in
