@@ -13,7 +13,7 @@ import numpy as np
 import torch
 
 from .. import _lib as L
-from . import _dist
+from . import _ckpt, _dist
 from ._nets import NetSet, action_dtype, returns_norm_stats
 
 
@@ -61,6 +61,8 @@ class PPOBase:
                                policy_lr, scratch_bytes, self._gen, inputs_bf16_exact=self.exact_obs)
         self._act_dtype = action_dtype(self.dist_kind, self.n_actions)
         self._iter = 0
+        self._progress = self._fresh_progress()
+        self._float_lists = _ckpt.FloatLists()
         # rows of the global batch (all ranks): shards may be unequal (_dist.shard leaves a remainder)
         rows = torch.tensor([float(self.B * self.T)], dtype=torch.float64, device=self.device)
         self.rows_global = int(_dist.all_reduce_sum_(rows).item())
@@ -90,6 +92,47 @@ class PPOBase:
         for i in range(self.n_agents):
             self.policies.load_state_dict(i, torch.load(f"{checkpoint_path}/agent_{i}.pth", map_location="cpu"))
         print("Models loaded!")
+
+    # ------------------------------------------------------------------ training state (resume an interrupted run)
+    _NET_SETS = ("policies",)          # subclasses add their value network
+    _REPLICATED_LISTS = ("score_test_list", "policy_loss_list", "value_loss_list")
+
+    def _extra_state(self):
+        return {}
+
+    def _load_extra_state(self, d):
+        pass
+
+    def save_training_state(self, path):
+        """Write everything that decides how ``train`` continues into the directory ``path``: both net sets with their
+        Adam state, the sampling-stream counter, the env's episode counter, the position of the train loop and the
+        lists ``train`` returns.  Call it between iterations; the next rollout resets the envs, so their buffers are
+        not part of the state.  Collective when a process group is active."""
+        p, f = self._progress, self._float_lists
+        replicated = {"nets": {k: getattr(self, k).training_state() for k in self._NET_SETS},
+                      "iter": self._iter, "env_episode": self.env.episode, "next_iter": p["next_iter"],
+                      "stopped": p["stopped"], **{k: f.to_tensor(k, p[k]) for k in self._REPLICATED_LISTS},
+                      **self._extra_state()}
+        local = {"scores_episode": f.to_tensor("scores_episode", p["scores_episode"])}   # each rank scores its own envs
+        _ckpt.save(path, _ckpt.config(self), replicated, local, self.device)
+
+    def load_training_state(self, path):
+        """Restore the state ``save_training_state`` wrote; ValueError if the stored run was set up differently."""
+        rep, loc = _ckpt.load(path, _ckpt.config(self))
+        for k in self._NET_SETS:
+            getattr(self, k).load_training_state(rep["nets"][k])
+        self._iter = int(rep["iter"])
+        self.env.set_episode(int(rep["env_episode"]) + 1)
+        self._load_extra_state(rep)
+        f = self._float_lists
+        self._progress = {"next_iter": int(rep["next_iter"]), "stopped": bool(rep["stopped"]),
+                          "scores_episode": f.to_list("scores_episode", loc["scores_episode"]),
+                          **{k: f.to_list(k, rep[k]) for k in self._REPLICATED_LISTS}}
+
+    @staticmethod
+    def _fresh_progress():
+        return {"next_iter": 0, "stopped": False, "scores_episode": [], "score_test_list": [], "policy_loss_list": [],
+                "value_loss_list": []}
 
     # ------------------------------------------------------------------ rollout
     def _sample_seed(self):
@@ -190,3 +233,34 @@ class PPOBase:
         if np.max(score_test_list) == score_test and self.save_path is not None:
             self.save(self.save_path)
         return bool((score_test == 1) & bool(self.early_stopping))
+
+    def _train(self, num_iter, n_epoch, num_episodes, test_freq, checkpoint_path, checkpoint_freq, resume):
+        """The train loop of both learners; ``_epoch_losses`` runs one epoch and returns the (policy, value) loss
+        entries the reference appends.  checkpoint_freq = k writes the training state after iterations 0, k, 2k, ... (their
+        epochs and tests done), after the last one and when early stopping fires; resume continues from the state in
+        checkpoint_path if there is one."""
+        if (checkpoint_freq or resume) and checkpoint_path is None:
+            raise ValueError("checkpoint_freq and resume need a checkpoint_path")
+        if resume and _ckpt.exists(checkpoint_path):
+            self.load_training_state(checkpoint_path)
+        else:
+            self._progress = self._fresh_progress()
+        p = self._progress
+        it = p["next_iter"]
+        while it < num_iter and not p["stopped"]:
+            scores = self.create_rollouts(num_episodes)[6].tolist()
+            p["scores_episode"] += scores
+            for epoch in range(n_epoch):
+                ploss, vloss = self._epoch_losses()
+                p["policy_loss_list"].append(ploss)
+                p["value_loss_list"].append(vloss)
+                if self._maybe_test(it, epoch, test_freq, scores, p["score_test_list"]):
+                    p["stopped"] = True
+                    break
+            p["next_iter"] = it + 1
+            # after iterations 0, k, 2k, ...: with k = test_freq right after each test iteration, so that a best model
+            # its tests saved belongs to the stored run
+            if checkpoint_freq and (it % checkpoint_freq == 0 or it + 1 == num_iter or p["stopped"]):
+                self.save_training_state(checkpoint_path)
+            it += 1
+        return p["scores_episode"], p["score_test_list"], p["policy_loss_list"], p["value_loss_list"]

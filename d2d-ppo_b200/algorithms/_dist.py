@@ -1,7 +1,10 @@
 """Multi-GPU plumbing: env instances are sharded across ranks (no data-path collective); the only exchanges are
-the PPO gradient all-reduce, the (sum, sum of squares) of the return statistics, and the HAPPO agent order.
+the PPO gradient all-reduce, the (sum, sum of squares) of the return statistics, and the HAPPO agent order (plus, at a
+training-state checkpoint, one broadcast and two all-reduces of a failure count).
 Works over NCCL (one rank per GPU) and over gloo on CPU tensors (the world_size-2 tests)."""
 from __future__ import annotations
+
+import os
 
 import numpy as np
 import torch
@@ -33,6 +36,14 @@ def broadcast_order(order, device):
     if active():
         dist.broadcast(t, src=0)
     return t
+
+
+def broadcast_token(device):
+    """A random 48-bit integer drawn by rank 0 and shared by every rank (names the files of one checkpoint)."""
+    t = torch.tensor([int.from_bytes(os.urandom(6), "little")], dtype=torch.int64, device=device)
+    if active():
+        dist.broadcast(t, src=0)
+    return int(t.item())
 
 
 def shard(n_total, r=None, w=None):

@@ -140,6 +140,30 @@ class NetSet:
             blk[off:off + rows * cols] = t
         self.params[agent].copy_(blk.to(self.device))
 
+    def training_state(self):
+        """Parameters, Adam moments and step count as CPU copies (the ``agent_{i}.pth`` files hold the parameters
+        only).  A handle that aliases another net set's buffers has nothing of its own: {}."""
+        if self._owner is not None:
+            return {}
+        return {"params": self.params.cpu(), "adam_m": self.adam_m.cpu(), "adam_v": self.adam_v.cpu(),
+                "adam_step": int(self.adam_step)}
+
+    def load_training_state(self, d):
+        """Inverse of ``training_state``: copies into the existing buffers, so handles that alias them see the
+        restored values."""
+        if self._owner is not None:
+            if d:
+                raise ValueError("this handle aliases another net set's parameters: load the owner")
+            return
+        for name in ("params", "adam_m", "adam_v"):
+            t = d[name]
+            if tuple(t.shape) != tuple(self.params.shape) or t.dtype != self.params.dtype:
+                raise ValueError(f"{name}: expected {self.params.dtype} {tuple(self.params.shape)}, got "
+                                 f"{t.dtype} {tuple(t.shape)}")
+        for name in ("params", "adam_m", "adam_v"):
+            getattr(self, name).copy_(d[name])
+        self.adam_step = int(d["adam_step"])
+
     def tensor_view(self, buf, agent, name):
         off, rows, cols = self._layout[agent][self.keys.index(name)]
         v = buf[agent, off:off + rows * cols]

@@ -15,12 +15,14 @@ import numpy as np
 import torch
 
 from .. import _lib as L
-from . import _dist
+from . import _ckpt, _dist
 from ._base import PPOBase
 from ._nets import NetSet, returns_emit, returns_stats
 
 
 class D2DPPO(PPOBase):
+    _NET_SETS = ("policies", "critic")
+
     def __init__(self, env, hidden_size=128, gamma=0.99, policy_lr=1e-3, value_lr=1e-3, beta_entropy=0.01, device=None,
                  useRNN=False, save_path=None, combinatorial=False, history_len=10, early_stopping=True,
                  *, seed=0, scratch_bytes=0):
@@ -84,15 +86,18 @@ class D2DPPO(PPOBase):
         order = cyc.tolist()
         return [ploss[i].item() for i in order], (vsum[0] / rows).item()
 
-    def train(self, num_iter, num_episodes=None, n_epoch=4, test_freq=100):
-        scores_episode, score_test_list, policy_loss_list, value_loss_list = [], [], [], []
-        for it in range(num_iter):
-            scores = self.create_rollouts(num_episodes)[6].tolist()
-            scores_episode += scores
-            for epoch in range(n_epoch):
-                ploss_agents, vloss = self.update_epoch()
-                policy_loss_list.append(ploss_agents)
-                value_loss_list.append(vloss)
-                if self._maybe_test(it, epoch, test_freq, scores, score_test_list):
-                    return scores_episode, score_test_list, policy_loss_list, value_loss_list
-        return scores_episode, score_test_list, policy_loss_list, value_loss_list
+    def _epoch_losses(self):
+        return self.update_epoch()                         # ([N] policy losses in cycle order, value loss)
+
+    def _extra_state(self):
+        return {"np_random": _ckpt.plain(self._np_rng.get_state(legacy=False))}
+
+    def _load_extra_state(self, d):
+        self._np_rng.set_state(d["np_random"])
+
+    def train(self, num_iter, num_episodes=None, n_epoch=4, test_freq=100, *, checkpoint_path=None, checkpoint_freq=0,
+              resume=False):
+        """Returns (scores_episode, score_test_list, policy_loss_list, value_loss_list).  checkpoint_freq = k > 0
+        writes the training state (with the global ``np.random`` state) into checkpoint_path after iterations
+        0, k, 2k, ...; resume=True continues the run stored there (``PPOBase._train``)."""
+        return self._train(num_iter, n_epoch, num_episodes, test_freq, checkpoint_path, checkpoint_freq, resume)

@@ -19,6 +19,8 @@ from ._nets import NetSet, returns_emit, returns_stats
 
 
 class iPPO(PPOBase):
+    _NET_SETS = ("policies", "values")
+
     def __init__(self, env, hidden_size=128, gamma=0.99, policy_lr=1e-3, value_lr=1e-3, device=None, useRNN=False,
                  save_path=None, combinatorial=False, history_len=10, early_stopping=True, *, seed=0, scratch_bytes=0):
         self._setup(env, hidden_size, gamma, policy_lr, value_lr, device, useRNN, save_path, combinatorial,
@@ -74,16 +76,13 @@ class iPPO(PPOBase):
         ploss = (-(sums[:, 0] / rows) - beta * sums[:, 1] / rows).tolist()
         return ploss, (vsum / rows).tolist()
 
-    def train(self, num_iter, n_epoch=4, num_episodes=None, test_freq=100):
-        scores_episode, score_test_list, policy_loss_list, value_loss_list = [], [], [], []
-        for it in range(num_iter):
-            scores = self.create_rollouts(num_episodes)[6]
-            scores = scores.tolist()
-            scores_episode += scores
-            for epoch in range(n_epoch):
-                ploss, vloss = self.update_epoch()
-                policy_loss_list.append(ploss[-1])         # the reference keeps the last agent's losses (:425-426)
-                value_loss_list.append(vloss[-1])
-                if self._maybe_test(it, epoch, test_freq, scores, score_test_list):
-                    return scores_episode, score_test_list, policy_loss_list, value_loss_list
-        return scores_episode, score_test_list, policy_loss_list, value_loss_list
+    def _epoch_losses(self):
+        ploss, vloss = self.update_epoch()
+        return ploss[-1], vloss[-1]                        # the reference keeps the last agent's losses (:425-426)
+
+    def train(self, num_iter, n_epoch=4, num_episodes=None, test_freq=100, *, checkpoint_path=None, checkpoint_freq=0,
+              resume=False):
+        """Returns (scores_episode, score_test_list, policy_loss_list, value_loss_list).  checkpoint_freq = k > 0
+        writes the training state into checkpoint_path after iterations 0, k, 2k, ...; resume=True continues the
+        run stored there (``PPOBase._train``)."""
+        return self._train(num_iter, n_epoch, num_episodes, test_freq, checkpoint_path, checkpoint_freq, resume)

@@ -20,7 +20,7 @@ import numpy as np
 import torch
 
 from .. import _lib as L
-from . import _dist
+from . import _ckpt, _dist
 from ._nets import NetSet, q_select, q_td_target
 
 _LOSSES = {"huber": L.QLOSS_HUBER, "mse": L.QLOSS_MSE}
@@ -63,6 +63,39 @@ class ReplayBuffer:
         self.rew[s].copy_(rewards)
         self.head = (s + 1) % self.n_slots
         self.n_stored = min(self.n_stored + 1, self.n_slots)
+
+    def _filled(self):
+        """The filled slots in ring order (oldest first) as at most two contiguous slot ranges."""
+        first = self.oldest_slot
+        if first + self.n_stored <= self.n_slots:
+            return [slice(first, first + self.n_stored)]
+        return [slice(first, self.n_slots), slice(0, self.head)]
+
+    def state_dict(self):
+        """The ``n_stored`` filled episodes in ring order (CPU tensors), ``head`` and the sampling generator's state."""
+        parts = self._filled()
+        return {"n_slots": self.n_slots, "n_stored": self.n_stored, "head": self.head,
+                "rng": _ckpt.plain(self._rng.bit_generator.state),
+                **{k: torch.cat([getattr(self, k)[s].cpu() for s in parts]) for k in ("obs", "act", "rew")}}
+
+    def load_state_dict(self, d):
+        if int(d["n_slots"]) != self.n_slots:
+            raise ValueError(f"replay buffer: n_slots is {d['n_slots']} in the stored state but {self.n_slots} here")
+        if not (0 <= int(d["n_stored"]) <= self.n_slots and 0 <= int(d["head"]) < self.n_slots):
+            raise ValueError(f"replay buffer: n_stored {d['n_stored']} / head {d['head']} out of range")
+        for k in ("obs", "act", "rew"):
+            own, t = getattr(self, k), d[k]
+            if tuple(t.shape[1:]) != tuple(own.shape[1:]) or t.shape[0] != int(d["n_stored"]) or t.dtype != own.dtype:
+                raise ValueError(f"replay buffer: {k} is {t.dtype} {tuple(t.shape)} in the stored state, expected "
+                                 f"{own.dtype} [{int(d['n_stored'])}, {', '.join(map(str, own.shape[1:]))}]")
+        self.n_stored, self.head = int(d["n_stored"]), int(d["head"])
+        done = 0
+        for s in self._filled():
+            n = s.stop - s.start
+            for k in ("obs", "act", "rew"):
+                getattr(self, k)[s].copy_(d[k][done:done + n])
+            done += n
+        self._rng.bit_generator.state = d["rng"]
 
     def sample_chunk(self, batch_size, chunk_size, start_idx=None, env_col=None):
         """``batch_size`` chunks of ``chunk_size`` consecutive transitions (irdqn.py:24-42), gathered on the device.
@@ -149,6 +182,8 @@ class iRDQN:
         self._loss_sum = torch.zeros(N, dtype=torch.float64, device=dev)
         self._episode = 0
         self.losses = []                                     # per train step: [N] losses (the reference drops them)
+        self._progress = self._fresh_progress()
+        self._float_lists = _ckpt.FloatLists()
 
     # ------------------------------------------------------------------ DQN.update_epsilon (irdqn.py:159-161)
     def update_epsilon(self, timestep, horizon_eps=1000):
@@ -219,12 +254,23 @@ class iRDQN:
         return self._loss_sum / rows
 
     # ------------------------------------------------------------------ iRDQN.train (irdqn.py:222-302)
-    def train(self, n_episodes, early_stopping=True, forced_actions=None, forced_samples=None):
+    def train(self, n_episodes, early_stopping=True, forced_actions=None, forced_samples=None, *, checkpoint_path=None,
+              checkpoint_freq=0, resume=False):
         """``n_episodes`` iterations of B lockstep episodes.  forced_actions(ep) -> u8 [T, N, B] and
         forced_samples(ep) -> (start_idx, env_col) are teacher-forcing hooks of the parity tests.
-        Returns (train_scores, test_list, reward_list) like the reference."""
-        test_list, reward_list, train_scores = [], [], []
-        for ep in range(n_episodes):
+        Returns (train_scores, test_list, reward_list) like the reference.  checkpoint_freq = k > 0 writes the training
+        state into checkpoint_path after episodes 0, k, 2k, ... (their optimiser step and target sync done), after the
+        last one and when early stopping fires; resume=True continues the run stored there, if there is one."""
+        if (checkpoint_freq or resume) and checkpoint_path is None:
+            raise ValueError("checkpoint_freq and resume need a checkpoint_path")
+        if resume and _ckpt.exists(checkpoint_path):
+            self.load_training_state(checkpoint_path)
+        else:
+            self._progress = self._fresh_progress()
+        p = self._progress
+        test_list, reward_list, train_scores = p["test_list"], p["reward_list"], p["train_scores"]
+        ep = p["next_episode"]
+        while ep < n_episodes and not p["stopped"]:
             ready = ep >= self.replay_start_size
             self._run_episode(L.ACT_SAMPLE, ready, None if forced_actions is None else forced_actions(ep), episode=ep)
             self._guard_exact_inputs()
@@ -239,14 +285,55 @@ class iRDQN:
                 if early_stopping and ts == 1:
                     if _dist.rank() == 0:
                         print(f"Early stopping at episode {ep}")
-                    break
-            if ready and ep % self.update_frequency == 0:
+                    p["stopped"] = True
+            if not p["stopped"] and ready and ep % self.update_frequency == 0:
                 s = (None, None) if forced_samples is None else forced_samples(ep)
                 tr_ = self.replay_buffer.sample_chunk(self.minibatch_size, self.history_len, s[0], s[1])
                 self.losses.append(self.train_step(tr_))
                 if ep % self.update_target_frequency == 0:
                     self.sync_target()
+            p["next_episode"] = ep + 1
+            if checkpoint_freq and (ep % checkpoint_freq == 0 or ep + 1 == n_episodes or p["stopped"]):
+                self.save_training_state(checkpoint_path)
+            ep += 1
         return train_scores, test_list, reward_list
+
+    # ------------------------------------------------------------------ training state (resume an interrupted run)
+    @staticmethod
+    def _fresh_progress():
+        return {"next_episode": 0, "stopped": False, "train_scores": [], "test_list": [], "reward_list": []}
+
+    def save_training_state(self, path):
+        """Write everything that decides how ``train`` continues into the directory ``path``: the network with its Adam
+        state, the target parameters, epsilon, the episode counters, the loop position, ``losses`` and the lists
+        ``train`` returns (rank 0), and every rank's replay shard with its sampling generator.  Call it between
+        episodes; the next episode resets the envs.  Collective when a process group is active."""
+        p, f = self._progress, self._float_lists
+        losses = torch.stack(self.losses).cpu() if self.losses else torch.zeros((0, self.n_agents), dtype=torch.float64)
+        replicated = {"network": self.network.training_state(), "target_params": self.target_params.cpu(),
+                      "epsilon": float(self.epsilon), "episode": self._episode, "env_episode": self.env.episode,
+                      "next_episode": p["next_episode"], "stopped": p["stopped"], "losses": losses,
+                      **{k: f.to_tensor(k, p[k]) for k in ("test_list", "reward_list")}}
+        local = {"replay": self.replay_buffer.state_dict(),
+                 "train_scores": f.to_tensor("train_scores", p["train_scores"])}
+        _ckpt.save(path, _ckpt.config(self), replicated, local, self.device)
+
+    def load_training_state(self, path):
+        """Restore the state ``save_training_state`` wrote; ValueError if the stored run was set up differently."""
+        rep, loc = _ckpt.load(path, _ckpt.config(self))
+        self.network.load_training_state(rep["network"])
+        if tuple(rep["target_params"].shape) != tuple(self.target_params.shape):
+            raise ValueError(f"target_params: expected {tuple(self.target_params.shape)}, got "
+                             f"{tuple(rep['target_params'].shape)}")
+        self.target_params.copy_(rep["target_params"])
+        self.replay_buffer.load_state_dict(loc["replay"])
+        self.epsilon, self._episode = float(rep["epsilon"]), int(rep["episode"])
+        self.env.set_episode(int(rep["env_episode"]) + 1)
+        self.losses = list(rep["losses"].to(self.device).unbind(0))
+        f = self._float_lists
+        self._progress = {"next_episode": int(rep["next_episode"]), "stopped": bool(rep["stopped"]),
+                          "train_scores": f.to_list("train_scores", loc["train_scores"]),
+                          **{k: f.to_list(k, rep[k]) for k in ("test_list", "reward_list")}}
 
     # ------------------------------------------------------------------ iRDQN.test (irdqn.py:305-353)
     def test(self, n_episodes, verbose=False, forced_actions=None):

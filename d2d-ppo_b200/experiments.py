@@ -39,6 +39,14 @@ def _learner(kind, env, save_path, seed, **kw):
     return cls(env, save_path=save_path, seed=seed, **kw)
 
 
+def _ckpt_kw(resume, folder, freq):
+    """train() arguments of a resumable run: the training state goes to the run's model folder after every
+    ``freq``-th iteration, i.e. right after each test iteration when freq = test_freq (and after the last one), and a
+    rerun continues from it; a run that had finished returns its stored lists at once, so only the evaluation after it
+    repeats."""
+    return dict(checkpoint_path=folder, checkpoint_freq=freq, resume=True) if resume else {}
+
+
 def _result(scores, jains, errors, rewards, training, **extra):
     out = {"scores": scores, "jains": jains, "channel_errors": errors, "average_rewards": rewards,
            "training": training}
@@ -48,8 +56,9 @@ def _result(scores, jains, errors, rewards, training, **extra):
 
 def xp_load(out_dir="combinatorial_load", learner="d2dppo", n_seeds=1, loads=None, num_iter=2000, n_epoch=5,
             n_envs=10, test_freq=100, test_episodes=1000, setup="setup_8_channels", device=None,
-            result_name="results/mcappo_8_channels.p"):
-    """xp_load.py: for every load, train on the heterogeneous 8-channel env, reload the best model, test."""
+            result_name="results/mcappo_8_channels.p", resume=False):
+    """xp_load.py: for every load, train on the heterogeneous 8-channel env, reload the best model, test.
+    resume=True: every training run checkpoints into its model folder (``_ckpt_kw``) and continues from there."""
     from .envs import CombinatorialEnv
     s = presets.SETUPS[setup]
     loads = s["loads_list"] if loads is None else loads
@@ -70,14 +79,15 @@ def xp_load(out_dir="combinatorial_load", learner="d2dppo", n_seeds=1, loads=Non
                              gamma=0.4, update_target_frequency=100, minibatch_size=64, learning_rate=1e-4,
                              update_frequency=1, initial_exploration_rate=1, final_exploration_rate=0.1,
                              adam_epsilon=1e-8, loss="huber", seed=seed)
-                res = idqn.train(num_iter)
+                res = idqn.train(num_iter, **_ckpt_kw(resume, folder, test_freq))
                 score, jain = idqn.test(test_episodes)
                 for lst, v in zip(row, (score, jain, "", "", res)):
                     lst.append(v)
                 continue
             ppo = _learner(learner, env, folder, seed, hidden_size=64, gamma=gamma, policy_lr=3e-4, value_lr=1e-3,
                            useRNN=True, combinatorial=True, history_len=s["n_agents"], early_stopping=True)
-            res = ppo.train(num_iter=num_iter, n_epoch=n_epoch, num_episodes=n_envs, test_freq=test_freq)
+            res = ppo.train(num_iter=num_iter, n_epoch=n_epoch, num_episodes=n_envs, test_freq=test_freq,
+                            **_ckpt_kw(resume, folder, test_freq))
             if os.path.exists(os.path.join(folder, "agent_0.pth")):
                 ppo.load(folder)
             out = ppo.test(test_episodes)
@@ -93,9 +103,10 @@ def xp_load(out_dir="combinatorial_load", learner="d2dppo", n_seeds=1, loads=Non
 
 def xp_n_agents(out_dir="xp_3gpp_homogeneous", learner="random_access", n_seeds=1, n_agents_list=(4, 8, 12, 16),
                 load=1 / 14, n_envs=500, cv_episodes=50, test_episodes=500, num_iter=2000, n_epoch=5, test_freq=100,
-                device=None, result_name="results/aloha.p"):
+                device=None, result_name="results/aloha.p", resume=False):
     """xp_n_agents.py: N-agent sweep on 4 channels; the active block of the script is the random-access baseline
-    with its transmission probability picked by ``get_best_transmission_probs`` (:137-140)."""
+    with its transmission probability picked by ``get_best_transmission_probs`` (:137-140).  resume=True: the learner
+    runs checkpoint into their model folders and continue from there (the baseline has no training state)."""
     from .algorithms.baselines import CombinatorialRandomAccess
     from .envs import CombinatorialEnv
     _mk(os.path.join(out_dir, "results"))
@@ -115,7 +126,8 @@ def xp_n_agents(out_dir="xp_3gpp_homogeneous", learner="random_access", n_seeds=
                 ppo = _learner(learner, env, folder, seed, hidden_size=64, gamma=0.6 if learner == "d2dppo" else 0.4,
                                policy_lr=3e-4, value_lr=1e-3, useRNN=True, combinatorial=True,
                                history_len=min(n_agents, 10), early_stopping=True)
-                res = ppo.train(num_iter=num_iter, n_epoch=n_epoch, num_episodes=n_envs, test_freq=test_freq)
+                res = ppo.train(num_iter=num_iter, n_epoch=n_epoch, num_episodes=n_envs, test_freq=test_freq,
+                                **_ckpt_kw(resume, folder, test_freq))
                 out = ppo.test(test_episodes)
             for lst, v in zip(row, (*out, res)):
                 lst.append(v)
@@ -185,8 +197,9 @@ def xp_gamma(out_dir=".", gammas=(0.2, 0.4, 0.6, 0.8, 0.99), n_agents=5, n_chann
 
 
 def run_ippo_combinatorial(out_dir="combinatorial_load", load=1 / 3, num_iter=2000, n_epoch=5, n_envs=10, test_freq=100,
-                           test_episodes=500, device=None, result_name="results/ippo_16_channels.p"):
-    """run_ippo_combinatorial.py:65-94: iPPO (gamma .99, value_lr 1e-2, history 6) on the 16-channel env."""
+                           test_episodes=500, device=None, result_name="results/ippo_16_channels.p", resume=False):
+    """run_ippo_combinatorial.py:65-94: iPPO (gamma .99, value_lr 1e-2, history 6) on the 16-channel env.
+    resume=True: the run checkpoints into its model folder and continues from there."""
     from .envs import CombinatorialEnv
     _mk(os.path.join(out_dir, "results"))
     env = CombinatorialEnv(n_envs=n_envs, device=device, seed=42,
@@ -194,7 +207,8 @@ def run_ippo_combinatorial(out_dir="combinatorial_load", load=1 / 3, num_iter=20
     folder = _mk(os.path.join(out_dir, "models_ippo_16"))
     ippo = _learner("ippo", env, folder, 0, hidden_size=64, gamma=0.99, policy_lr=3e-4, value_lr=1e-2, useRNN=True,
                     combinatorial=True, history_len=6, early_stopping=True)
-    res = ippo.train(num_iter=num_iter, n_epoch=n_epoch, num_episodes=n_envs, test_freq=test_freq)
+    res = ippo.train(num_iter=num_iter, n_epoch=n_epoch, num_episodes=n_envs, test_freq=test_freq,
+                     **_ckpt_kw(resume, folder, test_freq))
     if os.path.exists(os.path.join(folder, "agent_0.pth")):
         ippo.load(folder)                                             # run_ippo_combinatorial.py:93 reloads the best model
     out = ippo.test(test_episodes)
@@ -253,11 +267,15 @@ def main(argv=None):
     ap.add_argument("--num-iter", type=int, default=None)
     ap.add_argument("--n-envs", type=int, default=None)
     ap.add_argument("--test-episodes", type=int, default=None)
+    ap.add_argument("--resume", action="store_true", default=None,
+                    help="checkpoint every training run into its model folder and continue from there")
     a = ap.parse_args(argv)
     kw = {k: v for k, v in (("out_dir", a.out), ("learner", a.learner), ("num_iter", a.num_iter), ("n_envs", a.n_envs),
-                            ("test_episodes", a.test_episodes)) if v is not None}
+                            ("test_episodes", a.test_episodes), ("resume", a.resume)) if v is not None}
     fn = globals()[a.experiment]
     import inspect
+    if a.resume and "resume" not in inspect.signature(fn).parameters:
+        ap.error(f"--resume: {a.experiment} keeps no training state to resume")
     kw = {k: v for k, v in kw.items() if k in inspect.signature(fn).parameters}
     res = fn(**kw)
     print({k: (v if k != "training" else "...") for k, v in res.items()})
