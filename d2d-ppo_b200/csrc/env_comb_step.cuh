@@ -208,23 +208,28 @@ int launch_comb_mode(const StepArgs& a, int grid, int block, cudaStream_t s, boo
 }
 
 // n_inner consecutive fused random-access steps of ONE episode in one launch, one thread per env (the run form of
-// comb_step_kernel<W, uint8_t, CFIX, true, 2>, as sc_run_kernel is of sc_step_kernel).  The env's N <= NK records,
+// comb_step_kernel<W, uint8_t, C, true, 2>, as sc_run_kernel is of sc_step_kernel).  The env's N <= 8 records,
 // channel masks and disc / recv counters are loaded once, live in registers for every step and are stored once, so a
 // step moves no state through HBM: what it writes is the observation rows and the reward.  With the observations of
 // every step written to the same block (obs_stride 0, CombinatorialRandomAccess.run / bench.py) those rows of the
 // resident envs can stay in L2 (2 blocks of 256 per SM: 75,776 envs x 720 B = 55 MB of the 126 MB; one block per SM
 // measured slower, DESIGN.md section 3).  Same Philox counters and update order as comb_step_kernel: bit-identical.
-template <int W, int CFIX, int NK>
-__global__ void __launch_bounds__(256, 2) comb_run_kernel(const StepArgs a, const RunArgs ra) {
-  extern __shared__ __align__(16) uint8_t smem[];
-  const EnvParamsHdr* P = stage_params(a, smem);
-  const uint32_t* cdf = reinterpret_cast<const uint32_t*>(smem + P->off_cdf);
-  const uint32_t* swthr = reinterpret_cast<const uint32_t*>(smem + P->off_sw);
-  const int N = P->N;
-  constexpr int C = CFIX;
+// A step is bound by the instructions each warp issues, so the step body is straight-line code:
+//  - NF: the device count as a constant (no per-device guards or dead slots); 0 = any N <= 8 at run time;
+//  - DH: every device's observation carries DH slots (homogeneous sizes, D = DH), which fixes the rows of each device
+//    at compile time; 0 = the slot count and rows come from the tables at run time;
+//  - the env tables are kernel parameters (CombRunParams: constant-bank operands, no staging, no LDS);
+//  - each Philox call starts at round 2 from the thread's and the call's two-round heads (philox_rk_heads);
+//  - the ack / nack floats are formed once per step and stored for every device;
+//  - observation rows are plain stores, which ptxas may schedule among the Philox rounds (emit_slots_run).
+template <int W, int C, int NF, int DH>
+__global__ void __launch_bounds__(256, 2) comb_run_kernel(const StepArgs a, const RunArgs ra,
+                                                          const __grid_constant__ CombRunParams p) {
+  constexpr int NK = NF ? NF : kRunMaxN;
   constexpr uint32_t cmask = (1u << C) - 1u;
+  const int N = NF ? NF : p.N;
   const size_t B = (size_t)a.B;
-  const uint32_t Bu = (uint32_t)a.B;
+  const int Bi = a.B;
   uint8_t* chan = reinterpret_cast<uint8_t*>(a.chan);
   const int b = blockIdx.x * blockDim.x + threadIdx.x;
   if (b >= a.B) return;
@@ -233,12 +238,12 @@ __global__ void __launch_bounds__(256, 2) comb_run_kernel(const StepArgs a, cons
   uint32_t chv[NK], discv[NK], recvv[NK];
 #pragma unroll
   for (int k = 0; k < NK; ++k) {
-    const size_t idx = (size_t)min(k, N - 1) * B + b;
+    const size_t idx = (size_t)(NF ? k : min(k, N - 1)) * B + b;
     rec[k] = rec_load<W>(a.buf, idx);
     chv[k] = chan[idx], discv[k] = a.disc[idx], recvv[k] = a.recv[idx];
   }
   int32_t rew = a.reward_accum ? a.reward[b] : 0;
-  const uint32_t thr = a.tp_thr;
+  const PhiloxEnvHead eh = philox_env_head(a, env, 0u);   // C <= 8 and arrivals: block 0 only
 #pragma unroll 1
   for (int i = 0; i < ra.n_inner; ++i) {
     const uint32_t t = a.t + (uint32_t)i;
@@ -248,9 +253,9 @@ __global__ void __launch_bounds__(256, 2) comb_run_kernel(const StepArgs a, cons
     uint64_t att_pack = 0;
 #pragma unroll
     for (int k = 0; k < NK; ++k) {
-      if (k < N) {
-        const uint32_t want =
-            lane_mask_rk<CFIX>(a, env, t, (uint32_t)k | (kPurposePolicy << 16), C, [thr](int) { return thr; });
+      if (NF || k < N) {
+        const uint4 r = philox_rk_heads(a, eh, philox_call_head(a, t, (uint32_t)k | (kPurposePolicy << 16)));
+        const uint32_t want = lanes_below<C>(r, [&p](int) { return p.tp_lt; }, p.tp_all);
         const uint32_t at = rec_any<W>(rec[k]) ? (want & cmask) : 0u;
         twice |= once & at;
         once |= at;
@@ -260,13 +265,18 @@ __global__ void __launch_bounds__(256, 2) comb_run_kernel(const StepArgs a, cons
     }
     const uint32_t acked = once & ~twice & good_any;          // :155-157
     const uint32_t nacked = once & ~acked;
+    float* obs_i = a.obs ? a.obs + (size_t)i * (size_t)ra.obs_stride + b : nullptr;
+    float ackf[C];
+    if (obs_i) {
+#pragma unroll
+      for (int c = 0; c < C; ++c) ackf[c] = ((acked >> c) & 1u) ? 1.0f : (((nacked >> c) & 1u) ? -1.0f : 0.0f);
+    }
     // ---- serve, age, switch, arrive, observe (:160-206) ----
     int n_success = 0;
     uint4 arr4 = make_uint4(0u, 0u, 0u, 0u);
-    float* obs_i = a.obs ? a.obs + (size_t)i * (size_t)ra.obs_stride : nullptr;
 #pragma unroll
     for (int k = 0; k < NK; ++k) {
-      if (k < N) {
+      if (NF || k < N) {
         Rec<W>& r = rec[k];
         const uint32_t at = (uint32_t)(att_pack >> (k * 8)) & 0xFFu;
         const uint32_t ch = chv[k];
@@ -274,24 +284,35 @@ __global__ void __launch_bounds__(256, 2) comb_run_kernel(const StepArgs a, cons
         n_success += success;
         rec_pop_earliest<W>(r, success);
         discv[k] += rec_age<W>(r);
-        const uint32_t* sthr = swthr + k * C;
-        const uint32_t sw =
-            lane_mask_rk<CFIX>(a, env, t, (uint32_t)k | (kPurposeSwitch << 16), C, [sthr](int c) { return sthr[c]; });
+        const uint4 rs = philox_rk_heads(a, eh, philox_call_head(a, t, (uint32_t)k | (kPurposeSwitch << 16)));
+        const uint32_t sw = lanes_below<C>(rs, [&p, k](int c) { return p.sw_lt[k][c]; }, p.sw_all[k]);
         chv[k] = (ch ^ sw) & cmask;
-        const int dl = P->deadline[k];
+        const int dl = p.deadline[k];
         // one Philox call per four devices (env_common.cuh: ArrivalWords), drawn when any device of the group is active
         if ((k & 3) == 0 && ((active >> k) & 0xFull))
-          arr4 = philox_rk(a, env, t, (uint32_t)(k >> 2) | (kPurposeArrival << 16), 0u);
+          arr4 = philox_rk_heads(a, eh, philox_call_head(a, t, (uint32_t)(k >> 2) | (kPurposeArrival << 16)));
         if ((active >> k) & 1ull) {
-          const uint32_t arrived = arrival_from_u(P, cdf, k, pick_word(arr4, k & 3));
+          const uint32_t u = pick_word(arr4, k & 3);
+          uint32_t arrived = 0;
+          if (p.arrival_kind[k] == D2D_ARRIVAL_BERNOULLI) {
+            arrived = (uint64_t)u < p.bern_thr[k] ? 1u : 0u;
+          } else {
+#pragma unroll 1
+            for (int m = 0; m < D2D_POISSON_KMAX; ++m) {
+              if (u < p.cdf[k][m]) break;   // thresholds are non-decreasing (arrival_from_u)
+              ++arrived;
+            }
+          }
           rec_set_byte<W>(r, dl - 1, arrived);
           recvv[k] += arrived;
         }
         if (obs_i) {
-          float* o = obs_i + (size_t)P->obs_off[k] * B + b;
-          o = emit_slots<W>(r, P->homog ? P->D : dl, o, Bu);
-          o = emit_bits<CFIX>(ch, C, o, Bu);                  // pre-switch copy (:145)
-          emit_ack<CFIX>(acked, nacked, C, o, Bu);
+          float* o = obs_i + (size_t)(DH ? k * (DH + 2 * C) : (int)p.obs_off[k]) * B;
+          o = emit_slots_run<W, DH>(r, DH ? DH : (p.homog_slots ? p.homog_slots : dl), o, Bi);
+#pragma unroll
+          for (int c = 0; c < C; ++c, o += Bi) *o = ((ch >> c) & 1u) ? 1.0f : 0.0f;   // pre-switch copy (:145)
+#pragma unroll
+          for (int c = 0; c < C; ++c, o += Bi) *o = ackf[c];
         }
       }
     }
@@ -300,7 +321,7 @@ __global__ void __launch_bounds__(256, 2) comb_run_kernel(const StepArgs a, cons
   }
 #pragma unroll
   for (int k = 0; k < NK; ++k) {
-    if (k < N) {
+    if (NF || k < N) {
       const size_t idx = (size_t)k * B + b;
       rec_store<W>(a.buf, idx, rec[k]);
       chan[idx] = (uint8_t)chv[k];
@@ -311,12 +332,23 @@ __global__ void __launch_bounds__(256, 2) comb_run_kernel(const StepArgs a, cons
   if (a.done) a.done[b] = (uint8_t)a.done_flag;
 }
 
-// d2d_env_run_random_access's episode-in-one-launch path for the combinatorial env; C must be 4 or 8, N <= 8
+// d2d_env_run_random_access's episode-in-one-launch path for the combinatorial env; C must be 4 or 8, N <= 8.
+// Exact-N kernels for N = 4, 6, 8 with homogeneous observations of the record's usual deadline (7 for 8-byte records,
+// 14 for 16-byte ones: setup_8_channels and c1-c5); every other shape runs the general kernel.
 template <int W>
-int launch_comb_run(const StepArgs& a, const RunArgs& ra, int C, cudaStream_t s) {
+int launch_comb_run(const StepArgs& a, const RunArgs& ra, const CombRunParams& p, int C, cudaStream_t s) {
   const int block = 256, grid = (a.B + block - 1) / block;
-  if (C == 8) comb_run_kernel<W, 8, 8><<<grid, block, a.params_bytes, s>>>(a, ra);
-  else comb_run_kernel<W, 4, 8><<<grid, block, a.params_bytes, s>>>(a, ra);
+  constexpr int DH = W == 4 ? 14 : 7;
+  const int nf = p.homog_slots == DH && (p.N == 4 || p.N == 6 || p.N == 8) ? p.N : 0;
+#define D2D_RUN(CC)                                                                              \
+  switch (nf) {                                                                                  \
+    case 4: comb_run_kernel<W, CC, 4, DH><<<grid, block, 0, s>>>(a, ra, p); break;               \
+    case 6: comb_run_kernel<W, CC, 6, DH><<<grid, block, 0, s>>>(a, ra, p); break;               \
+    case 8: comb_run_kernel<W, CC, 8, DH><<<grid, block, 0, s>>>(a, ra, p); break;               \
+    default: comb_run_kernel<W, CC, 0, 0><<<grid, block, 0, s>>>(a, ra, p); break;               \
+  }
+  if (C == 8) D2D_RUN(8) else D2D_RUN(4)
+#undef D2D_RUN
   D2D_LAUNCHED();
   return D2D_OK;
 }

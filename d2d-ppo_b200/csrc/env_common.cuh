@@ -239,6 +239,86 @@ __device__ __forceinline__ uint4 philox_rk(const StepArgs& a, uint32_t c0, uint3
   return make_uint4(c0, c1, c2, c3);
 }
 
+// philox_rk split after its first two rounds, for callers that draw many counters (env, t, dp, blk) with the same env
+// and blk.  With M0 = 0xD2511F53, M1 = 0xCD9E8D57 and hi / lo the halves of the 64-bit product, round 0 gives
+//   c0 = hi(M1 dp) ^ t ^ rk0[0] =: A      c1 = lo(M1 dp)      c2 = hi(M0 env) ^ blk ^ rk1[0] =: X      c3 = lo(M0 env)
+// and round 1 multiplies A and X:
+//   c0 = hi(M1 X) ^ rk0[1] ^ lo(M1 dp)    c1 = lo(M1 X)       c2 = lo(M0 env) ^ rk1[1] ^ hi(M0 A)      c3 = lo(M0 A).
+// So after two rounds the state is three words of (env, blk) (PhiloxEnvHead, once per thread) XOR three words of
+// (t, dp) (PhiloxCallHead, warp-uniform; lo(M1 dp) is a constant for a compile-time dp), and a call continues at round 2.
+struct PhiloxEnvHead {
+  uint32_t e0, e1, e2;
+};
+struct PhiloxCallHead {
+  uint32_t u0, u2, u3;
+};
+
+__device__ __forceinline__ PhiloxEnvHead philox_env_head(const StepArgs& a, uint32_t env, uint32_t blk) {
+  const uint64_t p0 = (uint64_t)0xD2511F53u * env;
+  const uint32_t x = (uint32_t)(p0 >> 32) ^ blk ^ a.rk1[0];
+  const uint64_t p1 = (uint64_t)0xCD9E8D57u * x;
+  return {(uint32_t)(p1 >> 32) ^ a.rk0[1], (uint32_t)p1, (uint32_t)p0 ^ a.rk1[1]};
+}
+
+__device__ __forceinline__ PhiloxCallHead philox_call_head(const StepArgs& a, uint32_t t, uint32_t dev_purpose) {
+  const uint64_t p1 = (uint64_t)0xCD9E8D57u * dev_purpose;
+  const uint32_t c0 = (uint32_t)(p1 >> 32) ^ t ^ a.rk0[0];
+  const uint64_t p0 = (uint64_t)0xD2511F53u * c0;
+  return {(uint32_t)p1, (uint32_t)(p0 >> 32), (uint32_t)p0};
+}
+
+// philox_rk(a, env, t, dp, blk) == philox_rk_heads(a, philox_env_head(a, env, blk), philox_call_head(a, t, dp))
+__device__ __forceinline__ uint4 philox_rk_heads(const StepArgs& a, const PhiloxEnvHead& e, const PhiloxCallHead& u) {
+  uint32_t c0 = e.e0 ^ u.u0, c1 = e.e1, c2 = e.e2 ^ u.u2, c3 = u.u3;
+#pragma unroll
+  for (int r = 2; r < 10; ++r) {
+    const uint64_t p0 = (uint64_t)0xD2511F53u * c0;
+    const uint64_t p1 = (uint64_t)0xCD9E8D57u * c2;
+    const uint32_t n0 = (uint32_t)(p1 >> 32) ^ c1 ^ a.rk0[r];
+    const uint32_t n2 = (uint32_t)(p0 >> 32) ^ c3 ^ a.rk1[r];
+    c1 = (uint32_t)p1;
+    c3 = (uint32_t)p0;
+    c0 = n0;
+    c2 = n2;
+  }
+  return make_uint4(c0, c1, c2, c3);
+}
+
+// bit c of the C 16-bit lanes of r: lane c < thr(c), with the threshold given as lt(c) = thr(c) << 16 (0 for thr =
+// 65536) and all = the lanes whose thr is 65536.  Lane 2j + 1 is the high half of word j, so it is below thr exactly
+// when the word is below thr << 16; lane 2j is compared the same way after a shift.  One compare per lane.
+template <int C, typename LtFn>
+__device__ __forceinline__ uint32_t lanes_below(const uint4& r, LtFn lt, uint32_t all) {
+  const uint32_t w[4] = {r.x, r.y, r.z, r.w};
+  uint32_t m = all;
+#pragma unroll
+  for (int c = 0; c < C; ++c) {
+    const uint32_t v = (c & 1) ? w[c >> 1] : (w[c >> 1] << 16);
+    m |= (uint32_t)(v < lt(c)) << c;
+  }
+  return m;
+}
+
+// the per-device tables comb_run_kernel reads, passed by value: kernel parameters sit in the constant bank, so every
+// read is an instruction operand instead of a shared-memory load.  Built once per env (d2d_env_create) for N <= 8,
+// C <= 8; the policy threshold is set per call.
+constexpr int kRunMaxN = 8, kRunMaxC = 8;
+struct CombRunParams {
+  uint32_t sw_lt[kRunMaxN][kRunMaxC];   // switch threshold of (device, channel) for lanes_below
+  uint32_t sw_all[kRunMaxN];
+  uint32_t cdf[kRunMaxN][D2D_POISSON_KMAX];
+  uint64_t bern_thr[kRunMaxN];
+  uint32_t tp_lt, tp_all;               // the policy threshold for lanes_below (same for every lane)
+  int32_t N;
+  int32_t homog_slots;                  // slots per device in the observation: D if homogeneous, else 0 (own deadline)
+  uint16_t obs_off[kRunMaxN];
+  uint8_t deadline[kRunMaxN];
+  uint8_t arrival_kind[kRunMaxN];
+};
+
+// lanes_below's form of a 16-bit-lane threshold thr in [0, 65536]
+__host__ __device__ inline uint32_t lane_lt(uint32_t thr) { return thr >= 65536u ? 0u : thr << 16; }
+
 // bit c = (16-bit lane c < thr(c)) for c < C at Philox timestep t;  CFIX > 0 makes the lane count a compile-time constant
 template <int CFIX, typename ThrFn>
 __device__ __forceinline__ uint32_t lane_mask_rk(const StepArgs& a, uint32_t env, uint32_t t, uint32_t dev_purpose,
@@ -306,6 +386,33 @@ __device__ __forceinline__ float* emit_slots(const Rec<W>& r, int n, float* p, u
     }
   }
   return p;
+}
+
+// emit_slots for comb_run_kernel, with plain stores along an int-stride pointer chain that ptxas schedules freely (the
+// volatile st_f32 form measured slower there, DESIGN.md section 3).  DH > 0: the slot count is the constant DH (n unused).
+template <int W, int DH>
+__device__ __forceinline__ float* emit_slots_run(const Rec<W>& r, int n, float* p, int B) {
+  if constexpr (DH > 0) {
+#pragma unroll
+    for (int d = 0; d < DH; ++d, p += B) {
+      const uint32_t w = r.w[d >> 2];
+      *p = (d & 3) == 0 ? byte_f32<0>(w) : (d & 3) == 1 ? byte_f32<1>(w) : (d & 3) == 2 ? byte_f32<2>(w) : byte_f32<3>(w);
+    }
+    return p;
+  } else {
+    if (n == 7) return emit_slots_run<W, 7>(r, n, p, B);
+    if constexpr (W >= 4)
+      if (n == 14) return emit_slots_run<W, 14>(r, n, p, B);
+#pragma unroll
+    for (int d = 0; d < 4 * W; ++d) {
+      if (d < n) {
+        const uint32_t w = r.w[d >> 2];
+        *p = (d & 3) == 0 ? byte_f32<0>(w) : (d & 3) == 1 ? byte_f32<1>(w) : (d & 3) == 2 ? byte_f32<2>(w) : byte_f32<3>(w);
+        p += B;
+      }
+    }
+    return p;
+  }
 }
 
 template <int CFIX>

@@ -31,7 +31,8 @@ namespace d2d {
 template <int W>
 int launch_comb_step(const StepArgs& a, int N, int C, int mask_bytes, cudaStream_t s);  // env_comb_w{2,4,8}.cu
 template <int W>
-int launch_comb_run(const StepArgs& a, const RunArgs& ra, int C, cudaStream_t s);         // env_comb_w{2,4}.cu
+int launch_comb_run(const StepArgs& a, const RunArgs& ra, const CombRunParams& p, int C,
+                    cudaStream_t s);                                                   // env_comb_w{2,4}.cu
 
 // ================================================================================================
 // CombinatorialEnv reset (the step kernel lives in env_comb_step.cuh)
@@ -728,6 +729,7 @@ struct d2d_env {
   const void* rp_sw = nullptr;
   int rp_len = 0;
   struct HostPipe* pipe = nullptr;   // lazily created by d2d_env_step_host
+  CombRunParams comb_run;            // comb_run_kernel's tables (combinatorial env, N <= 8, C <= 8)
   size_t chan_elems() const { return kind == D2D_ENV_CHANNEL_SELECTION ? (size_t)B : (size_t)N * B; }
 };
 
@@ -891,6 +893,21 @@ extern "C" int d2d_env_create(const d2d_env_config* cfg, d2d_env** out) {
   std::vector<uint8_t> blob(h.total_bytes, 0);
   memcpy(blob.data(), &h, sizeof(h));
   memcpy(blob.data() + h.off_cdf, cfg->poisson_cdf, (size_t)N * D2D_POISSON_KMAX * 4);
+  memset(&e->comb_run, 0, sizeof(e->comb_run));
+  if (e->kind == D2D_ENV_COMBINATORIAL && N <= kRunMaxN && C <= kRunMaxC) {
+    CombRunParams& q = e->comb_run;
+    q.N = N, q.homog_slots = e->homog ? e->D : 0;
+    for (int k = 0; k < N; ++k) {
+      for (int c = 0; c < C; ++c) {
+        const uint32_t thr = cfg->switch_thr[k * C + c];
+        q.sw_lt[k][c] = lane_lt(thr);
+        q.sw_all[k] |= (uint32_t)(thr >= 65536u) << c;
+      }
+      memcpy(q.cdf[k], cfg->poisson_cdf + (size_t)k * D2D_POISSON_KMAX, D2D_POISSON_KMAX * 4);
+      q.bern_thr[k] = h.bern_thr[k], q.obs_off[k] = h.obs_off[k];
+      q.deadline[k] = h.deadline[k], q.arrival_kind[k] = h.arrival_kind[k];
+    }
+  }
   memcpy(blob.data() + h.off_sw, cfg->switch_thr, (size_t)n_sw * 4);
   memcpy(blob.data() + h.off_nbr_off, nbr_off.data(), (size_t)(N + 1) * 4);
   if (!nbr_idx.empty()) memcpy(blob.data() + h.off_nbr_idx, nbr_idx.data(), nbr_idx.size());
@@ -1123,8 +1140,10 @@ extern "C" int d2d_env_run_random_access(d2d_env* e, double tp, int n_steps, int
       ra.obs_stride = obs_step_stride;
       if (comb_multi) {
         a.obs = obs_i;
-        rc = e->W == 2 ? launch_comb_run<2>(a, ra, e->C, as_stream(stream))
-                       : launch_comb_run<4>(a, ra, e->C, as_stream(stream));
+        CombRunParams p = e->comb_run;
+        p.tp_lt = lane_lt(tp_thr), p.tp_all = tp_thr >= 65536u ? (1u << e->C) - 1u : 0u;
+        rc = e->W == 2 ? launch_comb_run<2>(a, ra, p, e->C, as_stream(stream))
+                       : launch_comb_run<4>(a, ra, p, e->C, as_stream(stream));
         if (rc) return rc;
       } else if (e->B <= kRunLanesMaxEnvs) {
         // small batches: four lanes per env (sc_run_lanes_kernel), 64-thread blocks = 16 envs spread over the SMs
