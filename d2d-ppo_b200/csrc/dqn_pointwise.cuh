@@ -19,7 +19,8 @@ struct QSelectArgs {
   float epsilon;
   int ready;             // is_training_ready (irdqn.py:233): not ready -> every action is the random draw
   int n_random;          // the random draw is uniform on {0 .. n_random - 1} (np.random.randint(0, 2) -> 2)
-  uint32_t k0, k1, env_offset;
+  PhiloxKey key;
+  uint32_t env_offset;
   int t_abs;
 };
 
@@ -39,8 +40,8 @@ __global__ void q_select_kernel(const QSelectArgs a) {
         if (v > best) best = v, act = (uint32_t)o;      // torch.argmax: first maximum
       }
       if (a.act_mode == kActSample) {
-        const uint4 r = philox4x32_10(a.env_offset + (uint32_t)b, (uint32_t)a.t_abs,
-                                      (uint32_t)g | (kPurposePolicy << 16), 0u, a.k0, a.k1);
+        const uint4 r = philox(a.key, a.env_offset + (uint32_t)b, (uint32_t)a.t_abs,
+                               (uint32_t)g | (kPurposePolicy << 16), 0u);
         const double u = ((double)r.x + 0.5) * (1.0 / 4294967296.0);
         const bool greedy = a.ready && u >= (double)a.epsilon;            // irdqn.py:151
         if (!greedy) act = (uint32_t)(((unsigned long long)r.y * (unsigned long long)a.n_random) >> 32);

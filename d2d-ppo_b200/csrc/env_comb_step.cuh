@@ -21,7 +21,7 @@ __global__ void __launch_bounds__(256, 4) comb_step_kernel(const StepArgs a) {
   constexpr bool REPLAY = (MODE & 1) != 0, RA = (MODE & 2) != 0;
   const EnvParamsHdr* P = stage_params(a, smem);
   const uint32_t* cdf = reinterpret_cast<const uint32_t*>(smem + P->off_cdf);
-  const uint32_t* swthr = reinterpret_cast<const uint32_t*>(smem + P->off_sw);
+  const uint32_t* swlt = reinterpret_cast<const uint32_t*>(smem + P->off_sw);
   const int N = P->N;
   const int C = CFIX ? CFIX : P->C;
   const size_t B = (size_t)a.B;
@@ -66,14 +66,13 @@ __global__ void __launch_bounds__(256, 4) comb_step_kernel(const StepArgs a) {
       for (int j = 0; j < CH; ++j) {
         const int k = k0 + j;
         if (k < k_hi) {
-          uint32_t want = ww[j];
+          uint32_t want = ww[j] & cmask;
           if constexpr (RA) {
-            const uint32_t thr = a.tp_thr;
-            want = lane_mask_rk<CFIX>(a, env, a.t, (uint32_t)k | (kPurposePolicy << 16), C,
-                                      [thr](int) { return thr; });
+            want = lanes16_below<CFIX>(a.key, env, a.t, (uint32_t)k | (kPurposePolicy << 16), C,
+                                       [&a](int) { return a.tp_lt; }, a.tp_all) & cmask;
             if (act_out) act_out[(size_t)k * B + b] = (MaskT)want;
           }
-          const uint32_t at = rec_any<W>(rr[j]) ? (want & cmask) : 0u;
+          const uint32_t at = rec_any<W>(rr[j]) ? want : 0u;
           twice |= once & at;
           once |= at;
           good_any |= at & cc[j];
@@ -103,7 +102,6 @@ __global__ void __launch_bounds__(256, 4) comb_step_kernel(const StepArgs a) {
     // ---- pass 2: serve, age, switch, arrive, observe; device k+1's state is fetched while k is processed ----
     int n_success = 0;
     uint4 arr4 = make_uint4(0u, 0u, 0u, 0u);
-    int arr_group = -1;
     const int k_first = G > 1 ? min(k_lo, N - 1) : 0;
     const size_t first = (size_t)k_first * B + b;
     Rec<W> r_nx = rec_load<W>(a.buf, first);       // second touch of the record: L1 hit
@@ -134,24 +132,18 @@ __global__ void __launch_bounds__(256, 4) comb_step_kernel(const StepArgs a) {
       if constexpr (REPLAY) {
         sw = rp_sw[idx];
       } else {
-        const uint32_t* thr = swthr + k * C;
-        sw = lane_mask_rk<CFIX>(a, env, a.t, (uint32_t)k | (kPurposeSwitch << 16), C,
-                                [thr](int c) { return thr[c]; });
+        const uint32_t* lt = swlt + k * P->sw_row;
+        sw = lanes16_below<CFIX>(a.key, env, a.t, (uint32_t)k | (kPurposeSwitch << 16), C,
+                                 [lt](int c) { return lt[c]; }, P->sw_all[k]);
       }
       const uint32_t ch_new = (ch ^ sw) & cmask;
       chan[idx] = (MaskT)ch_new;
       const int dl = P->deadline[k];
+      if constexpr (!REPLAY) arrival_call(a, env, k, arr4);   // k_lo is a multiple of 4
       if ((a.active >> k) & 1ull) {                               // :178-196
-        uint32_t arrived;
-        if constexpr (REPLAY) {
-          arrived = a.rp_arr[idx];
-        } else {
-          if ((k >> 2) != arr_group) {          // one Philox call per four devices (env_common.cuh: ArrivalWords)
-            arr_group = k >> 2;
-            arr4 = philox_rk(a, env, a.t, (uint32_t)arr_group | (kPurposeArrival << 16), 0u);
-          }
-          arrived = arrival_from_u(P, cdf, k, pick_word(arr4, k & 3));
-        }
+        const uint32_t arrived = REPLAY ? a.rp_arr[idx]
+                                        : arrival_count(word32(arr4, k), P->arrival_kind[k] == D2D_ARRIVAL_BERNOULLI,
+                                                        P->bern_thr[k], cdf + k * D2D_POISSON_KMAX);
         rec_set_byte<W>(r, dl - 1, arrived);
         if (arrived) a.recv[idx] = recv_v + arrived;
       }
@@ -187,22 +179,27 @@ __global__ void __launch_bounds__(256, 4) comb_step_kernel(const StepArgs a) {
 }
 
 
+// MODE from the call: replayed streams and / or the fused policy.  The CFIX > 0 fast paths are Philox-only
+// (launch_comb_step), so they instantiate modes 0 and 2 alone.
 template <int W, typename MaskT, int CFIX, bool PACK>
-int launch_comb_mode(const StepArgs& a, int grid, int block, cudaStream_t s, bool grouped = false) {
+int launch_comb_mode(const StepArgs& a, int grid, int block, cudaStream_t s) {
   const int mode = (a.rng_mode == D2D_RNG_REPLAY ? 1 : 0) | (a.act_mode != 0 ? 2 : 0);
-  if (grouped) {   // many devices per env: 32 envs x 8 device groups per block (Philox modes only)
-    const int g = a.B / 32;
-    if (mode == 0) comb_step_kernel<W, MaskT, CFIX, PACK, 0, kCombGroups><<<g, 256, a.params_bytes, s>>>(a);
-    else comb_step_kernel<W, MaskT, CFIX, PACK, 2, kCombGroups><<<g, 256, a.params_bytes, s>>>(a);
-    D2D_LAUNCHED();
-    return D2D_OK;
+  if (mode == 0) comb_step_kernel<W, MaskT, CFIX, PACK, 0><<<grid, block, a.params_bytes, s>>>(a);
+  else if (mode == 2) comb_step_kernel<W, MaskT, CFIX, PACK, 2><<<grid, block, a.params_bytes, s>>>(a);
+  else if constexpr (CFIX == 0) {
+    if (mode == 1) comb_step_kernel<W, MaskT, CFIX, PACK, 1><<<grid, block, a.params_bytes, s>>>(a);
+    else comb_step_kernel<W, MaskT, CFIX, PACK, 3><<<grid, block, a.params_bytes, s>>>(a);
   }
-  switch (mode) {
-    case 0: comb_step_kernel<W, MaskT, CFIX, PACK, 0><<<grid, block, a.params_bytes, s>>>(a); break;
-    case 1: comb_step_kernel<W, MaskT, CFIX, PACK, 1><<<grid, block, a.params_bytes, s>>>(a); break;
-    case 2: comb_step_kernel<W, MaskT, CFIX, PACK, 2><<<grid, block, a.params_bytes, s>>>(a); break;
-    default: comb_step_kernel<W, MaskT, CFIX, PACK, 3><<<grid, block, a.params_bytes, s>>>(a); break;
-  }
+  D2D_LAUNCHED();
+  return D2D_OK;
+}
+
+// many devices per env: 32 envs x 8 device groups per block (Philox modes only)
+template <int W, int CFIX>
+int launch_comb_grouped(const StepArgs& a, cudaStream_t s) {
+  const int g = a.B / 32;
+  if (a.act_mode == 0) comb_step_kernel<W, uint8_t, CFIX, true, 0, kCombGroups><<<g, 256, a.params_bytes, s>>>(a);
+  else comb_step_kernel<W, uint8_t, CFIX, true, 2, kCombGroups><<<g, 256, a.params_bytes, s>>>(a);
   D2D_LAUNCHED();
   return D2D_OK;
 }
@@ -219,7 +216,7 @@ int launch_comb_mode(const StepArgs& a, int grid, int block, cudaStream_t s, boo
 //  - DH: every device's observation carries DH slots (homogeneous sizes, D = DH), which fixes the rows of each device
 //    at compile time; 0 = the slot count and rows come from the tables at run time;
 //  - the env tables are kernel parameters (CombRunParams: constant-bank operands, no staging, no LDS);
-//  - each Philox call starts at round 2 from the thread's and the call's two-round heads (philox_rk_heads);
+//  - each Philox call starts at round 2 from the thread's and the call's two-round heads (philox.cuh);
 //  - the ack / nack floats are formed once per step and stored for every device;
 //  - observation rows are plain stores, which ptxas may schedule among the Philox rounds (emit_slots_run).
 template <int W, int C, int NF, int DH>
@@ -243,7 +240,7 @@ __global__ void __launch_bounds__(256, 2) comb_run_kernel(const StepArgs a, cons
     chv[k] = chan[idx], discv[k] = a.disc[idx], recvv[k] = a.recv[idx];
   }
   int32_t rew = a.reward_accum ? a.reward[b] : 0;
-  const PhiloxEnvHead eh = philox_env_head(a, env, 0u);   // C <= 8 and arrivals: block 0 only
+  const PhiloxEnvHead eh = philox_env_head(a.key, env, 0u);   // C <= 8 and arrivals: block 0 only
 #pragma unroll 1
   for (int i = 0; i < ra.n_inner; ++i) {
     const uint32_t t = a.t + (uint32_t)i;
@@ -254,8 +251,8 @@ __global__ void __launch_bounds__(256, 2) comb_run_kernel(const StepArgs a, cons
 #pragma unroll
     for (int k = 0; k < NK; ++k) {
       if (NF || k < N) {
-        const uint4 r = philox_rk_heads(a, eh, philox_call_head(a, t, (uint32_t)k | (kPurposePolicy << 16)));
-        const uint32_t want = lanes_below<C>(r, [&p](int) { return p.tp_lt; }, p.tp_all);
+        const uint4 r = philox(a.key, eh, philox_call_head(a.key, t, (uint32_t)k | (kPurposePolicy << 16)));
+        const uint32_t want = lanes_below<C>(r, [&a](int) { return a.tp_lt; }, a.tp_all);
         const uint32_t at = rec_any<W>(rec[k]) ? (want & cmask) : 0u;
         twice |= once & at;
         once |= at;
@@ -284,25 +281,16 @@ __global__ void __launch_bounds__(256, 2) comb_run_kernel(const StepArgs a, cons
         n_success += success;
         rec_pop_earliest<W>(r, success);
         discv[k] += rec_age<W>(r);
-        const uint4 rs = philox_rk_heads(a, eh, philox_call_head(a, t, (uint32_t)k | (kPurposeSwitch << 16)));
+        const uint4 rs = philox(a.key, eh, philox_call_head(a.key, t, (uint32_t)k | (kPurposeSwitch << 16)));
         const uint32_t sw = lanes_below<C>(rs, [&p, k](int c) { return p.sw_lt[k][c]; }, p.sw_all[k]);
         chv[k] = (ch ^ sw) & cmask;
         const int dl = p.deadline[k];
-        // one Philox call per four devices (env_common.cuh: ArrivalWords), drawn when any device of the group is active
+        // arrival_call's draw, from the heads
         if ((k & 3) == 0 && ((active >> k) & 0xFull))
-          arr4 = philox_rk_heads(a, eh, philox_call_head(a, t, (uint32_t)(k >> 2) | (kPurposeArrival << 16)));
+          arr4 = philox(a.key, eh, philox_call_head(a.key, t, word32_field(k) | (kPurposeArrival << 16)));
         if ((active >> k) & 1ull) {
-          const uint32_t u = pick_word(arr4, k & 3);
-          uint32_t arrived = 0;
-          if (p.arrival_kind[k] == D2D_ARRIVAL_BERNOULLI) {
-            arrived = (uint64_t)u < p.bern_thr[k] ? 1u : 0u;
-          } else {
-#pragma unroll 1
-            for (int m = 0; m < D2D_POISSON_KMAX; ++m) {
-              if (u < p.cdf[k][m]) break;   // thresholds are non-decreasing (arrival_from_u)
-              ++arrived;
-            }
-          }
+          const uint32_t arrived =
+              arrival_count(word32(arr4, k), p.arrival_kind[k] == D2D_ARRIVAL_BERNOULLI, p.bern_thr[k], p.cdf[k]);
           rec_set_byte<W>(r, dl - 1, arrived);
           recvv[k] += arrived;
         }
@@ -363,8 +351,8 @@ int launch_comb_step(const StepArgs& a, int N, int C, int mask_bytes, cudaStream
   // grouped mapping: when one thread per env cannot fill the GPU (few envs, many devices each)
   const int ng = ((N + kCombGroups - 1) / kCombGroups + 3) & ~3;
   if (a.rng_mode != D2D_RNG_REPLAY && N >= 32 && a.B % 32 == 0 && a.B < 148 * 1024 && ng * 8 * mask_bytes <= 64) {
-    if (C == 4) return launch_comb_mode<W, uint8_t, 4, true>(a, grid, block, s, true);
-    if (C == 8) return launch_comb_mode<W, uint8_t, 8, true>(a, grid, block, s, true);
+    if (C == 4) return launch_comb_grouped<W, 4>(a, s);
+    if (C == 8) return launch_comb_grouped<W, 8>(a, s);
   }
 #define D2D_CASE(MT, CF) return pack ? launch_comb_mode<W, MT, CF, true>(a, grid, block, s) \
                                      : launch_comb_mode<W, MT, CF, false>(a, grid, block, s)

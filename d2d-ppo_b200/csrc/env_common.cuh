@@ -1,5 +1,5 @@
-// Shared device code of the env kernels: parameter blob, launch arguments, packet-buffer records, Philox draws,
-// f32 row emission.  Included by env_kernels.cu and env_comb_step.cuh.
+// Shared device code of the env kernels: parameter blob, launch arguments, packet-buffer records, f32 row emission.
+// The random streams are philox.cuh's.  Included by env_kernels.cu and env_comb_step.cuh.
 #pragma once
 #include "common.cuh"
 #include "philox.cuh"
@@ -14,6 +14,11 @@ struct EnvParamsHdr {
   int32_t N, C, D, T, homog, kind, sum_dl, obs_rows, state_rows;
   int32_t off_cdf, off_sw, off_nbr_off, off_nbr_idx, total_bytes;
   int32_t self_nbr;   // single-channel env: every neighbourhood is the device itself (env.py:38-39 default)
+  // switch table at off_sw: lane_lt of each threshold, one row of sw_row (a multiple of 8, zero-padded) lanes per
+  // switch call -- device k (combinatorial), devices 8 r .. 8 r + 7 (single channel: lane16_shared), the env's C + 1
+  // channels (selection) -- and sw_all[r] = the lanes of row r whose threshold is 65536
+  int32_t sw_row;
+  uint32_t sw_all[D2D_MAX_AGENTS];
   uint8_t deadline[D2D_MAX_AGENTS];
   uint8_t arrival_kind[D2D_MAX_AGENTS];
   uint16_t obs_off[D2D_MAX_AGENTS];
@@ -42,13 +47,12 @@ struct StepArgs {
   const void* rp_sw;      // replay switch draws of this timestep
   int B;
   uint32_t t;  // timestep being produced (0 = reset)
-  uint32_t k0, k1;
-  uint32_t rk0[10], rk1[10];  // Philox round keys (k + r * W), precomputed on the host: constant-bank operands
+  uint32_t tp_lt, tp_all;  // act_mode 1: the transmission probability for lanes_below, the same for every lane
+  PhiloxKey key;
   uint32_t env_offset;
   uint64_t active;  // bit k: device k draws an arrival at timestep t
   int rng_mode;
   int act_mode;  // 0 = actions from memory, 1 = fused random-access policy
-  uint32_t tp_thr;
   int done_flag;
   int reward_accum;  // 1: reward[b] += this step's reward (d2d_env_run_random_access), 0: overwrite
 };
@@ -170,178 +174,35 @@ __device__ __forceinline__ void rec_emit(const Rec<W>& r, int n, float* p, size_
   }
 }
 
-// Arrival uniforms: one Philox call serves FOUR devices (counter device field = k / 4, device k takes word k % 4), so a
-// step draws ceil(N / 4) arrival calls per env instead of N.
-__device__ __forceinline__ uint32_t pick_word(const uint4& r, int i) {
-  return i == 0 ? r.x : (i == 1 ? r.y : (i == 2 ? r.z : r.w));
+// the arrival call of device k's word32 group, drawn at the group's first device when a device of the group is active
+__device__ __forceinline__ void arrival_call(const StepArgs& a, uint32_t env, int k, uint4& call) {
+  if ((k & 3) == 0 && ((a.active >> k) & 0xFull))
+    call = philox(a.key, env, a.t, word32_field(k) | (kPurposeArrival << 16), 0u);
 }
 
-__device__ __forceinline__ uint32_t arrival_from_u(const EnvParamsHdr* P, const uint32_t* cdf, int k, uint32_t u) {
-  if (P->arrival_kind[k] == D2D_ARRIVAL_BERNOULLI) return (uint64_t)u < P->bern_thr[k] ? 1u : 0u;
-  const uint32_t* c = cdf + k * D2D_POISSON_KMAX;
-  uint32_t n = 0;
-#pragma unroll 1
-  for (int m = 0; m < D2D_POISSON_KMAX; ++m) {
-    if (u < c[m]) break;  // thresholds are non-decreasing
-    ++n;
-  }
-  return n;
-}
-
-// the four arrival words of device group k / 4, fetched once and reused while the device loop stays in the group
-struct ArrivalWords {
-  uint4 r;
-  int group = -1;
-  __device__ __forceinline__ uint32_t get(const StepArgs& a, uint32_t env, int k) {
-    if ((k >> 2) != group) {
-      group = k >> 2;
-      r = philox4x32_10(env, a.t, (uint32_t)group | (kPurposeArrival << 16), 0u, a.k0, a.k1);
-    }
-    return pick_word(r, k & 3);
-  }
-};
-
-// arrival of device k at timestep a.t (only called when the device is active)
+// arrival of device k at timestep a.t (only called when the device is active); `call` is k's arrival_call
 __device__ __forceinline__ uint32_t draw_arrival(const StepArgs& a, const EnvParamsHdr* P, const uint32_t* cdf, int k,
-                                                 int b, ArrivalWords& words) {
+                                                 int b, const uint4& call) {
   if (a.rng_mode == D2D_RNG_REPLAY) return a.rp_arr[(size_t)k * a.B + b];
-  return arrival_from_u(P, cdf, k, words.get(a, a.env_offset + (uint32_t)b, k));
-}
-
-// 16-bit lanes shared by EIGHT devices (single-channel env: one switch / policy bit per device): counter device field
-// = k / 8, device k takes lane k % 8
-struct LaneWords {
-  uint4 r;
-  int group = -1;
-  __device__ __forceinline__ uint32_t get(const StepArgs& a, uint32_t env, int k, uint32_t purpose) {
-    if ((k >> 3) != group) {
-      group = k >> 3;
-      r = philox4x32_10(env, a.t, (uint32_t)group | (purpose << 16), 0u, a.k0, a.k1);
-    }
-    const uint32_t w = pick_word(r, (k & 7) >> 1);
-    return (k & 1) ? (w >> 16) : (w & 0xFFFFu);
-  }
-};
-
-// Philox with the host-precomputed round keys of StepArgs (one constant-bank operand per XOR).
-__device__ __forceinline__ uint4 philox_rk(const StepArgs& a, uint32_t c0, uint32_t c1, uint32_t c2, uint32_t c3) {
-#pragma unroll
-  for (int r = 0; r < 10; ++r) {
-    const uint64_t p0 = (uint64_t)0xD2511F53u * c0;
-    const uint64_t p1 = (uint64_t)0xCD9E8D57u * c2;
-    const uint32_t n0 = (uint32_t)(p1 >> 32) ^ c1 ^ a.rk0[r];
-    const uint32_t n2 = (uint32_t)(p0 >> 32) ^ c3 ^ a.rk1[r];
-    c1 = (uint32_t)p1;
-    c3 = (uint32_t)p0;
-    c0 = n0;
-    c2 = n2;
-  }
-  return make_uint4(c0, c1, c2, c3);
-}
-
-// philox_rk split after its first two rounds, for callers that draw many counters (env, t, dp, blk) with the same env
-// and blk.  With M0 = 0xD2511F53, M1 = 0xCD9E8D57 and hi / lo the halves of the 64-bit product, round 0 gives
-//   c0 = hi(M1 dp) ^ t ^ rk0[0] =: A      c1 = lo(M1 dp)      c2 = hi(M0 env) ^ blk ^ rk1[0] =: X      c3 = lo(M0 env)
-// and round 1 multiplies A and X:
-//   c0 = hi(M1 X) ^ rk0[1] ^ lo(M1 dp)    c1 = lo(M1 X)       c2 = lo(M0 env) ^ rk1[1] ^ hi(M0 A)      c3 = lo(M0 A).
-// So after two rounds the state is three words of (env, blk) (PhiloxEnvHead, once per thread) XOR three words of
-// (t, dp) (PhiloxCallHead, warp-uniform; lo(M1 dp) is a constant for a compile-time dp), and a call continues at round 2.
-struct PhiloxEnvHead {
-  uint32_t e0, e1, e2;
-};
-struct PhiloxCallHead {
-  uint32_t u0, u2, u3;
-};
-
-__device__ __forceinline__ PhiloxEnvHead philox_env_head(const StepArgs& a, uint32_t env, uint32_t blk) {
-  const uint64_t p0 = (uint64_t)0xD2511F53u * env;
-  const uint32_t x = (uint32_t)(p0 >> 32) ^ blk ^ a.rk1[0];
-  const uint64_t p1 = (uint64_t)0xCD9E8D57u * x;
-  return {(uint32_t)(p1 >> 32) ^ a.rk0[1], (uint32_t)p1, (uint32_t)p0 ^ a.rk1[1]};
-}
-
-__device__ __forceinline__ PhiloxCallHead philox_call_head(const StepArgs& a, uint32_t t, uint32_t dev_purpose) {
-  const uint64_t p1 = (uint64_t)0xCD9E8D57u * dev_purpose;
-  const uint32_t c0 = (uint32_t)(p1 >> 32) ^ t ^ a.rk0[0];
-  const uint64_t p0 = (uint64_t)0xD2511F53u * c0;
-  return {(uint32_t)p1, (uint32_t)(p0 >> 32), (uint32_t)p0};
-}
-
-// philox_rk(a, env, t, dp, blk) == philox_rk_heads(a, philox_env_head(a, env, blk), philox_call_head(a, t, dp))
-__device__ __forceinline__ uint4 philox_rk_heads(const StepArgs& a, const PhiloxEnvHead& e, const PhiloxCallHead& u) {
-  uint32_t c0 = e.e0 ^ u.u0, c1 = e.e1, c2 = e.e2 ^ u.u2, c3 = u.u3;
-#pragma unroll
-  for (int r = 2; r < 10; ++r) {
-    const uint64_t p0 = (uint64_t)0xD2511F53u * c0;
-    const uint64_t p1 = (uint64_t)0xCD9E8D57u * c2;
-    const uint32_t n0 = (uint32_t)(p1 >> 32) ^ c1 ^ a.rk0[r];
-    const uint32_t n2 = (uint32_t)(p0 >> 32) ^ c3 ^ a.rk1[r];
-    c1 = (uint32_t)p1;
-    c3 = (uint32_t)p0;
-    c0 = n0;
-    c2 = n2;
-  }
-  return make_uint4(c0, c1, c2, c3);
-}
-
-// bit c of the C 16-bit lanes of r: lane c < thr(c), with the threshold given as lt(c) = thr(c) << 16 (0 for thr =
-// 65536) and all = the lanes whose thr is 65536.  Lane 2j + 1 is the high half of word j, so it is below thr exactly
-// when the word is below thr << 16; lane 2j is compared the same way after a shift.  One compare per lane.
-template <int C, typename LtFn>
-__device__ __forceinline__ uint32_t lanes_below(const uint4& r, LtFn lt, uint32_t all) {
-  const uint32_t w[4] = {r.x, r.y, r.z, r.w};
-  uint32_t m = all;
-#pragma unroll
-  for (int c = 0; c < C; ++c) {
-    const uint32_t v = (c & 1) ? w[c >> 1] : (w[c >> 1] << 16);
-    m |= (uint32_t)(v < lt(c)) << c;
-  }
-  return m;
+  return arrival_count(word32(call, k), P->arrival_kind[k] == D2D_ARRIVAL_BERNOULLI, P->bern_thr[k],
+                       cdf + k * D2D_POISSON_KMAX);
 }
 
 // the per-device tables comb_run_kernel reads, passed by value: kernel parameters sit in the constant bank, so every
 // read is an instruction operand instead of a shared-memory load.  Built once per env (d2d_env_create) for N <= 8,
-// C <= 8; the policy threshold is set per call.
+// C <= 8.
 constexpr int kRunMaxN = 8, kRunMaxC = 8;
 struct CombRunParams {
   uint32_t sw_lt[kRunMaxN][kRunMaxC];   // switch threshold of (device, channel) for lanes_below
   uint32_t sw_all[kRunMaxN];
   uint32_t cdf[kRunMaxN][D2D_POISSON_KMAX];
   uint64_t bern_thr[kRunMaxN];
-  uint32_t tp_lt, tp_all;               // the policy threshold for lanes_below (same for every lane)
   int32_t N;
   int32_t homog_slots;                  // slots per device in the observation: D if homogeneous, else 0 (own deadline)
   uint16_t obs_off[kRunMaxN];
   uint8_t deadline[kRunMaxN];
   uint8_t arrival_kind[kRunMaxN];
 };
-
-// lanes_below's form of a 16-bit-lane threshold thr in [0, 65536]
-__host__ __device__ inline uint32_t lane_lt(uint32_t thr) { return thr >= 65536u ? 0u : thr << 16; }
-
-// bit c = (16-bit lane c < thr(c)) for c < C at Philox timestep t;  CFIX > 0 makes the lane count a compile-time constant
-template <int CFIX, typename ThrFn>
-__device__ __forceinline__ uint32_t lane_mask_rk(const StepArgs& a, uint32_t env, uint32_t t, uint32_t dev_purpose,
-                                                 int C, ThrFn thr) {
-  uint32_t m = 0;
-  const int nl = CFIX ? CFIX : C;
-#pragma unroll
-  for (int blk = 0; blk < (CFIX ? (CFIX + 7) / 8 : 4); ++blk) {
-    if (blk * 8 < nl) {
-      const uint4 r = philox_rk(a, env, t, dev_purpose, (uint32_t)blk);
-      const uint32_t w[4] = {r.x, r.y, r.z, r.w};
-#pragma unroll
-      for (int l = 0; l < 8; ++l) {
-        const int c = blk * 8 + l;
-        if (c < nl) {
-          const uint32_t u = (l & 1) ? (w[l >> 1] >> 16) : (w[l >> 1] & 0xFFFFu);
-          m |= (uint32_t)(u < thr(c)) << c;
-        }
-      }
-    }
-  }
-  return m;
-}
 
 // p += stride floats, as ONE 64-bit multiply-add on the (otherwise idle) FMA pipe
 __device__ __forceinline__ float* next_row(float* p, uint32_t stride) {

@@ -47,16 +47,17 @@ __global__ void __launch_bounds__(256) comb_reset_kernel(const StepArgs a) {
   MaskT* chan = reinterpret_cast<MaskT*>(a.chan);
   const uint32_t cmask = C >= 32 ? 0xFFFFFFFFu : ((1u << C) - 1u);
   for (int b = blockIdx.x * blockDim.x + threadIdx.x; b < a.B; b += gridDim.x * blockDim.x) {
-    ArrivalWords arr_words;
+    uint4 arr = make_uint4(0u, 0u, 0u, 0u);
     for (int k = 0; k < N; ++k) {
       const size_t idx = (size_t)k * B + b;
       Rec<W> r;
 #pragma unroll
       for (int j = 0; j < W; ++j) r.w[j] = 0;
       uint32_t arrived = 0;
+      arrival_call(a, a.env_offset + (uint32_t)b, k, arr);
       const int dl = P->deadline[k];
       if ((a.active >> k) & 1ull) {
-        arrived = draw_arrival(a, P, cdf, k, b, arr_words);
+        arrived = draw_arrival(a, P, cdf, k, b, arr);
         rec_set_byte<W>(r, dl - 1, arrived);
       }
       rec_store<W>(a.buf, idx, r);
@@ -91,7 +92,7 @@ __global__ void __launch_bounds__(256, NK ? 5 : 4) sc_step_kernel(const StepArgs
   extern __shared__ __align__(16) uint8_t smem[];
   const EnvParamsHdr* P = stage_params(a, smem);
   const uint32_t* cdf = reinterpret_cast<const uint32_t*>(smem + P->off_cdf);
-  const uint32_t* swthr = reinterpret_cast<const uint32_t*>(smem + P->off_sw);
+  const uint32_t* swlt = reinterpret_cast<const uint32_t*>(smem + P->off_sw);
   const int32_t* nbr_off = reinterpret_cast<const int32_t*>(smem + P->off_nbr_off);
   const uint8_t* nbr_idx = smem + P->off_nbr_idx;
   const int N = P->N;
@@ -103,11 +104,19 @@ __global__ void __launch_bounds__(256, NK ? 5 : 4) sc_step_kernel(const StepArgs
   const uint8_t* rp_sw = reinterpret_cast<const uint8_t*>(a.rp_sw);
   const bool self_obs = a.obs != nullptr && P->self_nbr != 0;
   constexpr int KR = NK ? NK : 1;
+  constexpr int SL = NK ? NK : 8;   // lanes of a lane16_shared call that can belong to a device
 
   for (int b = blockIdx.x * blockDim.x + threadIdx.x; b < a.B; b += gridDim.x * blockDim.x) {
-    ArrivalWords arr_words;
+    uint4 arr = make_uint4(0u, 0u, 0u, 0u);
     const uint32_t env = a.env_offset + (uint32_t)b;
-    LaneWords pol_lanes, sw_lanes;   // one Philox call per eight devices for the 1-bit policy / switch draws
+    // the 1-bit policy / switch draws of the devices of the current lane16_shared call
+    uint32_t pol_bits = 0, sw_bits = 0;
+    auto policy_bit = [&](int k) {
+      if (lane16_shared_lane(k) == 0)
+        pol_bits = lanes_below<SL>(philox(a.key, env, a.t, lane16_shared_field(k) | (kPurposePolicy << 16), 0u),
+                                   [&a](int) { return a.tp_lt; }, a.tp_all);
+      return (pol_bits >> lane16_shared_lane(k)) & 1u;
+    };
     Rec<W> rec[KR];
     uint32_t chv[KR], wantv[KR];
     // ---- pass 1 (env.py:125-127): attempts and the lone transmitter's channel ----
@@ -125,7 +134,7 @@ __global__ void __launch_bounds__(256, NK ? 5 : 4) sc_step_kernel(const StepArgs
         if (k < N) {
           uint32_t want = wantv[k] != 0;
           if (a.act_mode != 0) {
-            want = pol_lanes.get(a, env, k, kPurposePolicy) < a.tp_thr;
+            want = policy_bit(k);
             if (act_out) act_out[(size_t)k * B + b] = (uint8_t)want;
           }
           const uint64_t at = (want && rec_any<W>(rec[k])) ? 1ull : 0ull;
@@ -141,7 +150,7 @@ __global__ void __launch_bounds__(256, NK ? 5 : 4) sc_step_kernel(const StepArgs
         if (a.act_mode == 0) {
           want = act[idx] != 0;
         } else {
-          want = pol_lanes.get(a, env, k, kPurposePolicy) < a.tp_thr;
+          want = policy_bit(k);
           if (act_out) act_out[idx] = (uint8_t)want;
         }
         const uint64_t at = (want && rec_any<W>(r)) ? 1ull : 0ull;
@@ -187,13 +196,17 @@ __global__ void __launch_bounds__(256, NK ? 5 : 4) sc_step_kernel(const StepArgs
       if (a.rng_mode == D2D_RNG_REPLAY) {
         sw = rp_sw[idx] & 1u;
       } else {
-        sw = sw_lanes.get(a, env, k, kPurposeSwitch) < swthr[k];
+        if (lane16_shared_lane(k) == 0)
+          sw_bits = lanes_below<SL>(philox(a.key, env, a.t, lane16_shared_field(k) | (kPurposeSwitch << 16), 0u),
+                                    [swlt, k](int c) { return swlt[k + c]; }, P->sw_all[lane16_shared_field(k)]);
+        sw = (sw_bits >> lane16_shared_lane(k)) & 1u;
       }
       const uint32_t ch_new = (ch_old ^ sw) & 1u;
       chan[idx] = (uint8_t)ch_new;
       const int dl = P->deadline[k];
+      arrival_call(a, env, k, arr);
       if ((a.active >> k) & 1ull) {                             // :162-180
-        const uint32_t arrived = draw_arrival(a, P, cdf, k, b, arr_words);
+        const uint32_t arrived = draw_arrival(a, P, cdf, k, b, arr);
         rec_set_byte<W>(r, dl - 1, arrived);
         if (arrived) a.recv[idx] = (NK > 0 ? recv_v : a.recv[idx]) + arrived;
       }
@@ -242,9 +255,10 @@ __global__ void __launch_bounds__(256, NK ? 5 : 4) sc_step_kernel(const StepArgs
 // n_inner consecutive random-access steps of ONE episode in one launch (d2d_env_run_random_access without per-step
 // outputs): the env's records, channel bits and counters are loaded once, live in registers for every step and are
 // stored once; each step is the three Philox calls of sc_step_kernel (policy lanes, switch lanes, arrival words: one
-// call each serves all N <= 4 devices) plus the serve / age / switch / arrive logic.  A thread only ever touches its own
-// env, so no step needs a grid-wide barrier.  The per-step kernel at the named c2 size (4,096 envs) is launch-latency
-// bound (8.2 us a step for ~0.5 MB of state); this one is bound by the dependent-issue chain of a single warp.
+// call each serves all N <= 4 devices: lane16_shared and word32 of device field 0) plus the serve / age / switch /
+// arrive logic.  A thread only ever touches its own env, so no step needs a grid-wide barrier.  The per-step kernel at
+// the named c2 size (4,096 envs) is launch-latency bound (8.2 us a step for ~0.5 MB of state); this one is bound by
+// the dependent-issue chain of a single warp.
 // Same Philox counters and the same update order as sc_step_kernel: trajectories are bit-identical.
 // (RunArgs: env_common.cuh)
 template <int W, int NK>
@@ -252,7 +266,7 @@ __global__ void __launch_bounds__(256) sc_run_kernel(const StepArgs a, const Run
   extern __shared__ __align__(16) uint8_t smem[];
   const EnvParamsHdr* P = stage_params(a, smem);
   const uint32_t* cdf = reinterpret_cast<const uint32_t*>(smem + P->off_cdf);
-  const uint32_t* swthr = reinterpret_cast<const uint32_t*>(smem + P->off_sw);
+  const uint32_t* swlt = reinterpret_cast<const uint32_t*>(smem + P->off_sw);
   const int N = P->N;
   const size_t B = (size_t)a.B;
   uint8_t* chan = reinterpret_cast<uint8_t*>(a.chan);
@@ -260,7 +274,7 @@ __global__ void __launch_bounds__(256) sc_run_kernel(const StepArgs a, const Run
   if (b >= a.B) return;
   const uint32_t env = a.env_offset + (uint32_t)b;
   Rec<W> rec[NK];
-  uint32_t chv[NK], discv[NK], recvv[NK], thr_sw[NK];
+  uint32_t chv[NK], discv[NK], recvv[NK], lt_sw[NK];
   int dl[NK];
 #pragma unroll
   for (int k = 0; k < NK; ++k) {
@@ -268,28 +282,27 @@ __global__ void __launch_bounds__(256) sc_run_kernel(const StepArgs a, const Run
     const size_t idx = (size_t)kk * B + b;
     rec[k] = rec_load<W>(a.buf, idx);
     chv[k] = chan[idx] & 1u, discv[k] = a.disc[idx], recvv[k] = a.recv[idx];
-    thr_sw[k] = swthr[kk], dl[k] = P->deadline[kk];
+    lt_sw[k] = swlt[k], dl[k] = P->deadline[kk];
   }
+  const uint32_t all_sw = P->sw_all[0];
   uint32_t st0 = a.stats[b], st1 = a.stats[B + b];
   int32_t rew = a.reward_accum ? a.reward[b] : 0;
-  auto lane16 = [](const uint4& r, int k) {
-    const uint32_t w = pick_word(r, k >> 1);
-    return (k & 1) ? (w >> 16) : (w & 0xFFFFu);
-  };
 #pragma unroll 1
   for (int i = 0; i < ra.n_inner; ++i) {
     const uint32_t t = a.t + (uint32_t)i;
     const uint64_t active = ra.active[ra.t_plain + i];
     // the three draws are independent of the state: their Philox rounds interleave
-    const uint4 pol = philox_rk(a, env, t, kPurposePolicy << 16, 0u);
-    const uint4 sw4 = philox_rk(a, env, t, kPurposeSwitch << 16, 0u);
+    const uint32_t pol = lanes_below<NK>(philox(a.key, env, t, kPurposePolicy << 16, 0u),
+                                         [&a](int) { return a.tp_lt; }, a.tp_all);
+    const uint32_t sw = lanes_below<NK>(philox(a.key, env, t, kPurposeSwitch << 16, 0u),
+                                        [&lt_sw](int k) { return lt_sw[k]; }, all_sw);
     uint4 ar4 = make_uint4(0u, 0u, 0u, 0u);
-    if (active) ar4 = philox_rk(a, env, t, kPurposeArrival << 16, 0u);
+    if (active) ar4 = philox(a.key, env, t, kPurposeArrival << 16, 0u);
     uint32_t att = 0, good = 0;                                 // env.py:125-127
 #pragma unroll
     for (int k = 0; k < NK; ++k) {
       if (k < N) {
-        const uint32_t at = (lane16(pol, k) < a.tp_thr && rec_any<W>(rec[k])) ? 1u : 0u;
+        const uint32_t at = (((pol >> k) & 1u) && rec_any<W>(rec[k])) ? 1u : 0u;
         att |= at << k;
         good |= (at & chv[k]) << k;
       }
@@ -305,9 +318,10 @@ __global__ void __launch_bounds__(256) sc_run_kernel(const StepArgs a, const Run
       if (k < N) {
         rec_pop_earliest<W>(rec[k], decoded && ((att >> k) & 1u));   // :137-144
         discv[k] += rec_age<W>(rec[k]);                              // :157-158
-        chv[k] ^= lane16(sw4, k) < thr_sw[k] ? 1u : 0u;              // :107-109
+        chv[k] ^= (sw >> k) & 1u;                                    // :107-109
         if ((active >> k) & 1ull) {                                  // :162-180
-          const uint32_t arrived = arrival_from_u(P, cdf, k, pick_word(ar4, k));
+          const uint32_t arrived = arrival_count(word32(ar4, k), P->arrival_kind[k] == D2D_ARRIVAL_BERNOULLI,
+                                                 P->bern_thr[k], cdf + k * D2D_POISSON_KMAX);
           rec_set_byte<W>(rec[k], dl[k] - 1, arrived);
           recvv[k] += arrived;
         }
@@ -333,14 +347,15 @@ __global__ void __launch_bounds__(256) sc_run_kernel(const StepArgs a, const Run
 // The same episode-in-one-launch loop with FOUR LANES PER ENV (lane = device) for small batches, where sc_run_kernel is
 // bound by the dependent-issue chain of its few warps (4,096 envs = 128 warps on 148 SMs): every lane keeps ONE device's
 // record and counters, lanes 0 / 1 / 2 of a quad compute the policy / switch / arrival Philox call (one call per lane
-// and step instead of three per thread) and hand the words round with shuffles, the attempt bits meet in a ballot.
+// and step instead of three per thread) and hand the policy / switch bits and the arrival words round with shuffles,
+// the attempt bits meet in a ballot.
 // Same Philox counters and update order: trajectories are bit-identical to sc_run_kernel / sc_step_kernel.
 template <int W>
 __global__ void __launch_bounds__(128) sc_run_lanes_kernel(const StepArgs a, const RunArgs ra) {
   extern __shared__ __align__(16) uint8_t smem[];
   const EnvParamsHdr* P = stage_params(a, smem);
   const uint32_t* cdf = reinterpret_cast<const uint32_t*>(smem + P->off_cdf);
-  const uint32_t* swthr = reinterpret_cast<const uint32_t*>(smem + P->off_sw);
+  const uint32_t* swlt = reinterpret_cast<const uint32_t*>(smem + P->off_sw);
   const int N = P->N;
   const size_t B = (size_t)a.B;
   uint8_t* chan = reinterpret_cast<uint8_t*>(a.chan);
@@ -355,7 +370,11 @@ __global__ void __launch_bounds__(128) sc_run_lanes_kernel(const StepArgs a, con
   const uint32_t env = a.env_offset + (uint32_t)b;
   Rec<W> rec = rec_load<W>(a.buf, idx);
   uint32_t chv = chan[idx] & 1u, discv = a.disc[idx], recvv = a.recv[idx];
-  const uint32_t thr_sw = swthr[kk];
+  // lanes 0 / 1: the lanes_below thresholds of the policy / switch call (lane16_shared, device field 0)
+  uint32_t lt[4];
+#pragma unroll
+  for (int c = 0; c < 4; ++c) lt[c] = k == 0 ? a.tp_lt : swlt[c];
+  const uint32_t all = k == 0 ? a.tp_all : P->sw_all[0];
   const int dl = P->deadline[kk];
   uint32_t st0 = a.stats[b], st1 = a.stats[B + b];
   int32_t rew = a.reward_accum ? a.reward[b] : 0;
@@ -365,17 +384,12 @@ __global__ void __launch_bounds__(128) sc_run_lanes_kernel(const StepArgs a, con
     const uint64_t active = ra.active[ra.t_plain + i];
     // lane 0: policy words, lane 1: switch words, lane 2: arrival words (only when a device is active this step)
     uint4 r = make_uint4(0u, 0u, 0u, 0u);
-    if (k < 2 || (k == 2 && active)) r = philox_rk(a, env, t, (k == 0 ? kPurposePolicy : (k == 1 ? kPurposeSwitch : kPurposeArrival)) << 16, 0u);
-    // 16-bit policy / switch lanes of device k live in word k >> 1 (x or y for k < 4); the arrival word is word k
-    const uint32_t px = __shfl_sync(0xFFFFFFFFu, r.x, quad0), py = __shfl_sync(0xFFFFFFFFu, r.y, quad0);
-    const uint32_t sx = __shfl_sync(0xFFFFFFFFu, r.x, quad0 + 1), sy = __shfl_sync(0xFFFFFFFFu, r.y, quad0 + 1);
-    const uint32_t ax = __shfl_sync(0xFFFFFFFFu, r.x, quad0 + 2), ay = __shfl_sync(0xFFFFFFFFu, r.y, quad0 + 2);
-    const uint32_t az = __shfl_sync(0xFFFFFFFFu, r.z, quad0 + 2), aw = __shfl_sync(0xFFFFFFFFu, r.w, quad0 + 2);
-    const uint32_t pw = (k >> 1) ? py : px, sw = (k >> 1) ? sy : sx;
-    const uint32_t pol16 = (k & 1) ? (pw >> 16) : (pw & 0xFFFFu);
-    const uint32_t sw16 = (k & 1) ? (sw >> 16) : (sw & 0xFFFFu);
-    const uint32_t arw = k == 0 ? ax : (k == 1 ? ay : (k == 2 ? az : aw));
-    const bool at = live && pol16 < a.tp_thr && rec_any<W>(rec);          // env.py:125-127
+    if (k < 2 || (k == 2 && active)) r = philox(a.key, env, t, (k == 0 ? kPurposePolicy : (k == 1 ? kPurposeSwitch : kPurposeArrival)) << 16, 0u);
+    const uint32_t bits = lanes_below<4>(r, [&lt](int c) { return lt[c]; }, all);
+    const uint32_t pol = __shfl_sync(0xFFFFFFFFu, bits, quad0), sw = __shfl_sync(0xFFFFFFFFu, bits, quad0 + 1);
+    const uint4 ar = make_uint4(__shfl_sync(0xFFFFFFFFu, r.x, quad0 + 2), __shfl_sync(0xFFFFFFFFu, r.y, quad0 + 2),
+                                __shfl_sync(0xFFFFFFFFu, r.z, quad0 + 2), __shfl_sync(0xFFFFFFFFu, r.w, quad0 + 2));
+    const bool at = live && ((pol >> k) & 1u) && rec_any<W>(rec);       // env.py:125-127
     const uint32_t att = (__ballot_sync(0xFFFFFFFFu, at) >> quad0) & 0xFu;
     const uint32_t good = (__ballot_sync(0xFFFFFFFFu, at && chv) >> quad0) & 0xFu;
     const int n_att = __popc(att);                                        // :130-152
@@ -387,9 +401,10 @@ __global__ void __launch_bounds__(128) sc_run_lanes_kernel(const StepArgs a, con
     if (live) {
       rec_pop_earliest<W>(rec, decoded && at);                            // :137-144
       discv += rec_age<W>(rec);                                           // :157-158
-      chv ^= sw16 < thr_sw ? 1u : 0u;                                     // :107-109
+      chv ^= (sw >> k) & 1u;                                              // :107-109
       if ((active >> k) & 1ull) {                                         // :162-180
-        const uint32_t arrived = arrival_from_u(P, cdf, k, arw);
+        const uint32_t arrived = arrival_count(word32(ar, k), P->arrival_kind[k] == D2D_ARRIVAL_BERNOULLI,
+                                               P->bern_thr[k], cdf + k * D2D_POISSON_KMAX);
         rec_set_byte<W>(rec, dl - 1, arrived);
         recvv += arrived;
       }
@@ -420,15 +435,16 @@ __global__ void __launch_bounds__(256) sc_reset_kernel(const StepArgs a) {
   const size_t B = (size_t)a.B;
   uint8_t* chan = reinterpret_cast<uint8_t*>(a.chan);
   for (int b = blockIdx.x * blockDim.x + threadIdx.x; b < a.B; b += gridDim.x * blockDim.x) {
-    ArrivalWords arr_words;
+    uint4 arr = make_uint4(0u, 0u, 0u, 0u);
     for (int k = 0; k < N; ++k) {
       const size_t idx = (size_t)k * B + b;
       Rec<W> r;
 #pragma unroll
       for (int j = 0; j < W; ++j) r.w[j] = 0;
       uint32_t arrived = 0;
+      arrival_call(a, a.env_offset + (uint32_t)b, k, arr);
       if ((a.active >> k) & 1ull) {
-        arrived = draw_arrival(a, P, cdf, k, b, arr_words);
+        arrived = draw_arrival(a, P, cdf, k, b, arr);
         rec_set_byte<W>(r, P->deadline[k] - 1, arrived);
       }
       rec_store<W>(a.buf, idx, r);
@@ -469,7 +485,7 @@ __global__ void __launch_bounds__(256, 4) sel_step_kernel(const StepArgs a) {
   extern __shared__ __align__(16) uint8_t smem[];
   const EnvParamsHdr* P = stage_params(a, smem);
   const uint32_t* cdf = reinterpret_cast<const uint32_t*>(smem + P->off_cdf);
-  const uint32_t* swthr = reinterpret_cast<const uint32_t*>(smem + P->off_sw);
+  const uint32_t* swlt = reinterpret_cast<const uint32_t*>(smem + P->off_sw);
   const int N = P->N, C1 = P->C + 1;
   const size_t B = (size_t)a.B;
   const uint32_t Bu = (uint32_t)a.B;
@@ -480,12 +496,12 @@ __global__ void __launch_bounds__(256, 4) sel_step_kernel(const StepArgs a) {
   const uint32_t cmask = C1 >= 32 ? 0xFFFFFFFFu : ((1u << C1) - 1u);
   const int n_planes = 32 - __clz(N);     // a channel is picked by at most N devices: bits(N) counter planes suffice
   // act_mode 1: fused RandomAccess policy (algorithms/baselines.py:10-14): every device draws a channel id uniformly
-  // from 0..C (0 = stay idle) -- floor(u32 (C + 1) / 2^32) of the Philox policy stream, one call per four devices --
+  // from 0..C (0 = stay idle) -- floor(u32 (C + 1) / 2^32) of device k's word32 of the policy stream --
   // and devices without a packet are set to 0.  The drawn ids are kept in a local array for the second pass.
   const bool fused_policy = a.act_mode != 0;
 
   for (int b = blockIdx.x * blockDim.x + threadIdx.x; b < a.B; b += gridDim.x * blockDim.x) {
-    ArrivalWords arr_words;
+    uint4 arr = make_uint4(0u, 0u, 0u, 0u);
     const uint32_t env = a.env_offset + (uint32_t)b;
     const uint32_t ch = chan[b];
     // ---- pass 1 (channel_selection_env.py:124-128): per-channel attempt counts, bit-sliced ----
@@ -500,8 +516,8 @@ __global__ void __launch_bounds__(256, 4) sel_step_kernel(const StepArgs a) {
       const Rec<W> r = rec_load<W>(a.buf, idx);
       uint32_t sel;
       if (fused_policy) {
-        if ((k & 3) == 0) pol4 = philox4x32_10(env, a.t, (uint32_t)(k >> 2) | (kPurposePolicy << 16), 0u, a.k0, a.k1);
-        sel = rec_any<W>(r) ? __umulhi(pick_word(pol4, k & 3), (uint32_t)C1) : 0u;
+        if ((k & 3) == 0) pol4 = philox(a.key, env, a.t, word32_field(k) | (kPurposePolicy << 16), 0u);
+        sel = rec_any<W>(r) ? __umulhi(word32(pol4, k), (uint32_t)C1) : 0u;
         drawn[k] = (uint8_t)sel;
         if (act_out) act_out[idx] = (uint8_t)sel;
       } else {
@@ -554,8 +570,9 @@ __global__ void __launch_bounds__(256, 4) sel_step_kernel(const StepArgs a) {
       const uint32_t expired = rec_age<W>(r);
       if (expired) a.disc[idx] = disc_v + expired;
       const int dl = P->deadline[k];
+      arrival_call(a, env, k, arr);
       if ((a.active >> k) & 1ull) {
-        const uint32_t arrived = draw_arrival(a, P, cdf, k, b, arr_words);
+        const uint32_t arrived = draw_arrival(a, P, cdf, k, b, arr);
         rec_set_byte<W>(r, dl - 1, arrived);
         if (arrived) a.recv[idx] = recv_v + arrived;
       }
@@ -567,8 +584,8 @@ __global__ void __launch_bounds__(256, 4) sel_step_kernel(const StepArgs a) {
     if (a.rng_mode == D2D_RNG_REPLAY) {
       sw = rp_sw[b];
     } else {
-      sw = philox_lane_mask(env, a.t, kEnvLevelDevice | (kPurposeSwitch << 16), C1, a.k0, a.k1,
-                            [swthr](int c) { return swthr[c]; });
+      sw = lanes16_below<0>(a.key, env, a.t, kEnvLevelDevice | (kPurposeSwitch << 16), C1,
+                            [swlt](int c) { return swlt[c]; }, P->sw_all[0]);
     }
     const uint32_t ch_new = (ch ^ sw) & cmask;
     chan[b] = ch_new;
@@ -630,15 +647,16 @@ __global__ void __launch_bounds__(256) sel_reset_kernel(const StepArgs a) {
   uint32_t* chan = reinterpret_cast<uint32_t*>(a.chan);
   const uint32_t cmask = C1 >= 32 ? 0xFFFFFFFFu : ((1u << C1) - 1u);
   for (int b = blockIdx.x * blockDim.x + threadIdx.x; b < a.B; b += gridDim.x * blockDim.x) {
-    ArrivalWords arr_words;
+    uint4 arr = make_uint4(0u, 0u, 0u, 0u);
     for (int k = 0; k < N; ++k) {
       const size_t idx = (size_t)k * B + b;
       Rec<W> r;
 #pragma unroll
       for (int j = 0; j < W; ++j) r.w[j] = 0;
       uint32_t arrived = 0;
+      arrival_call(a, a.env_offset + (uint32_t)b, k, arr);
       if ((a.active >> k) & 1ull) {
-        arrived = draw_arrival(a, P, cdf, k, b, arr_words);
+        arrived = draw_arrival(a, P, cdf, k, b, arr);
         rec_set_byte<W>(r, P->deadline[k] - 1, arrived);
       }
       rec_store<W>(a.buf, idx, r);
@@ -857,13 +875,23 @@ extern "C" int d2d_env_create(const d2d_env_config* cfg, d2d_env** out) {
   auto align16 = [](int x) { return (x + 15) & ~15; };
   EnvParamsHdr h;
   memset(&h, 0, sizeof(h));
+  // the switch table in lanes_below's form (EnvParamsHdr): rows of sw_lanes thresholds, padded to sw_row
+  const int sw_lanes = e->kind == D2D_ENV_COMBINATORIAL ? C : (e->kind == D2D_ENV_SINGLE_CHANNEL ? 8 : C + 1);
+  const int sw_rows = (n_sw + sw_lanes - 1) / sw_lanes;
+  h.sw_row = (sw_lanes + 7) & ~7;
+  std::vector<uint32_t> sw_lt((size_t)sw_rows * h.sw_row, 0u);
+  for (int i = 0; i < n_sw; ++i) {
+    const uint32_t thr = cfg->switch_thr[i];
+    sw_lt[(size_t)(i / sw_lanes) * h.sw_row + i % sw_lanes] = lane_lt(thr);
+    h.sw_all[i / sw_lanes] |= (uint32_t)(thr >= 65536u) << (i % sw_lanes);
+  }
   h.N = N, h.C = C, h.D = e->D, h.T = e->T, h.homog = e->homog, h.kind = e->kind, h.sum_dl = e->sum_dl;
   h.self_nbr = 1;
   for (int k = 0; k < N && e->kind == D2D_ENV_SINGLE_CHANNEL; ++k)
     if (nbr_off[k + 1] - nbr_off[k] != 1 || nbr_idx[nbr_off[k]] != k) h.self_nbr = 0;
   h.off_cdf = align16((int)sizeof(EnvParamsHdr));
   h.off_sw = h.off_cdf + align16(N * D2D_POISSON_KMAX * 4);
-  h.off_nbr_off = h.off_sw + align16(n_sw * 4);
+  h.off_nbr_off = h.off_sw + align16((int)sw_lt.size() * 4);
   h.off_nbr_idx = h.off_nbr_off + align16((N + 1) * 4);
   h.total_bytes = h.off_nbr_idx + align16((int)nbr_idx.size() + 1);
   int row = 0, srow = 0;
@@ -898,17 +926,14 @@ extern "C" int d2d_env_create(const d2d_env_config* cfg, d2d_env** out) {
     CombRunParams& q = e->comb_run;
     q.N = N, q.homog_slots = e->homog ? e->D : 0;
     for (int k = 0; k < N; ++k) {
-      for (int c = 0; c < C; ++c) {
-        const uint32_t thr = cfg->switch_thr[k * C + c];
-        q.sw_lt[k][c] = lane_lt(thr);
-        q.sw_all[k] |= (uint32_t)(thr >= 65536u) << c;
-      }
+      for (int c = 0; c < C; ++c) q.sw_lt[k][c] = sw_lt[(size_t)k * h.sw_row + c];
+      q.sw_all[k] = h.sw_all[k];
       memcpy(q.cdf[k], cfg->poisson_cdf + (size_t)k * D2D_POISSON_KMAX, D2D_POISSON_KMAX * 4);
       q.bern_thr[k] = h.bern_thr[k], q.obs_off[k] = h.obs_off[k];
       q.deadline[k] = h.deadline[k], q.arrival_kind[k] = h.arrival_kind[k];
     }
   }
-  memcpy(blob.data() + h.off_sw, cfg->switch_thr, (size_t)n_sw * 4);
+  memcpy(blob.data() + h.off_sw, sw_lt.data(), sw_lt.size() * 4);
   memcpy(blob.data() + h.off_nbr_off, nbr_off.data(), (size_t)(N + 1) * 4);
   if (!nbr_idx.empty()) memcpy(blob.data() + h.off_nbr_idx, nbr_idx.data(), nbr_idx.size());
   e->params_bytes = h.total_bytes;
@@ -965,6 +990,12 @@ extern "C" int d2d_env_set_replay(d2d_env* e, const uint8_t* arrivals, const voi
   return D2D_OK;
 }
 
+// the fused random-access policy's Bernoulli(tp) on each 16-bit lane (thr16), in lanes_below's form
+static void set_policy_thr(StepArgs& a, double tp) {
+  const uint32_t thr = (uint32_t)std::min(65536.0, std::max(0.0, std::floor(tp * 65536.0 + 0.5)));
+  a.act_mode = 1, a.tp_lt = lane_lt(thr), a.tp_all = thr >= 65536u ? 0xFFFFFFFFu : 0u;
+}
+
 static int fill_args(d2d_env* e, StepArgs& a, uint32_t t, const char* who) {
   memset(&a, 0, sizeof(a));
   a.buf = e->buf, a.chan = e->chan, a.disc = e->disc, a.recv = e->recv, a.stats = e->stats;
@@ -972,8 +1003,7 @@ static int fill_args(d2d_env* e, StepArgs& a, uint32_t t, const char* who) {
   // Philox streams: the counter's timestep field is t + episode * (T + 1), so that every episode of an env draws
   // fresh traffic (replayed streams, arrival phases and the done flag use the plain episode timestep)
   const uint32_t t_ctr = t + (uint32_t)((unsigned long long)std::max<long long>(e->episode, 0) * (unsigned)(e->T + 1));
-  a.B = e->B, a.t = t_ctr, a.k0 = (uint32_t)(e->seed & 0xFFFFFFFFull), a.k1 = (uint32_t)(e->seed >> 32);
-  for (int r = 0; r < 10; ++r) a.rk0[r] = a.k0 + (uint32_t)r * 0x9E3779B9u, a.rk1[r] = a.k1 + (uint32_t)r * 0xBB67AE85u;
+  a.B = e->B, a.t = t_ctr, a.key = philox_key(e->seed);
   a.env_offset = (uint32_t)e->env_offset, a.active = e->active[t], a.rng_mode = e->rng_mode;
   a.done_flag = (int)t >= e->T;
   if (e->rng_mode == D2D_RNG_REPLAY) {
@@ -1088,8 +1118,7 @@ extern "C" int d2d_env_step_random_access(d2d_env* e, double tp, void* actions_o
   int rc = fill_args(e, a, (uint32_t)(e->t + 1), "d2d_env_step_random_access");
   if (rc) return rc;
   a.actions_out = actions_out, a.obs = obs, a.state = state, a.reward = reward, a.done = done, a.ack = ack;
-  a.act_mode = 1;
-  a.tp_thr = (uint32_t)std::min(65536.0, std::max(0.0, std::floor(tp * 65536.0 + 0.5)));
+  set_policy_thr(a, tp);
   return env_step_impl(e, a, stream);
 }
 
@@ -1110,7 +1139,6 @@ extern "C" int d2d_env_run_random_access(d2d_env* e, double tp, int n_steps, int
       return D2D_ERR_STATE;
     }
   }
-  const uint32_t tp_thr = (uint32_t)std::min(65536.0, std::max(0.0, std::floor(tp * 65536.0 + 0.5)));
   // the steps of one episode run inside ONE kernel with the env state in registers: the single-channel env with N <= 4
   // and no per-step observation rows (sc_run_kernel), the combinatorial env with N <= 8, C = 4 or 8 and the
   // one-thread-per-env mapping, observations at any stride or none (comb_run_kernel); never with state rows
@@ -1133,17 +1161,16 @@ extern "C" int d2d_env_run_random_access(d2d_env* e, double tp, int n_steps, int
       int rc = fill_args(e, a, (uint32_t)(e->t + 1), "d2d_env_run_random_access");
       if (rc) return rc;
       a.reward = reward + (size_t)i * reward_step_stride, a.done = done;
-      a.act_mode = 1, a.tp_thr = tp_thr, a.reward_accum = reward_accumulate ? 1 : 0;
+      set_policy_thr(a, tp);
+      a.reward_accum = reward_accumulate ? 1 : 0;
       a.done_flag = e->t + n_inner >= e->T;
       RunArgs ra;
       ra.active = e->active_dev, ra.t_plain = e->t + 1, ra.n_inner = n_inner, ra.reward_stride = reward_step_stride;
       ra.obs_stride = obs_step_stride;
       if (comb_multi) {
         a.obs = obs_i;
-        CombRunParams p = e->comb_run;
-        p.tp_lt = lane_lt(tp_thr), p.tp_all = tp_thr >= 65536u ? (1u << e->C) - 1u : 0u;
-        rc = e->W == 2 ? launch_comb_run<2>(a, ra, p, e->C, as_stream(stream))
-                       : launch_comb_run<4>(a, ra, p, e->C, as_stream(stream));
+        rc = e->W == 2 ? launch_comb_run<2>(a, ra, e->comb_run, e->C, as_stream(stream))
+                       : launch_comb_run<4>(a, ra, e->comb_run, e->C, as_stream(stream));
         if (rc) return rc;
       } else if (e->B <= kRunLanesMaxEnvs) {
         // small batches: four lanes per env (sc_run_lanes_kernel), 64-thread blocks = 16 envs spread over the SMs
@@ -1167,7 +1194,8 @@ extern "C" int d2d_env_run_random_access(d2d_env* e, double tp, int n_steps, int
     int rc = fill_args(e, a, (uint32_t)(e->t + 1), "d2d_env_run_random_access");
     if (rc) return rc;
     a.obs = obs_i, a.state = state_i, a.reward = reward + (size_t)i * reward_step_stride, a.done = done;
-    a.act_mode = 1, a.tp_thr = tp_thr, a.reward_accum = reward_accumulate ? 1 : 0;
+    set_policy_thr(a, tp);
+    a.reward_accum = reward_accumulate ? 1 : 0;
     if ((rc = env_step_impl(e, a, stream))) return rc;
     if (steps_done) *steps_done = i + 1;
   }
@@ -1331,7 +1359,7 @@ extern "C" int d2d_env_import_state(d2d_env* e, const uint8_t* buffers, const vo
 // is closest to its deadline transmits (ties: the first such device, as numpy's argmin); a uniformly drawn device when
 // no buffer holds a packet.  use_channel: devices whose channel is bad are skipped (:91-94).  One thread per env.
 __global__ void edf_policy_kernel(const uint32_t* __restrict__ buf, const uint8_t* __restrict__ chan, int N, int B,
-                                  int W, int use_channel, uint8_t* __restrict__ actions, uint32_t k0, uint32_t k1,
+                                  int W, int use_channel, uint8_t* __restrict__ actions, const PhiloxKey key,
                                   uint32_t env_offset, uint32_t t, uint32_t episode) {
   for (int b = blockIdx.x * blockDim.x + threadIdx.x; b < B; b += gridDim.x * blockDim.x) {
     int best = -1, best_d = 1 << 30;
@@ -1346,7 +1374,7 @@ __global__ void edf_policy_kernel(const uint32_t* __restrict__ buf, const uint8_
       if (d >= 0 && d < best_d) best_d = d, best = i;
     }
     if (best < 0) {
-      const uint4 r = philox4x32_10(env_offset + (uint32_t)b, t, kPurposePolicy << 16, episode, k0, k1);
+      const uint4 r = philox(key, env_offset + (uint32_t)b, t, kPurposePolicy << 16, episode);
       best = (int)(((unsigned long long)r.x * (unsigned long long)N) >> 32);
     }
     for (int i = 0; i < N; ++i) actions[(size_t)i * B + b] = (uint8_t)(i == best);
@@ -1359,8 +1387,7 @@ extern "C" int d2d_env_policy_edf(const d2d_env* e, int use_channel, uint8_t* ac
   D2D_REQUIRE(e->is_reset, "d2d_env_policy_edf: call reset first");
   edf_policy_kernel<<<grid_for(e->B, 128), 128, 0, as_stream(stream)>>>(
       e->buf, reinterpret_cast<const uint8_t*>(e->chan), e->N, e->B, e->W, use_channel != 0, actions,
-      (uint32_t)(e->seed & 0xFFFFFFFFull), (uint32_t)(e->seed >> 32), (uint32_t)e->env_offset, (uint32_t)e->t,
-      (uint32_t)e->episode);
+      philox_key(e->seed), (uint32_t)e->env_offset, (uint32_t)e->t, (uint32_t)e->episode);
   D2D_LAUNCHED();
   return D2D_OK;
 }

@@ -1094,7 +1094,7 @@ extern "C" int d2d_policy_head(int N, int B, int O, int n_t, int out_kind, int d
   h.logits = make_view(const_cast<float*>(logits), (long long)N * O * B, 0, N, O, B);
   if (probs) h.probs = make_view(probs, (long long)N * O * B, 0, N, O, B);
   h.t0 = 0, h.t1 = n_t, h.act_mode = act_mode, h.actions = actions, h.logp = logp, h.entropy = entropy;
-  h.k0 = (uint32_t)(seed & 0xFFFFFFFFull), h.k1 = (uint32_t)(seed >> 32), h.env_offset = (uint32_t)env_offset;
+  h.key = philox_key(seed), h.env_offset = (uint32_t)env_offset;
   h.t_abs_off = t_abs0;
   const long long rows = (long long)n_t * B;
   policy_head_kernel<<<dim3(grid_for(rows, 128), N), 128, 0, as_stream(stream)>>>(h);
@@ -1121,7 +1121,7 @@ extern "C" int d2d_net_rollout_act(d2d_net* n, const float* params, const float*
     HeadArgs h;
     fill_head(h, N, B, O, n->out_kind, dist_kind);
     h.act_mode = act_mode, h.actions = actions, h.logp = logp, h.act_t_off = -t;
-    h.k0 = (uint32_t)(seed & 0xFFFFFFFFull), h.k1 = (uint32_t)(seed >> 32), h.env_offset = (uint32_t)env_offset;
+    h.key = philox_key(seed), h.env_offset = (uint32_t)env_offset;
     h.t_abs_off = t_abs0 - t;
     const View hl = make_view(hs_ptr(n, c, false, n->L - 1), H * NB, -t, N, H, B);
     const View lgo = make_view(logits_out, O * NB, -t, N, O, B);   // p == nullptr: outputs are not written
@@ -1261,7 +1261,7 @@ extern "C" int d2d_q_select(int N, int B, int O, const float* q, int act_mode, f
   memset(&a, 0, sizeof(a));
   a.q = q, a.action = action_idx, a.mask = action_mask, a.mask_bytes = mask_bytes, a.N = N, a.B = B, a.O = O;
   a.act_mode = act_mode, a.epsilon = epsilon, a.ready = training_ready != 0, a.n_random = n_random;
-  a.k0 = (uint32_t)(seed & 0xFFFFFFFFull), a.k1 = (uint32_t)(seed >> 32), a.env_offset = (uint32_t)env_offset;
+  a.key = philox_key(seed), a.env_offset = (uint32_t)env_offset;
   a.t_abs = t_abs;
   q_select_kernel<<<grid_for((long long)N * B, 128), 128, 0, as_stream(stream)>>>(a);
   D2D_LAUNCHED();

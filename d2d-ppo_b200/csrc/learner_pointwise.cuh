@@ -103,7 +103,8 @@ struct DistArgs {
   int act_t_off;
   float* logp;              // [t][N][B] (same strides as actions)
   float* entropy;           // may be null
-  uint32_t k0, k1, env_offset;
+  PhiloxKey key;
+  uint32_t env_offset;
   int t_abs_off;            // Philox timestep = t + t_abs_off
 };
 
@@ -198,8 +199,8 @@ __device__ __forceinline__ void policy_select(const DistArgs& a, int g, int t, i
         for (int j = 0; j < a.A; ++j) act |= (uint32_t)(p[j] > 0.5f) << j;      // d2d_ppo.py:166
       } else {
         for (int blk = 0; blk * 4 < a.A; ++blk) {
-          const uint4 r = philox4x32_10(a.env_offset + (uint32_t)b, (uint32_t)(t + a.t_abs_off),
-                                        (uint32_t)g | (kPurposePolicy << 16), (uint32_t)blk, a.k0, a.k1);
+          const uint4 r = philox(a.key, a.env_offset + (uint32_t)b, (uint32_t)(t + a.t_abs_off),
+                                 (uint32_t)g | (kPurposePolicy << 16), (uint32_t)blk);
           const uint32_t u[4] = {r.x, r.y, r.z, r.w};
           for (int l = 0; l < 4 && blk * 4 + l < a.A; ++l) {
             const int j = blk * 4 + l;
@@ -214,8 +215,8 @@ __device__ __forceinline__ void policy_select(const DistArgs& a, int g, int t, i
         for (int j = 1; j < a.A; ++j)
           if (p[j] > best) best = p[j], act = (uint32_t)j;            // argmax, first maximum (d2d_ppo.py:176)
       } else {
-        const uint4 r = philox4x32_10(a.env_offset + (uint32_t)b, (uint32_t)(t + a.t_abs_off),
-                                      (uint32_t)g | (kPurposePolicy << 16), 0u, a.k0, a.k1);
+        const uint4 r = philox(a.key, a.env_offset + (uint32_t)b, (uint32_t)(t + a.t_abs_off),
+                               (uint32_t)g | (kPurposePolicy << 16), 0u);
         double s = 0.0;
         for (int j = 0; j < a.A; ++j) s += (double)p[j];
         const double uu = ((double)r.x + 0.5) * (1.0 / 4294967296.0) * s;

@@ -1,6 +1,6 @@
-"""The two-round split of Philox4x32-10 that comb_run_kernel uses (env_common.cuh: philox_env_head, philox_call_head,
-philox_rk_heads), restated in numpy and checked against oracle.philox_np.philox4x32_10 over random counters and keys,
-block words other than 0 included."""
+"""The two-round split of Philox4x32-10 that comb_run_kernel uses (philox.cuh: philox_env_head, philox_call_head and
+the philox overload that continues from them), restated in numpy and checked against oracle.philox_np.philox4x32_10
+over random counters and keys, block words other than 0 included."""
 import numpy as np
 
 from oracle import philox_np as px
