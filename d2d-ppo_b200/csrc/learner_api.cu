@@ -53,13 +53,17 @@ struct d2d_net {
 // ------------------------------------------------------------------------------------------------
 // helpers
 // ------------------------------------------------------------------------------------------------
-static View make_view(float* p, long long t_stride, int t_off, int N, int feat_per_agent, int B) {
+static View make_view(float* p, long long t_stride, int t_off, int N, int feat_per_agent) {
   View v;
   memset(&v, 0, sizeof(v));
   v.p = p, v.t_stride = t_stride, v.t_off = t_off;
   for (int g = 0; g < N; ++g) v.f_off[g] = g * feat_per_agent;
-  (void)B;
   return v;
+}
+
+// a buffer of the net's layout with F features per agent whose first time block is t_first
+static View chunk_view(const d2d_net* n, float* p, int F, int t_first) {
+  return make_view(p, (long long)F * n->N * n->B, -t_first, n->N, F);
 }
 
 // the observations: agent g's features are rows in_off[g] ... of each time block; time block t is x_lead blocks in
@@ -123,16 +127,23 @@ static int reduce_scratch(d2d_net* n, long long count, double** out) {
   return D2D_OK;
 }
 
+// raises kernel K's dynamic shared-memory limit to `bytes` on its first call
+template <auto K>
+static int opt_in_smem(int bytes) {
+  static bool done = false;
+  if (!done) {
+    D2D_CUDA(cudaFuncSetAttribute(K, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes));
+    done = true;
+  }
+  return D2D_OK;
+}
+
 template <int RPT, int OPT>
 static int launch_dense_tile(const d2d_net* n, const DenseArgs& a, int max_in, cudaStream_t s) {
   constexpr int ROWS = 32 * RPT;
   const size_t smem = ((size_t)std::max(max_in, 1) * 8 * OPT + 8 * OPT + 2 * kDenseKC * ROWS) * sizeof(float);
-  static bool attr = false;
-  if (!attr) {
-    D2D_CUDA(cudaFuncSetAttribute(dense_tile_kernel<RPT, OPT>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                  200 * 1024));
-    attr = true;
-  }
+  int rc = opt_in_smem<dense_tile_kernel<RPT, OPT>>(200 * 1024);
+  if (rc) return rc;
   const int tiles = (a.t1 - a.t0) * ((n->B + ROWS - 1) / ROWS);
   if (tiles <= 0) return D2D_OK;
   // persistent grid: exactly the number of blocks that are resident at once (registers + shared memory)
@@ -145,7 +156,7 @@ static int launch_dense_tile(const d2d_net* n, const DenseArgs& a, int max_in, c
   return D2D_OK;
 }
 
-static int launch_dense(const d2d_net* n, DenseArgs& a, int max_in, cudaStream_t s, int x_exact = 0) {
+static int launch_dense(const d2d_net* n, DenseArgs a, int max_in, cudaStream_t s, int x_exact = 0) {
   a.B = n->B;
   // more than 192 outputs (3H of the hidden sizes above 64, e.g. the reference's iRDQN networks with H = 100): the
   // register-tiled kernel takes at most 192, so the output rows are split into equal slices that each go through it
@@ -192,11 +203,8 @@ static int launch_dense(const d2d_net* n, DenseArgs& a, int max_in, cudaStream_t
   // trips per tile serialise inside a slot and the register-tiled FP32 kernel is faster (measured 212 vs 480 us)
   if (tc_enabled() && n->B >= 256 && a.out_dim <= 192 && max_in <= tcd::kKc &&
       tcd::smem_bytes(max_in, a.out_dim) <= 225 * 1024) {
-    static bool attr = false;
-    if (!attr) {
-      D2D_CUDA(cudaFuncSetAttribute(dense_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 225 * 1024));
-      attr = true;
-    }
+    const int rc = opt_in_smem<dense_tc_kernel>(225 * 1024);
+    if (rc) return rc;
     const int pairs = (a.t1 - a.t0) * ((n->B + 255) / 256);
     if (pairs <= 0) return D2D_OK;
     const int gx = std::max(1, std::min(pairs, 148 / n->N));
@@ -220,18 +228,12 @@ static int launch_dense(const d2d_net* n, DenseArgs& a, int max_in, cudaStream_t
   const int gx = std::max(1, std::min(tiles, (148 * 4 + n->N - 1) / n->N));
   dim3 grid(gx, n->N);
   if (OC == 64) {
-    static bool attr64 = false;
-    if (!attr64) {
-      D2D_CUDA(cudaFuncSetAttribute(dense_kernel<64>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-      attr64 = true;
-    }
+    const int rc = opt_in_smem<dense_kernel<64>>(200 * 1024);
+    if (rc) return rc;
     dense_kernel<64><<<grid, kRowsPerBlock, smem, s>>>(a);
   } else {
-    static bool attr16 = false;
-    if (!attr16) {
-      D2D_CUDA(cudaFuncSetAttribute(dense_kernel<16>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-      attr16 = true;
-    }
+    const int rc = opt_in_smem<dense_kernel<16>>(200 * 1024);
+    if (rc) return rc;
     dense_kernel<16><<<grid, kRowsPerBlock, smem, s>>>(a);
   }
   D2D_LAUNCHED();
@@ -247,7 +249,12 @@ struct Wt {
   int out_dim;
 };
 
-static void fill_dense_w(const d2d_net* n, DenseArgs& a, const float* params, const Wt& w, int trans) {
+// the launch_dense arguments of y = epilogue(W x + b) over time blocks [t0, t1), W the matrix of `w` (trans: its
+// transpose, no bias); aux: the activations kEpiReluBwd takes relu' of
+static DenseArgs dense_args(const d2d_net* n, const float* params, const Wt& w, int trans, const View& x, const View& y,
+                            int epilogue, int t0, int t1, const View* aux = nullptr) {
+  DenseArgs a;
+  memset(&a, 0, sizeof(a));
   a.w = params, a.w_agent_stride = n->stride, a.trans = trans;
   for (int g = 0; g < n->N; ++g) {
     const int K = w.in_dim ? (*w.in_dim)[g] : w.in_const;
@@ -257,6 +264,9 @@ static void fill_dense_w(const d2d_net* n, DenseArgs& a, const float* params, co
     a.in_dim[g] = trans ? w.out_dim : K;
   }
   a.out_dim = trans ? (w.in_dim ? 0 : w.in_const) : w.out_dim;
+  a.x = x, a.y = y, a.epilogue = epilogue, a.t0 = t0, a.t1 = t1;
+  if (aux) a.aux = *aux;
+  return a;
 }
 
 template <int TO, int TK>
@@ -328,11 +338,8 @@ static int launch_wgrad(d2d_net* n, const View& dy, const View& x, const Wt& w, 
   if (tc_enabled() && n->B % 8 == 0) {
     // tensor-core path (wgrad_tc.cuh): bf16 x 3 planes on tcgen05, accumulators in TMEM
     const size_t smem = tcw::smem_bytes(maxK);
-    static bool attr = false;
-    if (!attr) {
-      D2D_CUDA(cudaFuncSetAttribute(wgrad_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024));
-      attr = true;
-    }
+    const int rc = opt_in_smem<wgrad_tc_kernel>(160 * 1024);
+    if (rc) return rc;
     strips = std::max(1, std::min(n->n_strips, 296 / n->N));   // two CTAs per SM
     wgrad_tc_kernel<<<dim3(strips, n->N), tcw::kThreads, smem, s>>>(a);
   } else {
@@ -353,11 +360,8 @@ static int launch_gru_step(const d2d_net* n, GruStepArgs& a, const float* params
   for (int g = 0; g < n->N; ++g) a.whh_off[g] = n->o_whh[g], a.bhh_off[g] = n->o_bhh[g];
   constexpr int ROWS = 128, OUT_PAD = 192;
   const size_t smem = ((size_t)std::max(a.first ? 0 : n->H, 1) * OUT_PAD + OUT_PAD + 2 * kDenseKC * ROWS) * sizeof(float);
-  static bool attr = false;
-  if (!attr) {
-    D2D_CUDA(cudaFuncSetAttribute(gru_step_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-    attr = true;
-  }
+  const int rc = opt_in_smem<gru_step_kernel>(200 * 1024);
+  if (rc) return rc;
   const int tiles = (a.t1 - a.t0) * ((n->B + ROWS - 1) / ROWS);
   if (tiles <= 0) return D2D_OK;
   int per_sm = 1;
@@ -403,12 +407,8 @@ template <int H, int STORE, int OMAX>
 static int launch_gru_tc_k(const d2d_net* n, const GruTcArgs& a, cudaStream_t s) {
   const size_t smem =
       OMAX > 0 ? ((tc::Smem<H>::bytes + 15) & ~(size_t)15) + tc::Smem<H>::head_bytes(OMAX) : tc::Smem<H>::bytes;
-  static bool attr = false;
-  if (!attr) {
-    D2D_CUDA(cudaFuncSetAttribute(gru_window_tc_kernel<H, STORE, OMAX>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                  (int)smem));
-    attr = true;
-  }
+  const int rc = opt_in_smem<gru_window_tc_kernel<H, STORE, OMAX>>((int)smem);
+  if (rc) return rc;
   const int pairs = (a.t1 - a.t0) * ((n->B + 2 * tc::kM - 1) / (2 * tc::kM));
   if (pairs <= 0) return D2D_OK;
   const int gx = std::max(1, std::min(pairs, 148 / n->N));   // one CTA per SM (all of its shared memory and TMEM)
@@ -473,9 +473,8 @@ static int launch_head_fused(const d2d_net* n, const float* params, const View& 
                              int t1, cudaStream_t s) {
   HeadFusedArgs a;
   memset(&a, 0, sizeof(a));
-  const long long NB = (long long)n->N * n->B;
   a.h = h, a.out = out, a.w = params, a.w_agent_stride = n->stride, a.O = n->O, a.B = n->B, a.t0 = t0, a.t1 = t1;
-  if (y1) a.y1 = make_view(y1, n->H * NB, -t0, n->N, n->H, n->B);
+  if (y1) a.y1 = chunk_view(n, y1, n->H, t0);
   for (int g = 0; g < n->N; ++g)
     a.w1_off[g] = n->o_w1[g], a.b1_off[g] = n->o_b1[g], a.w2_off[g] = n->o_w2[g], a.b2_off[g] = n->o_b2[g];
   const int tiles = (t1 - t0) * ((n->B + 2 * kHeadThreads - 1) / (2 * kHeadThreads));
@@ -488,41 +487,17 @@ static int launch_head_fused(const d2d_net* n, const float* params, const View& 
   return D2D_OK;
 }
 
-template <int H>
-static int launch_gru_bptt_tc_h(const d2d_net* n, const GruBpttArgs& a, cudaStream_t s, int* strips) {
-  static bool attr = false;
-  if (!attr) {
-    D2D_CUDA(cudaFuncSetAttribute(gru_bptt_tc_kernel<H>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                  (int)tcr::Smem<H>::bytes));
-    D2D_CUDA(cudaFuncSetAttribute(gru_bptt_tc_kernel<H | kDgiSlices>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                  (int)tcr::Smem<H>::bytes));
-    attr = true;
-  }
+// one launch of a tcgen05 BPTT window kernel (gru_bptt_tc.cuh, gru_bwd_tc.cuh): K, or KS, its kDgiSlices
+// instantiation, when a.slice_step is set; *strips receives the CTAs per agent, each of which left one dW_hh partial sum
+template <auto K, auto KS, class Args>
+static int launch_bptt_window(const d2d_net* n, const Args& a, int threads, size_t smem, cudaStream_t s, int* strips) {
+  int rc;
+  if ((rc = opt_in_smem<K>((int)smem)) || (rc = opt_in_smem<KS>((int)smem))) return rc;
   const int tiles = (a.t1 - a.t0) * ((n->B + tc::kM - 1) / tc::kM);
   if (tiles <= 0) return D2D_OK;
   const int gx = std::max(1, std::min(std::min(tiles, 148 / n->N), n->n_strips));
-  if (a.slice_step) gru_bptt_tc_kernel<H | kDgiSlices><<<dim3(gx, n->N), tcr::kThreads, tcr::Smem<H>::bytes, s>>>(a);
-  else gru_bptt_tc_kernel<H><<<dim3(gx, n->N), tcr::kThreads, tcr::Smem<H>::bytes, s>>>(a);
-  D2D_LAUNCHED();
-  *strips = gx;
-  return D2D_OK;
-}
-
-template <int H>
-static int launch_gru_bwd_tc_h(const d2d_net* n, const GruBwdTcArgs& a, cudaStream_t s, int* strips) {
-  static bool attr = false;
-  if (!attr) {
-    D2D_CUDA(cudaFuncSetAttribute(gru_bwd_tc_kernel<H>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                  (int)tcb::Smem<H>::bytes));
-    D2D_CUDA(cudaFuncSetAttribute(gru_bwd_tc_kernel<H | kDgiSlices>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                  (int)tcb::Smem<H>::bytes));
-    attr = true;
-  }
-  const int tiles = (a.t1 - a.t0) * ((n->B + tc::kM - 1) / tc::kM);
-  if (tiles <= 0) return D2D_OK;
-  const int gx = std::max(1, std::min(std::min(tiles, 148 / n->N), n->n_strips));
-  if (a.slice_step) gru_bwd_tc_kernel<H | kDgiSlices><<<dim3(gx, n->N), tcb::kThreads, tcb::Smem<H>::bytes, s>>>(a);
-  else gru_bwd_tc_kernel<H><<<dim3(gx, n->N), tcb::kThreads, tcb::Smem<H>::bytes, s>>>(a);
+  if (a.slice_step) KS<<<dim3(gx, n->N), threads, smem, s>>>(a);
+  else K<<<dim3(gx, n->N), threads, smem, s>>>(a);
   D2D_LAUNCHED();
   *strips = gx;
   return D2D_OK;
@@ -622,33 +597,20 @@ static float* hs_ptr(const d2d_net* n, const Chunk& c, bool train, int s) {
 static int head_dense(const d2d_net* n, const float* params, const View& last, const View& y1, float* y2p,
                       const View& lg, int t0, int t1, cudaStream_t s) {
   const int H = n->H, O = n->O;
-  const long long NB = (long long)n->N * n->B;
   Wt w1{&n->o_w1, &n->o_b1, nullptr, H, H};
   Wt w2{&n->o_w2, &n->o_b2, nullptr, H, O};
   if (n->arch == D2D_NET_MLP) w1.in_dim = &n->in_dim;
   int rc;
-  {
-    DenseArgs a;
-    memset(&a, 0, sizeof(a));
-    fill_dense_w(n, a, params, w1, 0);
-    a.x = last, a.y = y1, a.epilogue = kEpiRelu, a.t0 = t0, a.t1 = t1;
-    if ((rc = launch_dense(n, a, n->arch == D2D_NET_MLP ? n->max_in : H, s))) return rc;
-  }
+  if ((rc = launch_dense(n, dense_args(n, params, w1, 0, last, y1, kEpiRelu, t0, t1),
+                         n->arch == D2D_NET_MLP ? n->max_in : H, s)))
+    return rc;
   View top = y1;
   if (n->head2) {
     Wt w1b{&n->o_w1b, &n->o_b1b, nullptr, H, H};
-    top = make_view(y2p, H * NB, -t0, n->N, H, n->B);
-    DenseArgs a;
-    memset(&a, 0, sizeof(a));
-    fill_dense_w(n, a, params, w1b, 0);
-    a.x = y1, a.y = top, a.epilogue = kEpiRelu, a.t0 = t0, a.t1 = t1;
-    if ((rc = launch_dense(n, a, H, s))) return rc;
+    top = chunk_view(n, y2p, H, t0);
+    if ((rc = launch_dense(n, dense_args(n, params, w1b, 0, y1, top, kEpiRelu, t0, t1), H, s))) return rc;
   }
-  DenseArgs a;
-  memset(&a, 0, sizeof(a));
-  fill_dense_w(n, a, params, w2, 0);
-  a.x = top, a.y = lg, a.epilogue = kEpiNone, a.t0 = t0, a.t1 = t1;
-  return launch_dense(n, a, H, s);
+  return launch_dense(n, dense_args(n, params, w2, 0, top, lg, kEpiNone, t0, t1), H, s);
 }
 
 // forward of chunk [c0, c1) (c1 - c0 <= Tc): fills c.logits (local time index t - c0)
@@ -657,64 +619,57 @@ static int forward_chunk(d2d_net* n, const float* params, const float* x, int x_
   const int N = n->N, B = n->B, H = n->H, O = n->O;
   const long long NB = (long long)N * B;
   const View xin = input_view(n, x, x_lead);
-  const View y1 = make_view(c.y1, H * NB, -c0, N, H, B);
-  const View lg = make_view(c.logits, O * NB, -c0, N, O, B);
+  const View y1 = chunk_view(n, c.y1, H, c0);
+  const View lg = chunk_view(n, c.logits, O, c0);
   int rc;
   View last = xin;
   if (n->arch == D2D_NET_GRU) {
     const int L = n->L, halo = c.halo;
     if (c.plan.window_tc) {   // tcgen05 fused window (gru_tc.cuh); training windows are padded and keep every step's h
       const bool head = c.plan.head == Head::kWindow;   // window + head (+ y1 when training) in one launch
-      const View hl = make_view(hs_ptr(n, c, train, L - 1), H * NB, -c0, N, H, B);
-      const View hv = make_view(c.hs, H * NB, -c0, N, H, B);
-      const View av = make_view(c.acts, 4 * H * NB, -c0, N, 4 * H, B);   // c.acts null: the BPTT recomputes the gates
+      const View hl = chunk_view(n, hs_ptr(n, c, train, L - 1), H, c0);
+      const View hv = chunk_view(n, c.hs, H, c0);
+      const View av = chunk_view(n, c.acts, 4 * H, c0);   // c.acts null: the BPTT recomputes the gates
       rc = launch_gru_tc(n, params, xin, hl, c0, c1, padded, s, train ? &hv : nullptr, train ? &av : nullptr,
                          (long long)c.Tc * H * NB, head ? &lg : nullptr, head && train ? &y1 : nullptr, nullptr);
       if (rc || head) return rc;
     } else {
       // input projections of every observation the chunk's windows touch: times [c0 - halo, c1)
-      const View gi = make_view(c.gi, 3 * H * NB, -(c0 - halo), N, 3 * H, B);
-      {
-        DenseArgs a;
-        memset(&a, 0, sizeof(a));
-        Wt wih{&n->o_wih, &n->o_bih, &n->in_dim, 0, 3 * H};
-        fill_dense_w(n, a, params, wih, 0);
-        a.x = xin, a.y = gi, a.epilogue = kEpiNone, a.t0 = c0 - halo, a.t1 = c1;
-        if ((rc = launch_dense(n, a, n->max_in, s, n->x_exact))) return rc;
-      }
-      const View gh = make_view(c.gh, 3 * H * NB, -c0, N, 3 * H, B);
+      const View gi = chunk_view(n, c.gi, 3 * H, c0 - halo);
+      Wt wih{&n->o_wih, &n->o_bih, &n->in_dim, 0, 3 * H};
+      if ((rc = launch_dense(n, dense_args(n, params, wih, 0, xin, gi, kEpiNone, c0 - halo, c1), n->max_in, s,
+                             n->x_exact)))
+        return rc;
+      const View gh = chunk_view(n, c.gh, 3 * H, c0);
+      Wt whh{&n->o_whh, &n->o_bhh, nullptr, H, 3 * H};
       for (int st = 0; st < L; ++st) {
-        const View hprev = make_view(hs_ptr(n, c, train, st - 1 < 0 ? 0 : st - 1), H * NB, -c0, N, H, B);
-        const View hout = make_view(hs_ptr(n, c, train, st), H * NB, -c0, N, H, B);
+        const View hprev = chunk_view(n, hs_ptr(n, c, train, st - 1 < 0 ? 0 : st - 1), H, c0);
+        const View hout = chunk_view(n, hs_ptr(n, c, train, st), H, c0);
+        const View acts = train ? chunk_view(n, c.acts + (long long)st * c.Tc * 4 * H * NB, 4 * H, c0) : View{};
         if (B % 4 == 0 && H <= 128) {   // fused hidden projection + gates (a register tile covers 64 units; H > 64: 2 launches)
           GruStepArgs fa;
           memset(&fa, 0, sizeof(fa));
           fa.h_prev = hprev, fa.h_out = hout, fa.gi = gi, fa.gi.t_off = gi.t_off - (L - 1 - st);
-          if (train) fa.acts = make_view(c.acts + (long long)st * c.Tc * 4 * H * NB, 4 * H * NB, -c0, N, 4 * H, B);
+          fa.acts = acts;
           fa.t0 = c0, fa.t1 = c1, fa.back = L - 1 - st, fa.padded = padded, fa.first = st == 0, fa.store = train;
           if ((rc = launch_gru_step(n, fa, params, s))) return rc;
           continue;
         }
-        {
-          DenseArgs a;
-          memset(&a, 0, sizeof(a));
-          Wt whh{&n->o_whh, &n->o_bhh, nullptr, st == 0 ? 0 : H, 3 * H};   // step 0: h = 0, gh = b_hh
-          fill_dense_w(n, a, params, whh, 0);
-          for (int g = 0; g < N; ++g) a.w_ld[g] = H;
-          a.x = hprev, a.y = gh, a.epilogue = kEpiNone, a.t0 = c0, a.t1 = c1;
-          if ((rc = launch_dense(n, a, H, s))) return rc;
-        }
+        DenseArgs a = dense_args(n, params, whh, 0, hprev, gh, kEpiNone, c0, c1);
+        if (st == 0)   // h = 0: no inputs, gh = b_hh (the rows of W_hh stay H floats apart)
+          for (int g = 0; g < N; ++g) a.in_dim[g] = 0;
+        if ((rc = launch_dense(n, a, H, s))) return rc;
         GateArgs ga;
         memset(&ga, 0, sizeof(ga));
         ga.gi = gi, ga.gi.t_off = gi.t_off - (L - 1 - st);
         ga.gh = gh, ga.h_prev = hprev, ga.h_out = hout;
-        if (train) ga.acts = make_view(c.acts + (long long)st * c.Tc * 4 * H * NB, 4 * H * NB, -c0, N, 4 * H, B);
+        ga.acts = acts;
         ga.H = H, ga.B = B, ga.t0 = c0, ga.t1 = c1, ga.back = L - 1 - st, ga.padded = padded, ga.first = st == 0;
         ga.store = train, ga.t_episode0 = 0;
         if ((rc = launch_gate(ga, N, false, s))) return rc;
       }
     }
-    last = make_view(hs_ptr(n, c, train, L - 1), H * NB, -c0, N, H, B);
+    last = chunk_view(n, hs_ptr(n, c, train, L - 1), H, c0);
   }
   if (c.plan.head == Head::kKernel) return launch_head_fused(n, params, last, train ? c.y1 : nullptr, lg, c0, c1, s);
   return head_dense(n, params, last, y1, c.y2, lg, c0, c1, s);
@@ -722,70 +677,48 @@ static int forward_chunk(d2d_net* n, const float* params, const float* x, int x_
 
 // backward of chunk [c0, c1) given c.dl = d(loss)/d(pre-activation outputs); accumulates into grads
 static int backward_chunk(d2d_net* n, const float* params, const float* x, int x_lead, int c0, int c1,
-                          const Chunk& c, float* grads, float inv_rows, cudaStream_t s) {
+                          const Chunk& c, float* grads, cudaStream_t s) {
   const int N = n->N, B = n->B, H = n->H, O = n->O;
   const long long NB = (long long)N * B;
   const View xin = input_view(n, x, x_lead);
-  const View y1 = make_view(c.y1, H * NB, -c0, N, H, B);
-  const View dl = make_view(c.dl, O * NB, -c0, N, O, B);
-  const View dy1 = make_view(c.dy1, H * NB, -c0, N, H, B);
+  const View y1 = chunk_view(n, c.y1, H, c0);
+  const View dl = chunk_view(n, c.dl, O, c0);
+  const View dy1 = chunk_view(n, c.dy1, H, c0);
   Wt w1{&n->o_w1, &n->o_b1, nullptr, H, H};
   Wt w2{&n->o_w2, &n->o_b2, nullptr, H, O};
   int rc;
   if (n->head2) {
     // Q-network head: dW2 = dl^T y2 ; dy2 = (dl W2) * relu'(y2) ; dW1b = dy2^T y1 ; dy1 = (dy2 W1b) * relu'(y1)
-    const View y2 = make_view(c.y2, H * NB, -c0, N, H, B);
-    const View dy2 = make_view(c.dy2, H * NB, -c0, N, H, B);
+    const View y2 = chunk_view(n, c.y2, H, c0);
+    const View dy2 = chunk_view(n, c.dy2, H, c0);
     Wt w1b{&n->o_w1b, &n->o_b1b, nullptr, H, H};
     if ((rc = launch_wgrad(n, dl, y2, w2, false, grads, c0, c1, s))) return rc;
-    {
-      DenseArgs a;
-      memset(&a, 0, sizeof(a));
-      fill_dense_w(n, a, params, w2, 1);
-      a.out_dim = H;
-      a.x = dl, a.y = dy2, a.aux = y2, a.epilogue = kEpiReluBwd, a.t0 = c0, a.t1 = c1;
-      if ((rc = launch_dense(n, a, O, s))) return rc;
-    }
+    if ((rc = launch_dense(n, dense_args(n, params, w2, 1, dl, dy2, kEpiReluBwd, c0, c1, &y2), O, s))) return rc;
     if ((rc = launch_wgrad(n, dy2, y1, w1b, false, grads, c0, c1, s))) return rc;
-    DenseArgs a;
-    memset(&a, 0, sizeof(a));
-    fill_dense_w(n, a, params, w1b, 1);
-    a.out_dim = H;
-    a.x = dy2, a.y = dy1, a.aux = y1, a.epilogue = kEpiReluBwd, a.t0 = c0, a.t1 = c1;
-    if ((rc = launch_dense(n, a, H, s))) return rc;
+    if ((rc = launch_dense(n, dense_args(n, params, w1b, 1, dy2, dy1, kEpiReluBwd, c0, c1, &y1), H, s))) return rc;
   } else {
     // head: dW2 = dl^T y1 ; dy1 = (dl W2) * relu'(y1)
     if ((rc = launch_wgrad(n, dl, y1, w2, false, grads, c0, c1, s))) return rc;
-    DenseArgs a;
-    memset(&a, 0, sizeof(a));
-    fill_dense_w(n, a, params, w2, 1);
-    a.out_dim = H;
-    a.x = dl, a.y = dy1, a.aux = y1, a.epilogue = kEpiReluBwd, a.t0 = c0, a.t1 = c1;
-    if ((rc = launch_dense(n, a, O, s))) return rc;
+    if ((rc = launch_dense(n, dense_args(n, params, w2, 1, dl, dy1, kEpiReluBwd, c0, c1, &y1), O, s))) return rc;
   }
   if (n->arch == D2D_NET_MLP) {
     w1.in_dim = &n->in_dim;
     return launch_wgrad(n, dy1, xin, w1, false, grads, c0, c1, s, true);
   }
   const int L = n->L, halo = c.halo;
-  const View hlast = make_view(hs_ptr(n, c, true, L - 1), H * NB, -c0, N, H, B);
+  const View hlast = chunk_view(n, hs_ptr(n, c, true, L - 1), H, c0);
   if ((rc = launch_wgrad(n, dy1, hlast, w1, false, grads, c0, c1, s))) return rc;
   float* dh_cur = c.dh0;
   float* dh_nxt = c.dh1;
-  {
-    DenseArgs a;   // d(h_last) = dy1 W1
-    memset(&a, 0, sizeof(a));
-    fill_dense_w(n, a, params, w1, 1);
-    a.out_dim = H;
-    a.x = dy1, a.y = make_view(dh_cur, H * NB, -c0, N, H, B), a.epilogue = kEpiNone, a.t0 = c0, a.t1 = c1;
-    if ((rc = launch_dense(n, a, H, s))) return rc;
-  }
+  // d(h_last) = dy1 W1
+  if ((rc = launch_dense(n, dense_args(n, params, w1, 1, dy1, chunk_view(n, dh_cur, H, c0), kEpiNone, c0, c1), H, s)))
+    return rc;
   // d(gi) slices: every element dgi_slice_sum_kernel reads is stored once, and it writes all of c.dgi
   if (!c.plan.dgi_slices) D2D_CUDA(cudaMemsetAsync(c.dgi, 0, (size_t)(c.Tc + halo) * 3 * H * NB * 4, s));
-  const View dgi = make_view(c.dgi, 3 * H * NB, -(c0 - halo), N, 3 * H, B);
-  const View dgi_s = c.plan.dgi_slices ? make_view(c.dgi_s, 3 * H * NB, -c0, N, 3 * H, B) : dgi;   // slice 0
+  const View dgi = chunk_view(n, c.dgi, 3 * H, c0 - halo);
+  const View dgi_s = c.plan.dgi_slices ? chunk_view(n, c.dgi_s, 3 * H, c0) : dgi;   // slice 0
   const long long slice_step = c.plan.dgi_slices ? (long long)c.Tc * 3 * H * NB : 0;
-  const View dgh = make_view(c.gh, 3 * H * NB, -c0, N, 3 * H, B);
+  const View dgh = chunk_view(n, c.gh, 3 * H, c0);
   Wt whh{&n->o_whh, &n->o_bhh, nullptr, H, 3 * H};
   if (c.plan.bptt != Bptt::kFp32) {
     // one kernel walks the whole window backwards (d(h) in registers, d(gh) W_hh on tcgen05) and accumulates d(gi) per
@@ -796,8 +729,8 @@ static int backward_chunk(d2d_net* n, const float* params, const float* x, int x
       GruBpttArgs ba;
       memset(&ba, 0, sizeof(ba));
       ba.x = xin;
-      ba.hs = make_view(c.hs, H * NB, -c0, N, H, B);
-      ba.dh = make_view(dh_cur, H * NB, -c0, N, H, B);
+      ba.hs = chunk_view(n, c.hs, H, c0);
+      ba.dh = chunk_view(n, dh_cur, H, c0);
       ba.dgi = dgi_s;
       ba.w = params, ba.w_agent_stride = n->stride;
       for (int g = 0; g < N; ++g) {
@@ -815,19 +748,21 @@ static int backward_chunk(d2d_net* n, const float* params, const float* x, int x
         D2D_LAUNCHED();
         ba.dh_absmax = reinterpret_cast<const float*>(amax);
       }
-      (void)inv_rows;
       ba.L = L, ba.B = B, ba.t0 = c0, ba.t1 = c1;
       ba.partial = n->partial, ba.part_stride = n->part_stride;
       ba.slice_step = slice_step;
-      rc = n->H == 32 ? launch_gru_bptt_tc_h<32>(n, ba, s, &strips) : launch_gru_bptt_tc_h<64>(n, ba, s, &strips);
+      rc = H == 32 ? launch_bptt_window<gru_bptt_tc_kernel<32>, gru_bptt_tc_kernel<32 | kDgiSlices>>(
+                         n, ba, tcr::kThreads, tcr::Smem<32>::bytes, s, &strips)
+                   : launch_bptt_window<gru_bptt_tc_kernel<64>, gru_bptt_tc_kernel<64 | kDgiSlices>>(
+                         n, ba, tcr::kThreads, tcr::Smem<64>::bytes, s, &strips);
     } else {
       // gru_bwd_tc reads the gates the forward stored; it leaves d(gh) of step s in the first 3H features of that
       // step's activation block
       GruBwdTcArgs ba;
       memset(&ba, 0, sizeof(ba));
-      ba.acts = make_view(c.acts, 4 * H * NB, -c0, N, 4 * H, B);
-      ba.hs = make_view(c.hs, H * NB, -c0, N, H, B);
-      ba.dh = make_view(dh_cur, H * NB, -c0, N, H, B);
+      ba.acts = chunk_view(n, c.acts, 4 * H, c0);
+      ba.hs = chunk_view(n, c.hs, H, c0);
+      ba.dh = chunk_view(n, dh_cur, H, c0);
       ba.dgi = dgi_s;
       ba.w = params, ba.w_agent_stride = n->stride;
       for (int g = 0; g < N; ++g) ba.whh_off[g] = n->o_whh[g];
@@ -835,7 +770,10 @@ static int backward_chunk(d2d_net* n, const float* params, const float* x, int x
       ba.L = L, ba.B = B, ba.t0 = c0, ba.t1 = c1;
       ba.partial = n->partial, ba.part_stride = n->part_stride;
       ba.slice_step = slice_step;
-      rc = n->H == 32 ? launch_gru_bwd_tc_h<32>(n, ba, s, &strips) : launch_gru_bwd_tc_h<64>(n, ba, s, &strips);
+      rc = H == 32 ? launch_bptt_window<gru_bwd_tc_kernel<32>, gru_bwd_tc_kernel<32 | kDgiSlices>>(
+                         n, ba, tcb::kThreads, tcb::Smem<32>::bytes, s, &strips)
+                   : launch_bptt_window<gru_bwd_tc_kernel<64>, gru_bwd_tc_kernel<64 | kDgiSlices>>(
+                         n, ba, tcb::kThreads, tcb::Smem<64>::bytes, s, &strips);
     }
     if (rc) return rc;
     if (c.plan.dgi_slices) {
@@ -848,26 +786,22 @@ static int backward_chunk(d2d_net* n, const float* params, const float* x, int x
     if (strips > 0 && (rc = launch_wreduce(n, whh, false, strips, grads, s))) return rc;
   }
   for (int st = L - 1; st >= 0 && c.plan.bptt == Bptt::kFp32; --st) {
-    const View hprev = make_view(hs_ptr(n, c, true, st - 1 < 0 ? 0 : st - 1), H * NB, -c0, N, H, B);
+    const View hprev = chunk_view(n, hs_ptr(n, c, true, st - 1 < 0 ? 0 : st - 1), H, c0);
+    const View dh_prev = chunk_view(n, dh_nxt, H, c0);
     GateArgs ga;
     memset(&ga, 0, sizeof(ga));
     ga.gh = dgh, ga.h_prev = hprev;
-    ga.h_out = make_view(dh_nxt, H * NB, -c0, N, H, B);
-    ga.dh = make_view(dh_cur, H * NB, -c0, N, H, B);
-    ga.acts = make_view(c.acts + (long long)st * c.Tc * 4 * H * NB, 4 * H * NB, -c0, N, 4 * H, B);
+    ga.h_out = dh_prev;
+    ga.dh = chunk_view(n, dh_cur, H, c0);
+    ga.acts = chunk_view(n, c.acts + (long long)st * c.Tc * 4 * H * NB, 4 * H, c0);
     ga.dgi = dgi, ga.dgi.t_off = dgi.t_off - (L - 1 - st);
     ga.H = H, ga.B = B, ga.t0 = c0, ga.t1 = c1, ga.back = L - 1 - st, ga.padded = 1, ga.first = st == 0;
     if ((rc = launch_gate(ga, N, true, s))) return rc;
     // dW_hh += d(gh)^T h_{s-1}, db_hh += sum d(gh)   (h_{-1} = 0: bias only)
     if ((rc = launch_wgrad(n, dgh, hprev, whh, st == 0, grads, c0, c1, s))) return rc;
-    if (st > 0) {
-      DenseArgs a;   // d(h_{s-1}) += d(gh) W_hh
-      memset(&a, 0, sizeof(a));
-      fill_dense_w(n, a, params, whh, 1);
-      a.out_dim = H;
-      a.x = dgh, a.y = make_view(dh_nxt, H * NB, -c0, N, H, B), a.epilogue = kEpiAccum, a.t0 = c0, a.t1 = c1;
-      if ((rc = launch_dense(n, a, 3 * H, s))) return rc;
-    }
+    // d(h_{s-1}) += d(gh) W_hh
+    if (st > 0 && (rc = launch_dense(n, dense_args(n, params, whh, 1, dgh, dh_prev, kEpiAccum, c0, c1), 3 * H, s)))
+      return rc;
     std::swap(dh_cur, dh_nxt);
   }
   // dW_ih = d(gi)^T x over every observation the chunk touched (zero observations before t = 0 feed b_ih only)
@@ -1034,44 +968,38 @@ extern "C" int d2d_net_rollout_step(d2d_net* n, const float* params, const float
   int rc = check_range(n, x_lead, t, t + 1, "d2d_net_rollout_step");
   if (rc) return rc;
   cudaStream_t s = as_stream(stream);
-  const int N = n->N, B = n->B, H = n->H, O = n->O, L = n->L;
-  const long long NB = (long long)N * B;
+  const int H = n->H, O = n->O, L = n->L;
   Chunk c;
   if ((rc = plan_chunk(n, false, 1, c))) return rc;
   const View xin = input_view(n, x, x_lead);
-  const View hl = make_view(hs_ptr(n, c, false, L - 1), H * NB, -t, N, H, B);
-  const View lg = make_view(out, O * NB, -t, N, O, B);
+  const View hl = chunk_view(n, hs_ptr(n, c, false, L - 1), H, t);
+  const View lg = chunk_view(n, out, O, t);
   if (c.plan.window_tc) {   // the tensor-core window kernel re-reads the L observations (L x I floats per row): no ring
     const bool head = c.plan.head == Head::kWindow;   // window + head in ONE launch, outputs written in place
     rc = launch_gru_tc(n, params, xin, hl, t, t + 1, 0, s, nullptr, nullptr, 0, head ? &lg : nullptr, nullptr, nullptr);
     if (rc || head) return rc;
   } else {
-    if (!n->gi_ring) D2D_CUDA(cudaMalloc((void**)&n->gi_ring, (size_t)L * 3 * H * NB * 4));
-    {   // input projection of the NEW observation only; the previous L - 1 are still in the ring
-      DenseArgs a;
-      memset(&a, 0, sizeof(a));
-      Wt wih{&n->o_wih, &n->o_bih, &n->in_dim, 0, 3 * H};
-      fill_dense_w(n, a, params, wih, 0);
-      a.x = xin, a.y = make_view(n->gi_ring, 3 * H * NB, (t % L) - t, N, 3 * H, B), a.epilogue = kEpiNone;
-      a.t0 = t, a.t1 = t + 1;
-      if ((rc = launch_dense(n, a, n->max_in, s))) return rc;
-    }
+    if (!n->gi_ring) D2D_CUDA(cudaMalloc((void**)&n->gi_ring, (size_t)L * 3 * H * n->N * n->B * 4));
+    // input projection of the NEW observation only, into ring slot t % L; the previous L - 1 are still in the ring
+    Wt wih{&n->o_wih, &n->o_bih, &n->in_dim, 0, 3 * H};
+    const View slot = chunk_view(n, n->gi_ring, 3 * H, t - t % L);
+    if ((rc = launch_dense(n, dense_args(n, params, wih, 0, xin, slot, kEpiNone, t, t + 1), n->max_in, s))) return rc;
     for (int st = 0; st < L; ++st) {
       const int back = L - 1 - st;
       if (t - back < 0 && st < L - 1) continue;   // the step does not exist and h stays zero: nothing to do
       GruStepArgs fa;
       memset(&fa, 0, sizeof(fa));
       const bool first = (t - back <= 0) || st == 0;   // first EXISTING step starts from h = 0
-      fa.h_prev = make_view(hs_ptr(n, c, false, st - 1 < 0 ? 0 : st - 1), H * NB, -t, N, H, B);
-      fa.h_out = make_view(hs_ptr(n, c, false, st), H * NB, -t, N, H, B);
-      fa.gi = make_view(n->gi_ring, 3 * H * NB, -back, N, 3 * H, B);
+      fa.h_prev = chunk_view(n, hs_ptr(n, c, false, st - 1 < 0 ? 0 : st - 1), H, t);
+      fa.h_out = chunk_view(n, hs_ptr(n, c, false, st), H, t);
+      fa.gi = chunk_view(n, n->gi_ring, 3 * H, back);
       fa.t_mod_gi = L;
       fa.t0 = t, fa.t1 = t + 1, fa.back = back, fa.padded = 0, fa.first = first, fa.store = 0;
       if ((rc = launch_gru_step(n, fa, params, s))) return rc;
     }
   }
   if (c.plan.head == Head::kKernel) return launch_head_fused(n, params, hl, nullptr, lg, t, t + 1, s);
-  return head_dense(n, params, hl, make_view(c.y1, H * NB, -t, N, H, B), c.y2, lg, t, t + 1, s);
+  return head_dense(n, params, hl, chunk_view(n, c.y1, H, t), c.y2, lg, t, t + 1, s);
 }
 
 static void fill_head(HeadArgs& h, int N, int B, int O, int out_kind, int dist_kind) {
@@ -1091,8 +1019,8 @@ extern "C" int d2d_policy_head(int N, int B, int O, int n_t, int out_kind, int d
               "d2d_policy_head: bad mode");
   HeadArgs h;
   fill_head(h, N, B, O, out_kind, dist_kind);
-  h.logits = make_view(const_cast<float*>(logits), (long long)N * O * B, 0, N, O, B);
-  if (probs) h.probs = make_view(probs, (long long)N * O * B, 0, N, O, B);
+  h.logits = make_view(const_cast<float*>(logits), (long long)N * O * B, 0, N, O);
+  if (probs) h.probs = make_view(probs, (long long)N * O * B, 0, N, O);
   h.t0 = 0, h.t1 = n_t, h.act_mode = act_mode, h.actions = actions, h.logp = logp, h.entropy = entropy;
   h.key = philox_key(seed), h.env_offset = (uint32_t)env_offset;
   h.t_abs_off = t_abs0;
@@ -1113,8 +1041,7 @@ extern "C" int d2d_net_rollout_act(d2d_net* n, const float* params, const float*
   int rc = check_range(n, x_lead, t, t + 1, "d2d_net_rollout_act");
   if (rc) return rc;
   cudaStream_t s = as_stream(stream);
-  const int N = n->N, B = n->B, H = n->H, O = n->O;
-  const long long NB = (long long)N * B;
+  const int N = n->N, B = n->B, O = n->O;
   Chunk c;
   if ((rc = plan_chunk(n, false, 1, c))) return rc;
   if (c.plan.head == Head::kWindow && O > 1 && n->B % 4 == 0) {
@@ -1123,8 +1050,8 @@ extern "C" int d2d_net_rollout_act(d2d_net* n, const float* params, const float*
     h.act_mode = act_mode, h.actions = actions, h.logp = logp, h.act_t_off = -t;
     h.key = philox_key(seed), h.env_offset = (uint32_t)env_offset;
     h.t_abs_off = t_abs0 - t;
-    const View hl = make_view(hs_ptr(n, c, false, n->L - 1), H * NB, -t, N, H, B);
-    const View lgo = make_view(logits_out, O * NB, -t, N, O, B);   // p == nullptr: outputs are not written
+    const View hl = chunk_view(n, hs_ptr(n, c, false, n->L - 1), n->H, t);
+    const View lgo = chunk_view(n, logits_out, O, t);   // p == nullptr: outputs are not written
     const DistArgs sel = h;
     return launch_gru_tc(n, params, input_view(n, x, x_lead), hl, t, t + 1, 0, s, nullptr, nullptr, 0, &lgo, nullptr,
                          &sel);
@@ -1136,6 +1063,44 @@ extern "C" int d2d_net_rollout_act(d2d_net* n, const float* params, const float*
                          env_offset, t_abs0, stream);
 }
 
+// forward, loss and backward of time blocks [t0, t1) in chunks of the scratch budget; loss(c0, c1, c) launches the
+// loss of chunk [c0, c1), which fills c.dl
+template <class Loss>
+static int train_chunks(d2d_net* n, const float* params, const float* x, int x_lead, int t0, int t1, float* grads,
+                        cudaStream_t s, const char* who, Loss loss) {
+  int rc = check_range(n, x_lead, t0, t1, who);
+  if (rc) return rc;
+  Chunk c;
+  if ((rc = plan_chunk(n, true, t1 - t0, c))) return rc;
+  for (int c0 = t0; c0 < t1; c0 += c.Tc) {
+    const int c1 = std::min(t1, c0 + c.Tc);
+    if ((rc = forward_chunk(n, params, x, x_lead, c0, c1, 1, true, c, s))) return rc;
+    if ((rc = loss(c0, c1, c))) return rc;
+    if ((rc = backward_chunk(n, params, x, x_lead, c0, c1, c, grads, s))) return rc;
+  }
+  return D2D_OK;
+}
+
+// a loss kernel of 128-thread blocks: with plan.det its per-warp partial sums (n_vals per agent and warp, zeroed first
+// if zero_part), then their fixed-order reduction into sums; else the kernel that adds them atomically
+template <class Args>
+static int launch_loss(d2d_net* n, const Chunk& c, void (*atomic_k)(Args), void (*part_k)(Args, double*),
+                       const Args& a, dim3 grid, int n_vals, bool zero_part, double* sums, cudaStream_t s) {
+  if (!c.plan.det) {
+    atomic_k<<<grid, 128, 0, s>>>(a);
+    D2D_LAUNCHED();
+    return D2D_OK;
+  }
+  const long long count = (long long)n_vals * n->N * grid.x * 4;
+  double* part;
+  int rc = reduce_scratch(n, count, &part);
+  if (rc) return rc;
+  if (zero_part) D2D_CUDA(cudaMemsetAsync(part, 0, sizeof(double) * count, s));
+  part_k<<<grid, 128, 0, s>>>(a, part);
+  D2D_LAUNCHED();
+  return launch_sum_partials(part, n->N, grid.x * 4, n_vals, sums, s);
+}
+
 extern "C" int d2d_ppo_policy_grad(d2d_net* n, const float* params, const float* x, int x_lead, int t0, int t1,
                                    int dist_kind, const void* actions, const float* logp_old, const float* weight,
                                    int weight_per_agent, const int32_t* cycle, float inv_rows, float cliprange,
@@ -1143,38 +1108,20 @@ extern "C" int d2d_ppo_policy_grad(d2d_net* n, const float* params, const float*
   D2D_REQUIRE(n && params && x && actions && logp_old && weight && grads && loss_sums,
               "d2d_ppo_policy_grad: null argument");
   D2D_REQUIRE(n->out_kind != D2D_OUT_IDENTITY, "d2d_ppo_policy_grad: net has no probability output");
-  int rc = check_range(n, x_lead, t0, t1, "d2d_ppo_policy_grad");
-  if (rc) return rc;
   cudaStream_t s = as_stream(stream);
-  Chunk c;
-  if ((rc = plan_chunk(n, true, t1 - t0, c))) return rc;
-  const long long NB = (long long)n->N * n->B;
-  for (int c0 = t0; c0 < t1; c0 += c.Tc) {
-    const int c1 = std::min(t1, c0 + c.Tc);
-    if ((rc = forward_chunk(n, params, x, x_lead, c0, c1, 1, true, c, s))) return rc;
+  auto loss = [&](int c0, int c1, const Chunk& c) {
     HeadArgs h;
     fill_head(h, n->N, n->B, n->O, n->out_kind, dist_kind);
-    h.logits = make_view(c.logits, n->O * NB, -c0, n->N, n->O, n->B);
-    h.dlogits = make_view(c.dl, n->O * NB, -c0, n->N, n->O, n->B);
+    h.logits = chunk_view(n, c.logits, n->O, c0);
+    h.dlogits = chunk_view(n, c.dl, n->O, c0);
     h.t0 = c0, h.t1 = c1, h.actions = const_cast<void*>(actions), h.logp_old = logp_old, h.weight = weight;
     h.weight_per_agent = weight_per_agent, h.cycle = cycle, h.ratio_out = ratio_out, h.inv_rows = inv_rows;
     h.cliprange = cliprange, h.beta = beta, h.loss_sums = loss_sums;
-    const long long rows = (long long)(c1 - c0) * n->B;
-    const int gx = grid_for(rows, 128);
-    if (c.plan.det) {   // per-warp partial sums, then the fixed-order reduction into loss_sums
-      double* part;
-      if ((rc = reduce_scratch(n, 2ll * n->N * gx * 4, &part))) return rc;
-      D2D_CUDA(cudaMemsetAsync(part, 0, sizeof(double) * 2 * n->N * gx * 4, s));
-      ppo_dlogits_part_kernel<<<gx, 128, 0, s>>>(h, part);
-      D2D_LAUNCHED();
-      if ((rc = launch_sum_partials(part, n->N, gx * 4, 2, loss_sums, s))) return rc;
-    } else {
-      ppo_dlogits_kernel<<<gx, 128, 0, s>>>(h);
-      D2D_LAUNCHED();
-    }
-    if ((rc = backward_chunk(n, params, x, x_lead, c0, c1, c, grads, inv_rows, s))) return rc;
-  }
-  return D2D_OK;
+    // one block row for all agents; the 2 sums (surrogate, entropy) per warp start from zeroed partials
+    const int gx = grid_for((long long)(c1 - c0) * n->B, 128);
+    return launch_loss(n, c, ppo_dlogits_kernel, ppo_dlogits_part_kernel, h, dim3(gx), 2, true, loss_sums, s);
+  };
+  return train_chunks(n, params, x, x_lead, t0, t1, grads, s, "d2d_ppo_policy_grad", loss);
 }
 
 extern "C" int d2d_value_grad(d2d_net* n, const float* params, const float* x, int x_lead, int t0, int t1,
@@ -1182,38 +1129,21 @@ extern "C" int d2d_value_grad(d2d_net* n, const float* params, const float* x, i
                               double* loss_sum, float* value_out, void* stream) {
   D2D_REQUIRE(n && params && x && target && grads && loss_sum, "d2d_value_grad: null argument");
   D2D_REQUIRE(n->O == 1 && n->out_kind == D2D_OUT_IDENTITY, "d2d_value_grad: net is not a critic (n_out 1, identity)");
-  int rc = check_range(n, x_lead, t0, t1, "d2d_value_grad");
-  if (rc) return rc;
   D2D_REQUIRE(padded == 1 || n->arch == D2D_NET_MLP, "d2d_value_grad: GRU critics train on padded windows");
   cudaStream_t s = as_stream(stream);
-  Chunk c;
-  if ((rc = plan_chunk(n, true, t1 - t0, c))) return rc;
   const long long NB = (long long)n->N * n->B;
-  for (int c0 = t0; c0 < t1; c0 += c.Tc) {
-    const int c1 = std::min(t1, c0 + c.Tc);
-    if ((rc = forward_chunk(n, params, x, x_lead, c0, c1, 1, true, c, s))) return rc;
+  auto loss = [&](int c0, int c1, const Chunk& c) {
     MseArgs m;
     memset(&m, 0, sizeof(m));
-    m.value = make_view(c.logits, NB, -c0, n->N, 1, n->B);
-    m.dvalue = make_view(c.dl, NB, -c0, n->N, 1, n->B);
+    m.value = chunk_view(n, c.logits, 1, c0);
+    m.dvalue = chunk_view(n, c.dl, 1, c0);
     m.target = target, m.per_agent = per_agent, m.tgt_t_stride = per_agent ? NB : n->B, m.tgt_t_off = 0;
     m.B = n->B, m.t0 = c0, m.t1 = c1, m.inv_rows = inv_rows, m.loss_sum = loss_sum;
     m.value_out = value_out, m.out_t_stride = NB;
-    const long long rows = (long long)(c1 - c0) * n->B;
-    const int gx = grid_for(rows, 128);
-    if (c.plan.det) {
-      double* part;
-      if ((rc = reduce_scratch(n, (long long)n->N * gx * 4, &part))) return rc;
-      mse_dvalue_part_kernel<<<dim3(gx, n->N), 128, 0, s>>>(m, part);
-      D2D_LAUNCHED();
-      if ((rc = launch_sum_partials(part, n->N, gx * 4, 1, loss_sum, s))) return rc;
-    } else {
-      mse_dvalue_kernel<<<dim3(gx, n->N), 128, 0, s>>>(m);
-      D2D_LAUNCHED();
-    }
-    if ((rc = backward_chunk(n, params, x, x_lead, c0, c1, c, grads, inv_rows, s))) return rc;
-  }
-  return D2D_OK;
+    const int gx = grid_for((long long)(c1 - c0) * n->B, 128);
+    return launch_loss(n, c, mse_dvalue_kernel, mse_dvalue_part_kernel, m, dim3(gx, n->N), 1, false, loss_sum, s);
+  };
+  return train_chunks(n, params, x, x_lead, t0, t1, grads, s, "d2d_value_grad", loss);
 }
 
 extern "C" int d2d_adam_step(float* params, float* m, float* v, const float* grads, int N, int64_t per_agent,
@@ -1284,36 +1214,18 @@ extern "C" int d2d_q_grad(d2d_net* n, const float* params, const float* x, int x
   D2D_REQUIRE(n && params && x && actions && target && grads && loss_sum, "d2d_q_grad: null argument");
   D2D_REQUIRE(n->out_kind == D2D_OUT_IDENTITY, "d2d_q_grad: a Q-network has identity outputs");
   D2D_REQUIRE(loss_kind == D2D_QLOSS_HUBER || loss_kind == D2D_QLOSS_MSE, "d2d_q_grad: unknown loss_kind");
-  int rc = check_range(n, x_lead, t0, t1, "d2d_q_grad");
-  if (rc) return rc;
   cudaStream_t s = as_stream(stream);
-  Chunk c;
-  if ((rc = plan_chunk(n, true, t1 - t0, c))) return rc;
-  const long long NB = (long long)n->N * n->B;
-  for (int c0 = t0; c0 < t1; c0 += c.Tc) {
-    const int c1 = std::min(t1, c0 + c.Tc);
-    if ((rc = forward_chunk(n, params, x, x_lead, c0, c1, 1, true, c, s))) return rc;
+  auto loss = [&](int c0, int c1, const Chunk& c) {
     QLossArgs q;
     memset(&q, 0, sizeof(q));
-    q.q = make_view(c.logits, n->O * NB, -c0, n->N, n->O, n->B);
-    q.dq = make_view(c.dl, n->O * NB, -c0, n->N, n->O, n->B);
+    q.q = chunk_view(n, c.logits, n->O, c0);
+    q.dq = chunk_view(n, c.dl, n->O, c0);
     q.actions = actions, q.target = target, q.q_out = q_out, q.O = n->O, q.B = n->B, q.t0 = c0, q.t1 = c1;
     q.loss_kind = loss_kind, q.inv_rows = inv_rows, q.loss_sum = loss_sum;
-    const long long rows = (long long)(c1 - c0) * n->B;
-    const int gx = grid_for(rows, 128);
-    if (c.plan.det) {
-      double* part;
-      if ((rc = reduce_scratch(n, (long long)n->N * gx * 4, &part))) return rc;
-      q_loss_grad_part_kernel<<<dim3(gx, n->N), 128, 0, s>>>(q, part);
-      D2D_LAUNCHED();
-      if ((rc = launch_sum_partials(part, n->N, gx * 4, 1, loss_sum, s))) return rc;
-    } else {
-      q_loss_grad_kernel<<<dim3(gx, n->N), 128, 0, s>>>(q);
-      D2D_LAUNCHED();
-    }
-    if ((rc = backward_chunk(n, params, x, x_lead, c0, c1, c, grads, inv_rows, s))) return rc;
-  }
-  return D2D_OK;
+    const int gx = grid_for((long long)(c1 - c0) * n->B, 128);
+    return launch_loss(n, c, q_loss_grad_kernel, q_loss_grad_part_kernel, q, dim3(gx, n->N), 1, false, loss_sum, s);
+  };
+  return train_chunks(n, params, x, x_lead, t0, t1, grads, s, "d2d_q_grad", loss);
 }
 
 extern "C" int d2d_replay_gather(const float* obs_ring, const uint8_t* act_ring, const int32_t* rew_ring,
